@@ -35,7 +35,8 @@ def _headers_digest():
     files.append(os.path.join(root, 'include', 'acsr.h'))
     for f in files:
         with open(f, 'rb') as fh:
-            h.update(f.encode() + b'\0' + fh.read())
+            # paths relative to the checkout: a tree copied or moved after the build stays up to date
+            h.update(os.path.relpath(f, root).encode() + b'\0' + fh.read())
     h.update(' '.join(NVCC_FLAGS).encode())
     return h.hexdigest()
 

@@ -4,6 +4,7 @@ synthetic Amazon-Beauty shape (22,363 users, 12,101 items + pad -> V=12,102, L=5
 
     python bench.py --gpus N --steps K --warmup W            # this implementation
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU arm (oracle port of the reference)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also writes the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the training hot path over one batch of 256 sequences: both losses, both
 routed backward passes, Adam (trainer.py:660-687).  `value` times it with the batch already resident
@@ -117,6 +118,14 @@ def timed_steps(fn, n, flush):
         evs.append((e0, e1))
     torch.cuda.synchronize()
     return sum(a.elapsed_time(b) for a, b in evs)
+
+
+def dump_outputs(out_dir, arrays):
+    """write each host tensor as out_dir/<name>.npy: floating point as float32, integers as float64 (exact)"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.numpy().astype(np.float32 if t.is_floating_point() else np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -418,9 +427,10 @@ def run_ours(args):
     model.train()
     step = trainer.graphed_step if use_graph else trainer.train_step
     it = [0]
+    last = {}                                                          # what the latest timed train step / eval batch returned
 
     def dev_step():
-        step(devb[it[0] % nb])
+        last['train'] = step(devb[it[0] % nb])
         it[0] += 1
     loss_pin = torch.empty(3, dtype=torch.float32).pin_memory()
 
@@ -449,6 +459,13 @@ def run_ours(args):
     barrier()
     ms_dev = timed_steps(dev_step, K, flush)
     barrier()
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        # what the caller of the step receives: the two losses.  The graphed step returns them in its static buffers, so they are
+        # copied before the next step.  The parameters are not written: the step accumulates gradients with float atomics, whose
+        # order varies from run to run, and Adam turns that rounding into visible noise in parameters whose true gradient is zero.
+        la, lc = last['train']
+        outputs['train_loss_attacked'], outputs['train_loss_calibrated'] = la.detach().cpu(), lc.detach().cpu()
     for _ in range(3):
         e2e_step()
     barrier()
@@ -490,7 +507,7 @@ def run_ours(args):
     def eval_dev():
         b = devb[it[0] % nb]
         with torch.no_grad():
-            trainer.eval_batch((b, None, None, b['item_id']))
+            last['eval'] = trainer.eval_batch((b, None, None, b['item_id']))
         it[0] += 1
 
     def eval_e2e():
@@ -503,12 +520,16 @@ def run_ours(args):
         eval_dev()
     barrier()
     ms_eval = timed_steps(eval_dev, K, flush)
+    if args.dump_outputs and rank == 0:
+        outputs['eval_rec_topk'] = last['eval'].cpu()
     for _ in range(3):
         eval_e2e()
     barrier()
     ms_eval_e2e = timed_steps(eval_e2e, K, flush)
     barrier()
     clocks = sampler.stop()
+    if outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
     model.train()
     kernels, launches_per_step, eager_ms = kernel_breakdown(A, trainer, devb, nb, cfg, B, V, K)
@@ -1028,9 +1049,14 @@ def main():
     ap.add_argument('--full-len', action='store_true', help='every sequence has the maximum length (worst case) instead of LogNormal lengths')
     ap.add_argument('--batch', type=int, default=0, help='override the per-GPU batch of the workload')
     ap.add_argument('--dp-graph', type=int, default=1, help='capture the NCCL all-reduce inside the CUDA graph at N>1 (0 = eager launches)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what their callers receive: the two losses of the last timed training '
+                         'step and the hit flags of the last timed eval batch, as DIR/<name>.npy')
     ap.add_argument('--profile', action='store_true',
                     help='launch-list mode for ncu: W+K eager training steps and K eval batches, nothing else')
     args = ap.parse_args()
+    if args.dump_outputs and (args.profile or args.impl != 'ours'):
+        ap.error('--dump-outputs writes the outputs of the timed steps of --impl ours')
     WORKLOAD.clear()
     WORKLOAD.update(WORKLOADS[args.workload])
     if args.batch > 0:

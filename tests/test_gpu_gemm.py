@@ -125,8 +125,9 @@ def test_gemm_act(A, act, d, I):
     A.ops.gemm_batch([A.ops.gemm_problem(X, W, Z, R, I, d, bias=b, epilogue=A.ops.EPI_ACT, act=A.ops.ACT_IDS[act], C2=A1)])
     zr = X.double() @ W.double().t()
     close(Z, zr, 3e-6 if d <= 256 else 2e-5, 'Z')
-    # activations with slope <= ~1.1: the output error is bounded by the input error (relative to max |z|, not max |act|)
-    ref = O.act_fn(act)((zr + b.double()).float().cpu()).double()
+    # activations with slope <= ~1.1: the output error is bounded by the input error (relative to max |z|, not max |act|).
+    # The reference is evaluated in float64: a float32 evaluation of erf on the host has been off by 4e-4, beyond the bound.
+    ref = O.act_fn(act)((zr + b.double()).cpu())
     err = float((A1.double().cpu() - ref).abs().max())
     assert err <= 1e-5 * float(ref.abs().max()) + 4e-6 * float(zr.abs().max()), (err, float(zr.abs().max()))
 
