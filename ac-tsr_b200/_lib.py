@@ -172,10 +172,24 @@ def _ab_gemm_batch(a):
     return tot
 
 
+def _ab_neg_sample(a):
+    # (users, positives, perm, cursor, n_rows, M, N, ...): per row the user id, positive, permutation entry and two offsets in;
+    # the M*N negatives out (the used-set probes of the binary searches are L2-resident and not counted)
+    M, N = a[5], a[6]
+    return 8 * (M * N + 5 * M)
+
+
+def _ab_candidate_rank(a):
+    # (out, table, V, d, cand, M, n_cand, kmax, rec, scores, stream): out rows and candidate ids in, one table row per candidate
+    # gathered, hit flags (and scores) out
+    d, M, C, kmax = a[3], a[5], a[6], a[7]
+    return 4 * M * d + M * C * (8 + 4 * d) + 4 * M * (kmax + 1) + (4 * M * C if a[9] else 0)
+
+
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
 ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_ragged': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl, 'acsr_dense_fwd': _ab_dense_fwd, 'acsr_linear_tok_actbwd': _ab_linear_tok_actbwd,
               'acsr_linear_wgrad': _ab_linear_wgrad, 'acsr_linear_wgrad_batched': _ab_linear_wgrad_batched,
-              'acsr_gemm_batch': _ab_gemm_batch}
+              'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank}
 
 
 class KernelTimer:

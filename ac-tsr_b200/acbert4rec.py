@@ -232,3 +232,12 @@ class AcBERT4Rec(SequentialRecommender):
         """fused scores -> scores[:,0] = -inf -> top-k -> hit flags of the calibrated stream (trainer.py:941-942, collector.py:145-153)"""
         _, cal = self._test_outputs(interaction)
         return ops.full_sort_topk(cal.contiguous(), self.item_embedding.weight[:self.n_items], k, positive, self.logits_passes)
+
+    def sampled_topk(self, interaction, candidates, k, positive=None):
+        """sampled-candidate ranking of the calibrated stream (candidates [B, 1+N], positive in column 0, written there from
+        `positive` when given) over the table without the mask-token row -> (scores [B, 1+N], rec_topk [B, k+1])"""
+        if positive is not None:
+            candidates[:, 0].copy_(positive)
+        _, cal = self._test_outputs(interaction)
+        rec, scores = ops.candidate_rank(cal, self.item_embedding.weight[:self.n_items], candidates, k, want_scores=True)
+        return scores, rec

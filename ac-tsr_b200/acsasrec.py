@@ -223,3 +223,22 @@ class ACSASRec(SequentialRecommender):
         finally:
             if was is not None:
                 ops.LIB.query('acsr_set_pdl', was)
+
+    def sampled_topk(self, interaction, candidates, k, positive=None):
+        """Sampled-candidate ranking (`eval_args.mode: uniN / popN`; trainer.py _neg_sample_batch_eval + collector.py
+        eval_batch_collect): candidates [B, 1+N] int64 with the positive in column 0 (written there from `positive` when
+        given).  Encodes each sequence once (the reference predicts on the interaction repeated 1+N times) and ranks the
+        calibrated scores -> (scores [B, 1+N], rec_topk [B, k+1])."""
+        vp = getattr(self, '_vp', None)
+        if vp is not None and vp.sharded:
+            raise ValueError('sampled evaluation is not implemented for a vocab-sharded item table')
+        if positive is not None:
+            candidates[:, 0].copy_(positive)
+        was = ops.LIB.query('acsr_set_pdl', 1) if self._eval_pdl else None
+        try:
+            out, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], need_attacked=False)
+            rec, scores = ops.candidate_rank(out, self.item_embedding.weight, candidates, k, want_scores=True)
+            return scores, rec
+        finally:
+            if was is not None:
+                ops.LIB.query('acsr_set_pdl', was)

@@ -209,3 +209,14 @@ class ACSSEPT(SequentialRecommender):
         cal, _ = self._encode(item_seq, interaction[self.ITEM_SEQ_LEN], user_id, need_attacked=False)
         val, idx, rec = ops.full_sort_topk(self._item_part(cal), self.item_embedding.weight, k, positive, self.logits_passes)
         return val + self._user_term(cal, self.user_test_embedding(user_id)).view(-1, 1), idx, rec
+
+    def sampled_topk(self, interaction, candidates, k, positive=None):
+        """sampled-candidate ranking of the calibrated stream (candidates [B, 1+N], positive in column 0, written there from
+        `positive` when given) -> (scores [B, 1+N], rec_topk [B, k+1]).  The user term is added to the returned scores; it is
+        the same for every candidate of a row and cannot change the rank."""
+        if positive is not None:
+            candidates[:, 0].copy_(positive)
+        user_id = interaction[self.USER_ID]
+        cal, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], user_id, need_attacked=False)
+        rec, scores = ops.candidate_rank(self._item_part(cal), self.item_embedding.weight, candidates, k, want_scores=True)
+        return scores + self._user_term(cal, self.user_test_embedding(user_id)).view(-1, 1), rec

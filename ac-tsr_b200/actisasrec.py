@@ -168,3 +168,13 @@ class ACTiSASRec(SequentialRecommender):
         time_matrix = self.get_time_matrix(interaction[self.timestamp])
         cal, _ = self._encode(item_seq, interaction[self.ITEM_SEQ_LEN], time_matrix, need_attacked=False)
         return ops.full_sort_topk(cal.contiguous(), self.item_embedding.weight, k, positive, self.logits_passes)
+
+    def sampled_topk(self, interaction, candidates, k, positive=None):
+        """sampled-candidate ranking of the calibrated stream (candidates [B, 1+N], positive in column 0, written there from
+        `positive` when given) -> (scores [B, 1+N], rec_topk [B, k+1])"""
+        if positive is not None:
+            candidates[:, 0].copy_(positive)
+        time_matrix = self.get_time_matrix(interaction[self.timestamp])
+        cal, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], time_matrix, need_attacked=False)
+        rec, scores = ops.candidate_rank(cal, self.item_embedding.weight, candidates, k, want_scores=True)
+        return scores, rec

@@ -3,6 +3,7 @@ the trainer iterates (recbole/data/dataloader/general_dataloader.py:23-65, 161-2
 Only what AC-SASRec reads is carried: item_id_list int64[B,L], item_length int64[B], item_id int64[B]
 (the reference moves 5 more unused fields per step, SURVEY a19)."""
 import math
+from contextlib import nullcontext as _nullcontext
 
 import numpy as np
 import torch
@@ -64,12 +65,18 @@ def _model_fields(config):
     return f
 
 
+def _with_user(config, fields):
+    """fields + the user id, which the negative sampler reads (once)"""
+    uid = config['USER_ID_FIELD']
+    return list(fields) + ([uid] if uid not in fields else [])
+
+
 class _PackedBatches(object):
     """The three int64 fields the model reads, re-laid out batch by batch in ONE pinned buffer (refilled in place after every
     shuffle), so that each batch is a single contiguous host->device copy.  Full batches only; a ragged tail stays unpacked."""
 
-    def __init__(self, config, batch_size):
-        self.fields, self.bs, self.buf = _model_fields(config), batch_size, None
+    def __init__(self, config, batch_size, fields=None):
+        self.fields, self.bs, self.buf = (fields or _model_fields(config)), batch_size, None
 
     def fill(self, inter_feat):
         n = len(inter_feat)
@@ -100,11 +107,16 @@ class _PackedBatches(object):
 class TrainDataLoader(object):
     """general_dataloader.py:23-65: per-epoch CPU randperm shuffle, then contiguous batch slices."""
 
-    def __init__(self, config, dataset, shuffle=True, batch_size=None):
+    def __init__(self, config, dataset, shuffle=True, batch_size=None, neg_sampler=None):
         self.config, self.dataset, self.shuffle = config, dataset, shuffle
         self.batch_size = batch_size or config['train_batch_size']
         self.pr = 0
-        self._packed = _PackedBatches(config, self.batch_size) if config.get('packed_batches', True) else None
+        # BPR with `neg_sampling`: batches carry the user id; the trainer draws the negatives on the device (ops.NegSampler)
+        self.neg_sampler = neg_sampler
+        if neg_sampler is not None:
+            neg_sampler.check_users(dataset.inter_feat[config['USER_ID_FIELD']])
+        fields = _with_user(config, _model_fields(config)) if neg_sampler is not None else None
+        self._packed = _PackedBatches(config, self.batch_size, fields) if config.get('packed_batches', True) else None
         self._filled = False
 
     @property
@@ -149,7 +161,7 @@ class DeviceTrainDataLoader(object):
 
     device_resident = True
 
-    def __init__(self, config, dataset, shuffle=True, batch_size=None, device=None):
+    def __init__(self, config, dataset, shuffle=True, batch_size=None, device=None, neg_sampler=None):
         from ._lib import LIB
         from .compat import PackedInteraction
         self.LIB, self.PackedInteraction = LIB, PackedInteraction
@@ -168,7 +180,13 @@ class DeviceTrainDataLoader(object):
         self.tgts = feat[f[2]].to(self.device).contiguous()
         neg_field = config['NEG_PREFIX'] + config['ITEM_ID_FIELD']
         self.negs = feat[neg_field].to(self.device).contiguous() if neg_field in feat else None
-        if self.negs is not None:
+        # BPR with `neg_sampling`: the user ids stay in HBM too, and the sampler fills the neg slot of every gathered batch
+        self.neg_sampler = neg_sampler if self.negs is None else None
+        self.uids = None
+        if self.neg_sampler is not None:
+            self.neg_sampler.check_users(feat[config['USER_ID_FIELD']])
+            self.uids = feat[config['USER_ID_FIELD']].to(self.device).contiguous()
+        if self.negs is not None or self.neg_sampler is not None:
             self.fields.append(neg_field)
         self.n, self.L = int(self.seqs.shape[0]), int(self.seqs.shape[1])
         self.perm = torch.arange(self.n, dtype=torch.int64, device=self.device)
@@ -211,11 +229,18 @@ class DeviceTrainDataLoader(object):
         self.pr = 0
 
     def gather_into(self, packed, stream=None):
-        """enqueue: packed <- batch `cursor` of the permutation; cursor += 1  (two launches; graph-capturable)"""
+        """enqueue: packed <- batch `cursor` of the permutation; with a negative sampler its draws for the same rows into the
+        neg slot; cursor += 1  (two or three launches; graph-capturable)"""
         st = torch.cuda.current_stream().cuda_stream if stream is None else stream
         self.LIB.call('acsr_batch_gather', self.seqs.data_ptr(), self.lens.data_ptr(), self.tgts.data_ptr(),
                       self.negs.data_ptr() if self.negs is not None else None, self.perm.data_ptr(), self.cursor.data_ptr(), self.n,
                       self.batch_size, self.L, packed.data_ptr(), st)
+        if self.neg_sampler is not None:
+            lay = dict((k, off) for k, off, _ in self.layout()[0])
+            off = lay[self.fields[3]]
+            with torch.cuda.stream(torch.cuda.ExternalStream(st)) if stream is not None else _nullcontext():
+                self.neg_sampler.draw(self.uids, 1, positives=self.tgts, out=packed[off:off + self.batch_size].view(-1, 1), ld=1,
+                                      perm=self.perm, cursor=self.cursor, n_rows=self.n, rows=self.batch_size)
         self.LIB.call('acsr_cursor_advance', self.cursor.data_ptr(), st)
 
     def tail_batch(self):
@@ -227,6 +252,8 @@ class DeviceTrainDataLoader(object):
         f = {self.fields[0]: self.seqs[idx], self.fields[1]: self.lens[idx], self.fields[2]: self.tgts[idx]}
         if self.negs is not None:
             f[self.fields[3]] = self.negs[idx]
+        elif self.neg_sampler is not None:
+            f[self.fields[3]] = self.neg_sampler.draw(self.uids[idx], 1, positives=f[self.fields[2]]).view(-1)
         return Interaction(f)
 
     def __iter__(self):
@@ -282,3 +309,23 @@ class FullSortEvalDataLoader(object):
         n = len(interaction)
         self.pr += self.batch_size
         return interaction, None, torch.arange(n), interaction[self.iid_field]
+
+
+class NegSampleEvalDataLoader(FullSortEvalDataLoader):
+    """`eval_args.mode: uniN / popN` (general_dataloader.py NegSampleEvalDataLoader, sequential branch): yields
+    (interaction, None, positive_u=arange(B), positive_i=item_id) like FullSortEvalDataLoader, with the user id in every batch.
+    The N negatives of a batch are not drawn here but on the device by the trainer (`neg_sampler`, an ops.NegSampler holding
+    this phase's used sets), fresh for every batch of every pass."""
+
+    def __init__(self, config, dataset, neg_sampler, neg_num, batch_size=None):
+        self.neg_sampler, self.neg_num = neg_sampler, int(neg_num)
+        neg_sampler.check_users(dataset.inter_feat[config['USER_ID_FIELD']])
+        self.uid_field = config['USER_ID_FIELD']
+        self.config, self.dataset = config, dataset
+        self.batch_size = batch_size or config['eval_batch_size']
+        self.iid_field = config['ITEM_ID_FIELD']
+        self.pr = 0
+        self._packed = (_PackedBatches(config, self.batch_size, _with_user(config, _model_fields(config)))
+                        if config.get('packed_batches', True) else None)
+        if self._packed is not None:
+            self._packed.fill(dataset.inter_feat)

@@ -14,7 +14,8 @@ Rebuilds, for sequential models, what the reference does between a `<dataset>.in
 All of it is vectorised numpy (the reference loops in Python over interactions); results are bit-identical to the reference's
 pipeline (tests/test_dataset_pipeline.py compares every tensor on ml-100k).  Only the fields the model reads are materialised
 (`item_id_list`, `item_length`, `item_id`, `user_id`; the reference also builds `rating_list` / `timestamp_list`, which nothing
-consumes -- SURVEY a19).  Out of scope here: user / item side-feature files, knowledge graphs, negative sampling, `RS` splits.
+consumes -- SURVEY a19).  Out of scope here: user / item side-feature files, knowledge graphs, `RS` splits.  Negative sampling
+(`neg_sampling` for BPR, `eval_args.mode: uniN / popN`) is drawn on the device (ops.NegSampler); this module builds its used sets.
 """
 import copy
 import gzip
@@ -24,7 +25,7 @@ import os
 import numpy as np
 import torch
 
-from .compat import Interaction
+from .compat import Interaction, cfg_get
 
 
 # ---------------------------------------------------------------------------------------------
@@ -307,12 +308,70 @@ def device_resident_training(config):
             and str(config.get('model', 'ACSASRec')) == 'ACSASRec')
 
 
+def parse_eval_mode(mode):
+    """eval_args.mode (config/configurator.py, data/utils.py:96-150) -> ('full', 0) | ('uniform', N) | ('popularity', N)"""
+    m = str('full' if mode is None else mode)
+    if m == 'full':
+        return 'full', 0
+    for prefix, dist in (('uni', 'uniform'), ('pop', 'popularity')):
+        if m.startswith(prefix) and m[len(prefix):].isdigit() and int(m[len(prefix):]) > 0:
+            return dist, int(m[len(prefix):])
+    raise NotImplementedError('eval_args.mode %r: only full, uniN and popN evaluation are implemented' % m)
+
+
+def parse_neg_sampling(config):
+    """`neg_sampling` -> 'uniform' | 'popularity' | None.  Only loss_type BPR reads it (with CE it is ignored, as in the reference's
+    sequential models); one negative per row, since RecBole repeats the batch rows for more."""
+    ns = config['neg_sampling']
+    if not ns or str(cfg_get(config, 'loss_type', 'CE')) != 'BPR':
+        return None
+    if not isinstance(ns, dict) or len(ns) != 1:
+        raise ValueError('neg_sampling must be one of {uniform: 1} / {popularity: 1} (got %r)' % (ns,))
+    (dist, num), = ns.items()
+    if dist not in ('uniform', 'popularity'):
+        raise ValueError('neg_sampling distribution %r: must be uniform or popularity' % (dist,))
+    if int(num) != 1:
+        raise NotImplementedError('neg_sampling {%s: %s}: only one negative per training row is implemented' % (dist, num))
+    return dist
+
+
+def build_neg_samplers(config, splits, train_dist, eval_dist):
+    """-> (train, valid, test) ops.NegSampler | None.  Used ids of a phase: the targets of the user's rows in the splits up to
+    and including it (sampler.py get_used_ids; a history's first item is never a target and stays drawable); popularity: the
+    item counts over the targets of all three splits."""
+    from .ops import NegSampler, alias_table, used_item_csr
+    ds = splits[0]
+    uf, itf = ds.uid_field, ds.iid_field
+    n_users, n_items = ds.user_num, ds.item_num
+    uids = [s.inter_feat[uf].numpy() for s in splits]
+    iids = [s.inter_feat[itf].numpy() for s in splits]
+    counts = np.bincount(np.concatenate(iids), minlength=n_items).astype(np.float64)
+    seed = int(config['seed'] if config['seed'] is not None else 0)
+    alias = alias_table(counts) if 'popularity' in (train_dist, eval_dist) else None       # built once, shared by the phases
+    out = []
+    for phase, dist in enumerate((train_dist, eval_dist, eval_dist)):
+        if dist is None:
+            out.append(None)
+            continue
+        off, items = used_item_csr(np.concatenate(uids[:phase + 1]), np.concatenate(iids[:phase + 1]), n_users, n_items)
+        out.append(NegSampler(dist, off, items, n_items, seed, phase=phase, counts=counts, alias=alias))
+    return out
+
+
 def data_preparation(config, dataset):
     """data/utils.py:96-150 -> (train_data, valid_data, test_data)"""
-    from .data import TrainDataLoader, DeviceTrainDataLoader, FullSortEvalDataLoader
+    from .data import TrainDataLoader, DeviceTrainDataLoader, FullSortEvalDataLoader, NegSampleEvalDataLoader
     train, valid, test = dataset.build()
-    if (config['eval_args'] or {}).get('mode', 'full') != 'full':
-        raise NotImplementedError('eval_args.mode: only full-sort evaluation is on the hot path')
+    eval_dist, n_eval_neg = parse_eval_mode((config['eval_args'] or {}).get('mode', 'full'))
+    eval_dist = None if eval_dist == 'full' else eval_dist
+    train_dist = parse_neg_sampling(config)
+    if str(config.get('model', '')) == 'AcBERT4Rec':
+        train_dist = None                        # its masked-item loss draws its own negatives (acbert4rec.py:89-93)
+    samplers = build_neg_samplers(config, (train, valid, test), train_dist, eval_dist) if (train_dist or eval_dist) else (None,) * 3
     # training data resident in HBM with the epoch shuffle on the device (f-2) unless `device_resident_data: False`
-    train_loader = (DeviceTrainDataLoader if device_resident_training(config) else TrainDataLoader)(config, train, shuffle=True)
-    return (train_loader, FullSortEvalDataLoader(config, valid), FullSortEvalDataLoader(config, test))
+    train_loader = (DeviceTrainDataLoader if device_resident_training(config) else TrainDataLoader)(
+        config, train, shuffle=True, **({'neg_sampler': samplers[0]} if samplers[0] is not None else {}))
+    if eval_dist is None:
+        return (train_loader, FullSortEvalDataLoader(config, valid), FullSortEvalDataLoader(config, test))
+    return (train_loader, NegSampleEvalDataLoader(config, valid, samplers[1], n_eval_neg),
+            NegSampleEvalDataLoader(config, test, samplers[2], n_eval_neg))

@@ -4,6 +4,7 @@ PyTorch is plumbing here: it owns device memory, the stream and the autograd tap
 below launches hand-written sm_100a kernels from libacsr.so.  Tensors must be CUDA, contiguous,
 float32 (ids int64) -- anything else raises; there is no CPU or eager fallback.
 """
+import numpy as np
 import torch
 
 from ._lib import LIB, AcsrError
@@ -861,6 +862,144 @@ def full_sort_topk(out, table, k, positive=None, passes=3):
         return topk_select(logits_scores(out, table, passes), k, positive)
     pv, pi = logits_topk_partial(out, table, k, 0, True, passes)
     return topk_merge(pv, pi, k, positive)
+
+
+# ------------------------------------------------------------------------------------------
+# negative sampling and sampled-candidate ranking (negsample.cu)
+# ------------------------------------------------------------------------------------------
+def neg_sample(users, n_neg, used_offsets, used_items, n_items, rng, rng_stream, positives=None, alias=None, out=None, ld=None,
+               perm=None, cursor=None, n_rows=0, rows=None):
+    """-> negs [M, n_neg] int64: per row, items of [1, n_items) outside the user's used set (acsr_neg_sample).  out may be a
+    row-strided view (ld = its row stride, e.g. columns 1.. of a candidate matrix).  With perm / cursor, row m reads users /
+    positives at perm[cursor * rows + m] (the batch acsr_batch_gather writes)."""
+    M = int(rows if rows is not None else users.shape[0])
+    n_src = int(n_rows) if perm is not None else M                   # rows users / positives are read at
+    if users.dim() != 1 or users.shape[0] < n_src or (positives is not None and tuple(positives.shape) != tuple(users.shape)):
+        raise AcsrError('neg_sample: users (and positives) must be 1-D with at least %d rows (got %s)' % (n_src, tuple(users.shape)))
+    if perm is not None and perm.numel() != n_src:
+        raise AcsrError('neg_sample: perm has %d entries, n_rows is %d' % (perm.numel(), n_src))
+    if out is None:
+        out = torch.empty((M, n_neg), dtype=torch.int64, device=used_items.device)
+        ld = n_neg
+    if out.dim() != 2 or tuple(out.shape) != (M, int(n_neg)):
+        raise AcsrError('neg_sample: out must be a [%d, %d] matrix (got %s)' % (M, n_neg, tuple(out.shape)))
+    if ld is None:
+        ld = out.stride(0)
+    if not out.is_cuda or out.dtype != torch.int64 or out.stride(1) != 1 or (M > 1 and out.stride(0) != ld) or ld < n_neg:
+        raise AcsrError('neg_sample: out must be an int64 CUDA matrix with unit column stride and row stride ld >= n_neg')
+    prob, idx = alias if alias is not None else (None, None)
+    LIB.call('acsr_neg_sample', _p(users, torch.int64), _p(positives, torch.int64), _p(perm, torch.int64), _p(cursor, torch.int64),
+             int(n_rows), M, int(n_neg), _p(used_offsets, torch.int64), _p(used_items, torch.int64), used_offsets.numel() - 1,
+             int(n_items), _p(prob), _p(idx, torch.int64), rng.ptr, int(rng_stream), out.data_ptr(), int(ld), _stream())
+    return out
+
+
+def candidate_rank(out, table, cand, k, want_scores=False):
+    """rank of column 0 of cand [M, 1+N] among the distinct other candidates by out[m] . table[c] (fp32), as the hit-flag
+    matrix rec [M, k+1] int32 of the evaluator (acsr_candidate_rank) -> (rec, scores [M, 1+N] | None)"""
+    out, table, cand = out.contiguous(), table.contiguous(), cand.contiguous()
+    if out.dim() != 2 or table.dim() != 2 or cand.dim() != 2:
+        raise AcsrError('candidate_rank: out [M, d], table [V, d] and cand [M, 1+N] must be matrices')
+    M, d = out.shape
+    if table.shape[1] != d or cand.shape[0] != M or int(k) < 1:
+        raise AcsrError('candidate_rank: out %s, table %s and cand %s disagree (or k=%d < 1)' % (tuple(out.shape), tuple(table.shape),
+                                                                                            tuple(cand.shape), int(k)))
+    rec = torch.empty((M, k + 1), dtype=torch.int32, device=out.device)
+    scores = torch.empty(cand.shape, dtype=torch.float32, device=out.device) if want_scores else None
+    LIB.call('acsr_candidate_rank', _p(out), _p(table), table.shape[0], d, _p(cand, torch.int64), M, cand.shape[1], int(k),
+             _p(rec, torch.int32), _p(scores), _stream())
+    return rec, scores
+
+
+def used_item_csr(uid, iid, n_users, n_items):
+    """per-user sorted unique items as a CSR (offsets [n_users+1], items) from parallel id arrays"""
+    uid, iid = np.asarray(uid, dtype=np.int64), np.asarray(iid, dtype=np.int64)
+    key = np.unique(uid * int(n_items) + iid)
+    users, items = key // int(n_items), key % int(n_items)
+    offsets = np.zeros(int(n_users) + 1, dtype=np.int64)
+    np.cumsum(np.bincount(users, minlength=int(n_users)), out=offsets[1:])
+    return offsets, items.astype(np.int64)
+
+
+def alias_table(counts):
+    """Walker alias table of the distribution counts / counts.sum() -> (prob float32, alias int64): draw i uniform, u uniform on
+    (0, 1]; the item is i when u <= prob[i], else alias[i].  Vose's pairing, vectorised: the smalls (scaled mass < 1) are poured
+    in order into the larges in order, so small i goes to the large whose cumulative excess E first reaches the smalls'
+    cumulative deficit D before it, and large j, once D passes E_j, keeps 1 + E_j - D (its overflow) and aliases large j + 1."""
+    w = np.asarray(counts, dtype=np.float64)
+    n = len(w)
+    scaled = w * (n / w.sum())
+    prob = np.ones(n, dtype=np.float64)
+    alias = np.arange(n, dtype=np.int64)
+    small, large = np.nonzero(scaled < 1.0)[0], np.nonzero(scaled >= 1.0)[0]
+    if len(small) and len(large):
+        D = np.cumsum(1.0 - scaled[small])
+        E = np.cumsum(scaled[large] - 1.0)
+        j = np.searchsorted(E, np.concatenate(([0.0], D[:-1])), side='left')     # the large each small is poured into
+        ok = j < len(large)                                                    # (beyond the last: rounding leftovers, kept ~1)
+        prob[small[ok]], alias[small[ok]] = scaled[small[ok]], large[j[ok]]
+        i = np.searchsorted(D, E, side='right')                                # the small whose deficit overflows large j
+        sw = np.nonzero((i < len(small)) & (np.arange(len(large)) + 1 < len(large)))[0]
+        prob[large[sw]], alias[large[sw]] = 1.0 + E[sw] - D[i[sw]], large[sw + 1]
+    return prob.astype(np.float32), alias
+
+
+class NegSampler(object):
+    """Device-side negative sampler of one phase (RecBole 1.0.1's non-repeatable Sampler, sampler.py): the users' used sets as
+    a CSR, for popularity the alias table of the item counts, and its own Philox state {seed, step} -- a DeviceRng separate
+    from the model's dropout stream, so drawing negatives leaves training randomness untouched.  Every draw() advances the
+    state first: each training step and each evaluation batch gets fresh negatives, reproducible from the seed."""
+
+    RNG_STREAM = 0x4E470000                       # + phase: train / valid / test draw from disjoint counters
+
+    def __init__(self, distribution, used_offsets, used_items, n_items, seed, phase=0, counts=None, alias=None):
+        if distribution not in ('uniform', 'popularity'):
+            raise ValueError('negative sampling distribution must be uniform or popularity (got %r)' % (distribution,))
+        self.distribution, self.n_items, self.seed = distribution, int(n_items), int(seed)
+        self.used_offsets, self.used_items = np.asarray(used_offsets, np.int64), np.asarray(used_items, np.int64)
+        self.n_users = len(self.used_offsets) - 1
+        self.rng_stream = self.RNG_STREAM + int(phase)
+        self.alias = None
+        if distribution == 'popularity':
+            counts = np.asarray(counts, dtype=np.float64)
+            if counts.shape != (self.n_items,) or counts.sum() <= 0:
+                raise ValueError('popularity sampling needs item counts of shape [n_items] with a positive sum')
+            self.counts = counts
+            self.alias = alias if alias is not None else alias_table(counts)      # phases of one dataset share one table
+        full = np.diff(self.used_offsets) >= self.n_items - 1
+        if full.any():
+            raise ValueError('user %d has interacted with every item: no negative can be drawn' % int(np.nonzero(full)[0][0]))
+        self.rng = None
+        self._dev = None
+
+    def check_users(self, user_ids):
+        """a row whose user id lies outside [0, n_users) gets item 0 from acsr_neg_sample: loaders reject such data up front"""
+        u = np.asarray(user_ids.cpu() if torch.is_tensor(user_ids) else user_ids)
+        if u.size and (u.min() < 0 or u.max() >= self.n_users):
+            raise ValueError('user ids must lie in [0, %d) for this sampler (got %d..%d)' % (self.n_users, int(u.min()), int(u.max())))
+
+    def to_device(self, device):
+        """upload once per device ('cuda' and 'cuda:<current>' are the same device: the state a captured graph points at must
+        not be replaced)"""
+        device = torch.device(device)
+        if device.type == 'cuda' and device.index is None:
+            device = torch.device('cuda', torch.cuda.current_device())
+        if self._dev is None or self._dev[0].device != device:
+            t = [torch.from_numpy(self.used_offsets).to(device), torch.from_numpy(self.used_items).to(device)]
+            if self.alias is not None:
+                t += [torch.from_numpy(self.alias[0]).to(device), torch.from_numpy(self.alias[1]).to(device)]
+            self._dev = t
+            self.rng = DeviceRng(self.seed, device)
+        return self
+
+    def draw(self, users, n_neg, positives=None, out=None, ld=None, perm=None, cursor=None, n_rows=0, rows=None, advance=True):
+        """advance the sampler's state (unless advance=False), then enqueue acsr_neg_sample -> negs [M, n_neg]"""
+        self.to_device(users.device)
+        if advance:
+            self.rng.advance()
+        alias = (self._dev[2], self._dev[3]) if self.alias is not None else None
+        return neg_sample(users, n_neg, self._dev[0], self._dev[1], self.n_items, self.rng, self.rng_stream, positives, alias,
+                          out, ld, perm, cursor, n_rows, rows)
 
 
 def adam_step(param, grad, exp_avg, exp_avg_sq, step_count, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0):

@@ -212,6 +212,9 @@ class ACSASRecTrainer(object):
             self.fused = FusedTrainStep(model, self.optimizer)
             model._fused_step = self.fused          # eval batches reuse the fused forward (ACSASRec._encode)
         self.nan_check_interval = int(cfg_get(config, 'nan_check_interval', 50))
+        # BPR with `neg_sampling` on host-side batches: the ops.NegSampler that draws each step's negatives on the device
+        # (set from the training loader by _train_epoch; a DeviceTrainDataLoader draws inside its own gather instead)
+        self.train_neg_sampler = None
         self.logger.info('use attack trainer!!!')
 
     # ------------------------------------------------------------------------------------------
@@ -322,17 +325,32 @@ class ACSASRecTrainer(object):
 
     def train_step(self, interaction):
         """One optimisation step on a device-resident Interaction (eager launch path)."""
-        return self._step_body(interaction)
+        return self._step_body(self._draw_negatives(interaction))
+
+    def _needs_negatives(self, interaction):
+        return self.train_neg_sampler is not None and self.model.NEG_ITEM_ID not in interaction
+
+    def _draw_negatives(self, interaction):
+        """a device batch without negatives under BPR + `neg_sampling`: the same batch plus one negative per row, drawn on the
+        device by the training sampler (recbole/data/dataloader/general_dataloader.py's neg_sample_by, sampler.py)"""
+        if not self._needs_negatives(interaction):
+            return interaction
+        m = self.model
+        f = dict(interaction.interaction)
+        f[m.NEG_ITEM_ID] = self.train_neg_sampler.draw(interaction[m.USER_ID], 1, positives=interaction[m.POS_ITEM_ID]).view(-1)
+        return Interaction(f)
 
     # -------- CUDA-graph replay of the whole step ----------------------------------------------
     def _graph_key(self, interaction):
-        return tuple((k, tuple(interaction[k].shape)) for k in self._fields())
+        return tuple((k, tuple(interaction[k].shape)) for k in self._fields() if k in interaction)
 
     def _fields(self):
         m = self.model
         f = [m.ITEM_SEQ, m.ITEM_SEQ_LEN, m.POS_ITEM_ID]
         if m.loss_type == 'BPR':
             f.append(m.NEG_ITEM_ID)
+        if self.train_neg_sampler is not None and m.USER_ID not in f:
+            f.append(m.USER_ID)                    # read by the negative sampler
         return f + [k for k in getattr(m, 'EXTRA_FIELDS', []) if k not in f]      # ACSSEPT: user id; ACTiSASRec: time stamps
 
     def _capture(self, interaction=None, loader=None):
@@ -340,33 +358,53 @@ class ACSASRecTrainer(object):
         before each replay; loader (data.DeviceTrainDataLoader): the batch is gathered from the HBM-resident data by the first
         two nodes of the graph itself (acsr_batch_gather + acsr_cursor_advance) -- a replay needs no input at all."""
         dev = self.device
+        m = self.model
+        # BPR + neg_sampling on host batches: the static buffers get a neg slot the sampler fills inside the graph
+        draw = loader is None and self._needs_negatives(interaction)
+        present = [k for k in self._fields() if loader is not None or k in interaction]
         # static input buffers: one flat buffer with the fields as views, so a packed host batch arrives as ONE copy
         if loader is not None:
             lay, total = loader.layout()
         else:
             lay, total = None, 0
-            if all(interaction[k].dtype == torch.int64 for k in self._fields()):
-                lay, total = PackedInteraction.layout_of({k: interaction[k] for k in self._fields()})
+            if all(interaction[k].dtype == torch.int64 for k in present):
+                lay, total = PackedInteraction.layout_of({k: interaction[k] for k in present})
+                if draw:
+                    B = int(interaction[m.POS_ITEM_ID].shape[0])
+                    lay, total = lay + [(m.NEG_ITEM_ID, total, (B,))], total + B
         if loader is None and lay is None:        # a float field (ACTiSASRec's time stamps): one static tensor per field
-            static_inter = Interaction({k: torch.empty_like(interaction[k], device=dev) for k in self._fields()})
+            f = {k: torch.empty_like(interaction[k], device=dev) for k in present}
+            if draw:
+                f[m.NEG_ITEM_ID] = torch.empty_like(interaction[m.POS_ITEM_ID], device=dev)
+            static_inter = Interaction(f)
         else:
             static_inter = PackedInteraction(torch.empty(total, dtype=torch.int64, device=dev), lay)
-        static = {k: static_inter[k] for k in self._fields()}
+        static = {k: static_inter[k] for k in self._fields() if k in static_inter}
         if loader is None:
-            for k in static:
+            for k in present:
                 static[k].copy_(interaction[k])
         self.model._runtime(dev)               # creates the device RNG state, so the snapshot below covers it
+        sampler = self.train_neg_sampler if draw else None
+        if sampler is not None:
+            sampler.to_device(dev)
 
         def body():
             if loader is not None:
                 loader.gather_into(static_inter.packed)
+            if sampler is not None:
+                sampler.draw(static_inter[m.USER_ID], 1, positives=static_inter[m.POS_ITEM_ID],
+                             out=static_inter[m.NEG_ITEM_ID].view(-1, 1), ld=1)
             return self._step_body(static_inter)
+        loader_sampler = getattr(loader, 'neg_sampler', None) if loader is not None else None
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):          # warm-up on a side stream (allocator + lazy inits), state restored after
+            if loader_sampler is not None:
+                loader_sampler.to_device(dev)
+            rngs = [s.rng.state for s in (sampler, loader_sampler) if s is not None]
             snap = (self.optimizer.flat_param.clone(), self.optimizer.exp_avg.clone(), self.optimizer.exp_avg_sq.clone(),
                     self.optimizer.step_count.clone(), self.model._rng.state.clone() if self.model._rng else None,
-                    loader.cursor.clone() if loader is not None else None)
+                    loader.cursor.clone() if loader is not None else None, [r.clone() for r in rngs])
             for _ in range(2):
                 body()
             self.optimizer.flat_param.copy_(snap[0]); self.optimizer.exp_avg.copy_(snap[1])
@@ -375,6 +413,8 @@ class ACSASRecTrainer(object):
                 self.model._rng.state.copy_(snap[4])
             if snap[5] is not None:
                 loader.cursor.copy_(snap[5])
+            for r, v in zip(rngs, snap[6]):
+                r.copy_(v)
         torch.cuda.current_stream().wait_stream(side)
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
@@ -383,7 +423,7 @@ class ACSASRecTrainer(object):
         if loader is not None:
             self._dgraph = dict(rec, loader=loader)
         else:
-            self._graph = dict(rec, key=self._graph_key(interaction))
+            self._graph = dict(rec, key=self._graph_key(interaction), sampler=sampler)
 
     def device_loader_step(self, loader):
         """one optimisation step on the next batch of a data.DeviceTrainDataLoader: a bare graph replay (the batch is gathered
@@ -406,22 +446,27 @@ class ACSASRecTrainer(object):
         static buffers on the current stream and replays the captured step."""
         if self._host_schedule() or int(interaction[self.model.ITEM_SEQ].shape[1]) > 64:
             # annealing: see _host_schedule; sequences longer than 64: the attention backward's workspace may have to grow
-            return self._step_body(interaction.to(self.device))
+            return self.train_step(interaction.to(self.device))
         if self.fused is None and hasattr(self.model, 'prepare_batch'):
             if self._graph is not None and self._graph['key'][0][1] != tuple(interaction[self.model.ITEM_SEQ].shape):
                 return self._step_body(interaction.to(self.device))      # ragged last batch: eager launch (masks itself)
             interaction = self.model.prepare_batch(interaction)          # host half of the step (AcBERT4Rec's python masking)
+        if self._graph is not None and self._graph['sampler'] is not (self.train_neg_sampler if self._needs_negatives(interaction) else None):
+            self._graph = None                     # the captured step draws from another sampler's device state: capture anew
         if self._graph is None or self._graph['key'] != self._graph_key(interaction):
             if self._graph is not None:
-                return self._step_body(interaction.to(self.device))      # ragged last batch: eager launch
+                return self.train_step(interaction.to(self.device))      # ragged last batch: eager launch
             self._capture(interaction)
         si = self._graph['static_inter']
-        if getattr(interaction, 'layout', None) == getattr(si, 'layout', ()):
-            si.packed.copy_(interaction.packed, non_blocking=True)          # packed batch: one copy
+        lay = getattr(interaction, 'layout', None)
+        if lay is not None and lay == getattr(si, 'layout', [])[:len(lay)]:
+            # packed batch: one copy (a trailing neg slot the captured sampler fills is not part of it)
+            si.packed[:interaction.packed.numel()].copy_(interaction.packed, non_blocking=True)
         else:
             st = self._graph['static']
             for k in st:
-                st[k].copy_(interaction[k], non_blocking=True)
+                if k in interaction:
+                    st[k].copy_(interaction[k], non_blocking=True)
         self._graph['graph'].replay()
         return self._graph['la'], self._graph['lc']
 
@@ -439,6 +484,8 @@ class ACSASRecTrainer(object):
         # (GRAPH_SAFE_STEP) -- the autograd Functions' forward + routed double backward + Adam as they launch
         graph_ok = (self.use_graph and (self.fused is not None or getattr(self.model, 'GRAPH_SAFE_STEP', False))
                     and isinstance(self.optimizer, FlatAdam) and not self.clip_grad_norm)
+        if not getattr(train_data, 'device_resident', False):
+            self.train_neg_sampler = getattr(train_data, 'neg_sampler', None)
         if (getattr(train_data, 'device_resident', False) and graph_ok and self.fused is not None and not self._host_schedule()
                 and train_data.L <= 64 and train_data.full_batches > 0):
             # HBM-resident data (f-2): the epoch is graph replays + one eager step for the ragged tail
@@ -581,11 +628,15 @@ class ACSASRecTrainer(object):
             scores[history_index] = -np.inf
         return interaction, scores, positive_u, positive_i
 
-    def eval_batch(self, batched_data, rec_out=None):
+    def eval_batch(self, batched_data, rec_out=None, neg_sampler=None, neg_num=0):
         """-> rec_topk [B, kmax+1] int32 on the device (collector.py:145-153 'rec.topk'); with rec_out (a pinned host tensor)
-        the graphed path copies the result straight into it (no device-side clone) and returns rec_out."""
+        the graphed path copies the result straight into it (no device-side clone) and returns rec_out.  With neg_sampler (the
+        batch of a data.NegSampleEvalDataLoader, `eval_args.mode: uniN / popN`): the positive is ranked against neg_num
+        negatives drawn on the device (trainer.py _neg_sample_batch_eval, collector.py eval_batch_collect)."""
         interaction, history_index, positive_u, positive_i = batched_data
         kmax = max(self.topk)
+        if neg_sampler is not None:
+            return self._sampled_eval(interaction, positive_i, neg_sampler, int(neg_num), kmax, rec_out)
         if self.fused_topk and history_index is None:
             if kmax > 64:                      # the fused top-k keeps at most 64 candidates per row: materialised scores + torch.topk
                 return self._eval_materialised(batched_data, kmax, rec_out)
@@ -659,6 +710,84 @@ class ACSASRecTrainer(object):
             return rec_out
         return g['rec'].clone()
 
+    def _sampled_body(self, inter, pos, cand, sampler, kmax):
+        """negatives into cand[:, 1:] (the sampler's state advances), the positive into column 0, rank -> rec [B, kmax+1]"""
+        m = self.model
+        N = cand.shape[1] - 1
+        sampler.draw(inter[m.USER_ID], N, positives=pos, out=cand[:, 1:], ld=N + 1)
+        _, rec = m.sampled_topk(inter, cand, kmax, pos)
+        return rec
+
+    @torch.no_grad()
+    def _sampled_eval(self, interaction, positive_i, sampler, N, kmax, rec_out=None):
+        """one batch of sampled-candidate evaluation: sampler -> encoder -> acsr_candidate_rank, eagerly or as a CUDA-graph
+        replay (one graph per batch shape; every replay draws fresh negatives)"""
+        m = self.model
+        if self._sharded():
+            raise ValueError('sampled evaluation (eval_args.mode uniN / popN) needs the replicated item table; '
+                             'it is not implemented for a vocab-sharded table')
+        if not hasattr(m, 'sampled_topk'):
+            raise NotImplementedError('%s has no sampled_topk: sampled evaluation is not available for it' % type(m).__name__)
+        dev = self.device
+        sampler.to_device(dev)
+        if not (self.use_graph and not m.training and not self._host_schedule()):
+            inter = interaction.to(dev)
+            pos = positive_i.to(dev)
+            cand = torch.empty((pos.shape[0], N + 1), dtype=torch.int64, device=dev)
+            rec = self._sampled_body(inter, pos, cand, sampler, kmax)
+            if rec_out is not None:
+                rec_out.copy_(rec, non_blocking=True)
+                return rec_out
+            return rec
+        fields = list(getattr(m, 'EVAL_FIELDS', None) or [m.ITEM_SEQ, m.ITEM_SEQ_LEN])
+        if m.USER_ID not in fields:
+            fields.append(m.USER_ID)
+        # the graph captures the sampler's device state (used sets, alias table, Philox state): one graph per sampler, which the
+        # record keeps alive so its id cannot be reused by another
+        key = ('sampled', id(sampler), N, kmax) + tuple(tuple(interaction[k].shape) for k in fields)
+        g = self._eval_graphs.get(key)
+        own = getattr(interaction, 'layout', None) is not None and positive_i is interaction.interaction.get(m.POS_ITEM_ID)
+        if g is None:
+            if own and all(k in interaction for k in fields):
+                # a packed loader batch: the static buffer takes the batch's own layout, so each replay's input is ONE copy
+                inter = PackedInteraction(torch.empty(interaction.packed.numel(), dtype=torch.int64, device=dev), interaction.layout)
+            elif all(interaction[k].dtype == torch.int64 for k in fields):
+                lay, total = PackedInteraction.layout_of({**{k: interaction[k] for k in fields}, m.POS_ITEM_ID: positive_i})
+                inter = PackedInteraction(torch.empty(total, dtype=torch.int64, device=dev), lay)
+            else:                             # a float field (ACTiSASRec's time stamps): one static tensor per field
+                inter = Interaction({**{k: torch.empty_like(interaction[k], device=dev) for k in fields},
+                                     m.POS_ITEM_ID: torch.empty_like(positive_i, device=dev)})
+            for k in fields:
+                inter[k].copy_(interaction[k])
+            pos = inter[m.POS_ITEM_ID]
+            pos.copy_(positive_i)
+            cand = torch.empty((pos.shape[0], N + 1), dtype=torch.int64, device=dev)
+            side = torch.cuda.Stream()
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):      # warm-up; the sampler's state is put back so the graph starts where eager would
+                snap = sampler.rng.state.clone()
+                for _ in range(2):
+                    self._sampled_body(inter, pos, cand, sampler, kmax)
+                sampler.rng.state.copy_(snap)
+            torch.cuda.current_stream().wait_stream(side)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                rec = self._sampled_body(inter, pos, cand, sampler, kmax)
+            g = dict(graph=graph, pos=pos, rec=rec, inter=inter, cand=cand, fields=fields, sampler=sampler)
+            self._eval_graphs[key] = g
+        assert g['sampler'] is sampler
+        if own and interaction.layout == getattr(g['inter'], 'layout', ()):
+            g['inter'].packed.copy_(interaction.packed, non_blocking=True)
+        else:
+            for k in fields:
+                g['inter'][k].copy_(interaction[k], non_blocking=True)
+            g['pos'].copy_(positive_i, non_blocking=True)
+        g['graph'].replay()
+        if rec_out is not None:
+            rec_out.copy_(g['rec'], non_blocking=True)
+            return rec_out
+        return g['rec'].clone()
+
     @torch.no_grad()
     def evaluate(self, eval_data, load_best_model=True, model_file=None, show_progress=False):
         """trainer.py:964-1019."""
@@ -672,7 +801,8 @@ class ACSASRecTrainer(object):
             self.logger.info('Loading model structure and parameters from {}'.format(checkpoint_file))
         self.model.eval()
         self.tot_item_num = eval_data.dataset.item_num
-        recs = [self.eval_batch(b) for b in eval_data]
+        sampler = getattr(eval_data, 'neg_sampler', None)      # data.NegSampleEvalDataLoader: sampled-candidate evaluation
+        recs = [self.eval_batch(b, neg_sampler=sampler, neg_num=getattr(eval_data, 'neg_num', 0)) for b in eval_data]
         rec = torch.cat(recs, dim=0).cpu().numpy()
         return self.evaluator.evaluate(rec)
 

@@ -457,6 +457,33 @@ int acsr_batch_gather(const int64_t* seqs, const int64_t* lens, const int64_t* t
                       const int64_t* cursor, int64_t n_rows, int B, int L, int64_t* out_packed, void* stream);
 int acsr_cursor_advance(int64_t* cursor, void* stream);
 
+/* ---- negative sampling and sampled-candidate ranking (negsample.cu) ----
+ * acsr_neg_sample replaces recbole/sampler/sampler.py sample_by_user_ids (RecBole 1.0.1's non-repeatable Sampler, as called by
+ * data/dataloader/general_dataloader.py for `neg_sampling` and for `eval_args.mode: uniN / popN`).  negs[m * ld_negs + j],
+ * j < N, is a negative for row m: an item of [1, n_items) outside the user's used set used_items[used_offsets[u] ..
+ * used_offsets[u+1]) (sorted ascending, unique, per user id u = users[row]) and != positives[row] (positives may be NULL).
+ * Uniform (alias_prob == NULL): exactly uniform over that complement, one draw and a binary search per negative.  Popularity
+ * (alias_prob [n_items] float32 / alias_idx [n_items] int64, a Walker alias table of the item counts): alias draws rejected
+ * while they hit the excluded set, at most 16 per negative, after which the uniform-complement draw is taken.  Draws are with
+ * replacement and keyed by Philox4x32-10 (rng->seed, rng->step, rng_stream, row * N + j): advance rng with acsr_rng_advance
+ * for fresh draws.  With perm / cursor (both or neither), row m reads users / positives at perm[cursor[0] * M + m] of n_rows
+ * rows -- the batch acsr_batch_gather writes, when launched between it and acsr_cursor_advance.  A user id outside [0, n_users)
+ * or a user whose complement is empty gets item 0 (never a valid draw).  Graph-capturable. */
+int acsr_neg_sample(const int64_t* users, const int64_t* positives, const int64_t* perm, const int64_t* cursor, int64_t n_rows, int M,
+                    int N, const int64_t* used_offsets, const int64_t* used_items, int64_t n_users, int64_t n_items,
+                    const float* alias_prob, const int64_t* alias_idx, const void* rng, uint32_t rng_stream, int64_t* negs,
+                    int64_t ld_negs, void* stream);
+/* acsr_candidate_rank replaces trainer/trainer.py _neg_sample_batch_eval (predict on the repeated interaction, scatter into a
+ * -inf [B, n_items] matrix) and evaluator/collector.py eval_batch_collect (topk + hit flags) for sampled evaluation.
+ * cand [M, n_cand] int64, column 0 the positive; scores[m, c] = out[m] . table[cand[m, c]] in fp32 (out [M, d], table [V, d],
+ * d a multiple of 4 up to 1024; scores may be NULL).  rank = number of DISTINCT candidates c >= 1 whose score is strictly
+ * greater than the positive's (duplicates collapse as in the scattered matrix; ties count for the positive).
+ * rec [M, kmax+1] int32: rec[m, rank] = 1 when rank < kmax, rec[m, kmax] = 1 (pos_len), else 0.
+ * n_cand <= acsr_candidate_rank_max_candidates() (8192) and kmax <= 1024, else ACSR_ERR_UNSUPPORTED. */
+int acsr_candidate_rank_max_candidates(void);
+int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
+                        int32_t* rec, float* scores, void* stream);
+
 /* ---- K13: fused Adam over one flat fp32 buffer (trainer/trainer.py:614-615,687) ---------
  * torch.optim.Adam semantics (no amsgrad); step_count device int64[1], incremented by the call. */
 int acsr_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,
