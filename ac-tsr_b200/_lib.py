@@ -147,6 +147,13 @@ def _ab_linear_tok_bdrl(a):
     return 4 * (rows * K + 64 * K + 3 * rows * 64 + 2 * rows)
 
 
+def _ab_proj_input_grad(a):
+    # (d_qkv, d_aqk, plane_rows, d_gl, L, Wqkv, Waqk, Wg, d, rows, rows_keep, d_x, ...): d_aq, d_ak, d_mq, d_mk, d_mv (+ d_gl) in,
+    # rows_keep rows of d_mq / d_mk written back, d_x read and written, weights in
+    L, d, rows, keep = (a[4] if a[3] else 0), a[8], a[9], a[10]
+    return 4 * (rows * (5 * d + L) + 2 * keep * d + 2 * rows * d + 5 * d * d + L * d)
+
+
 def _ab_linear_wgrad(a):
     # (dY, X, T, N, K, dW, db, stream)
     T, N, K = a[2], a[3], a[4]
@@ -188,6 +195,7 @@ def _ab_candidate_rank(a):
 
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
 ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_ragged': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl, 'acsr_dense_fwd': _ab_dense_fwd, 'acsr_linear_tok_actbwd': _ab_linear_tok_actbwd,
+              'acsr_proj_input_grad': _ab_proj_input_grad,
               'acsr_linear_wgrad': _ab_linear_wgrad, 'acsr_linear_wgrad_batched': _ab_linear_wgrad_batched,
               'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank}
 

@@ -643,18 +643,16 @@ class FusedTrainStep(object):
             st3 = self._stacked(l)
             gp = ops.gemm_problem
             rows_x = T2 if l > 0 else T                      # below the first layer only the calibrated stream trains anything
-            if self.tc and st3 is not None:
-                ops.linear_tok(lb['d_aqk'], T2, d, st3['Waqk'], d, lb['d_qkv'], d, w_sn=1, w_sk=d, wkb=64 * d, accumulate=True,
-                               batch=2, sx=T2 * d, sw=d * d, sb=0, sy=T2 * d)
-                if gate:
-                    ops.linear_tok(lb['d_gl'], T2, L, layer.gate.weight, d, lb['d_mq'], d, ldx=L, w_sn=1, w_sk=d, wkb=64 * d,
-                                   accumulate=True)
-                # d_x += [d_mq d_mk d_mv] . [Wq; Wk; Wv]: one K = 3d GEMM
-                ops.linear_tok(lb['d_qkv'], rows_x, 3 * d, st3['Wqkv'], d, d_x, d, ldx=d, xkb=T2 * d, w_sn=1, w_sk=d, wkb=d * d,
-                               accumulate=True)
+            if self.tc and st3 is not None and (not gate or L <= d):
+                # d_mq += d_aq.Waq (+ d_gl.Wg), d_mk += d_ak.Wak, d_x += [d_mq d_mk d_mv] . [Wq; Wk; Wv]: one launch.  Only rows
+                # [0,T) of the summed d_mq / d_mk are read afterwards (the Q / K weight gradients): the kernel writes back those.
+                LIB.call('acsr_proj_input_grad', _p(lb['d_qkv']), _p(lb['d_aqk']), T2, _p(lb['d_gl']) if gate else None, L,
+                         _p(st3['Wqkv']), _p(st3['Waqk']), _p(layer.gate.weight) if gate else None, d, rows_x, T, _p(d_x),
+                         self.passes, st)
             else:
-                # any width (K-streamed tcgen05 kernel): d_mq += d_aq.Waq, d_mk += d_ak.Wak in one launch; the gate's d_mq += d_gl.Wg
-                # accumulates into the same rows, so it follows in its own launch; then d_x += sum of the three projections
+                # any width, or a gate wider than the hidden size (K-streamed tcgen05 kernel): d_mq += d_aq.Waq, d_mk += d_ak.Wak in
+                # one launch; the gate's d_mq += d_gl.Wg accumulates into the same rows, so it follows in its own launch; then d_x +=
+                # sum of the three projections
                 ops.gemm_batch([gp(lb['d_aq'], aqt.weight, lb['d_mq'], T2, d, d, b_strides=(1, d, 0, d), accumulate=True),
                                 gp(lb['d_ak'], akt.weight, lb['d_mk'], T2, d, d, b_strides=(1, d, 0, d), accumulate=True)],
                                passes=self.passes)

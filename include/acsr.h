@@ -321,6 +321,15 @@ int acsr_linear_tok_bdrl(const float* X, int64_t ldx, int64_t rows, int K, const
                          const float* res, int64_t res_rows, const float* ln_w, const float* ln_b, float eps,
                          float p_drop, const float* mask, const void* rng, uint32_t rng_stream,
                          float* HZ, float* out, float* stats, int passes, void* stream);
+/* input gradient of a layer's projections in ONE launch (backward of model/layers.py:658-659, 687-689, 887), hidden size d = 64:
+ *   d_mq_tot = d_mq + d_aq.Waq (+ d_gl.Wg) ; d_mk_tot = d_mk + d_ak.Wak ; d_x[r] += d_mq_tot.Wq + d_mk_tot.Wk + d_mv.Wv,  r < rows
+ * (the three acsr_linear_tok launches d_qkv[0:2] += d_aqk.Waqk, d_mq += d_gl.Wg, d_x += d_qkv.Wqkv).  d_qkv [3, plane_rows, 64] =
+ * (d_mq, d_mk, d_mv), d_aqk [2, plane_rows, 64] = (d_aq, d_ak); rows r < rows_keep of d_mq_tot / d_mk_tot are written back into
+ * d_qkv[0] / d_qkv[1], the others are left as they were.  d_gl [plane_rows, L] and Wg [L, 64] (L <= 64) are both NULL without
+ * the gate.  Wqkv [3,64,64], Waqk [2,64,64] row-major [out, in]; d_x [rows, 64] already holds the residual-path gradient. */
+int acsr_proj_input_grad(float* d_qkv, const float* d_aqk, int64_t plane_rows, const float* d_gl, int L, const float* Wqkv,
+                         const float* Waqk, const float* Wg, int d, int64_t rows, int64_t rows_keep, float* d_x, int passes,
+                         void* stream);
 
 /* ---- token-parallel linear layer on tcgen05 (3xTF32):  Y[rows, N] (+)= X[rows, K] . Wt^T + bias,  K == 64 (ABI v1).
  * replaces the forward nn.Linear calls at layers.py:658-659, 680, 687-689, 791 and their input-gradient GEMMs.
