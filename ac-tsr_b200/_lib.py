@@ -141,6 +141,14 @@ def _ab_dense_fwd(a):
     return 4 * (rows * d + min(rows, res_rows) * d + 4 * rows * d + 2 * rows * I + 4 * rows + d * d + 2 * d * I)
 
 
+def _ab_dense_bwd(a):
+    # (d_out, rows, act_rows, res_rows, param_rows, d, I, ...): d_out, the saved z2 / h / hz [., 64], z1 [., I], stats and the residual
+    # in; d_xres, d_ctx [rows, 64] out, d_z2 / d_hz [param_rows, 64] and d_z1 [param_rows, I] out; weights in
+    rows, act_rows, res_rows, keep, d, I = a[1], a[2], a[3], a[4], a[5], a[6]
+    ra = min(rows, act_rows)
+    return 4 * (rows * d + ra * (3 * d + I + 4) + min(rows, res_rows) * d + 2 * rows * d + keep * (2 * d + I) + d * d + 2 * d * I)
+
+
 def _ab_linear_tok_bdrl(a):
     # (X, ldx, rows, K, W, bias, res, res_rows, ...): X, W in; HZ, out, stats out; residual in
     rows, K = a[2], a[3]
@@ -195,7 +203,7 @@ def _ab_candidate_rank(a):
 
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
 ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_ragged': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl, 'acsr_dense_fwd': _ab_dense_fwd, 'acsr_linear_tok_actbwd': _ab_linear_tok_actbwd,
-              'acsr_proj_input_grad': _ab_proj_input_grad,
+              'acsr_proj_input_grad': _ab_proj_input_grad, 'acsr_dense_bwd': _ab_dense_bwd,
               'acsr_linear_wgrad': _ab_linear_wgrad, 'acsr_linear_wgrad_batched': _ab_linear_wgrad_batched,
               'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank}
 

@@ -79,6 +79,9 @@ class FusedTrainStep(object):
         # is serial inside a tile and each per-row epilogue (Philox + LayerNorm / erf, one warp per SM sub-partition) costs microseconds;
         # separate launches spread the same epilogues over more CTAs.  Off by default (ACSR_DENSE_FUSED=1 turns it on).
         self.dense_fused = (self.tc and model.inner_size % 64 == 0 and os.environ.get('ACSR_DENSE_FUSED', '0') == '1')
+        # backward of a layer's dense part (two LayerNorm backwards, the activation backward, three input-gradient GEMMs) as ONE
+        # tcgen05 launch (acsr_dense_bwd: d_a1 / d_z1 stay in tensor memory); ACSR_DENSE_BWD=0: the six launches
+        self.dense_bwd = (self.tc and model.inner_size % 64 == 0 and os.environ.get('ACSR_DENSE_BWD', '1') == '1')
         self.split_wgrad = int(os.environ.get('ACSR_SPLIT_WGRAD', '1'))       # 1: two weight-gradient launches for the first layer (see _backward_branch); 2: every layer
         # CE backward without the [2B,V] gradient matrix (acsr_ce_bwd_dout / _dtable, hidden size 64); ACSR_CE_FUSED_BWD=0 keeps Gt
         self.ce_fused_bwd = model.hidden_size == 64 and os.environ.get('ACSR_CE_FUSED_BWD', '1') == '1'
@@ -373,6 +376,19 @@ class FusedTrainStep(object):
                 dbuf['done'].record(so)
                 dense_ops[l] = dbuf
         b['dense_ops'] = dense_ops
+        bwd_ops = {}
+        if self.dense_bwd and training and not self.fuse_act_bwd:
+            # the same weights transposed for acsr_dense_bwd.  Enqueued ahead of the sequence ordering, whose event the first
+            # attention launch waits for: complete before any backward kernel starts (and static for its PDL chain)
+            for l in range(N):
+                if l == N - 1 and self.compact_last and self.tail_fused:
+                    continue
+                lay = m.trm_encoder.layer[l]
+                dbuf = self._dense_bwd_ops_buffer(l, s, seq.device)
+                LIB.call('acsr_dense_bwd_prep', _p(lay.attack_attention.dense.weight), _p(lay.feed_forward.dense_1.weight),
+                         _p(lay.feed_forward.dense_2.weight), d, I, _p(dbuf), so.cuda_stream)
+                bwd_ops[l] = dbuf
+        b['dense_bwd_ops'] = bwd_ops
         LIB.call('acsr_seq_order', _p(seq, torch.int64), Bs, L, _p(b['order'], torch.int32), so.cuda_stream)
         order_done = torch.cuda.Event()
         order_done.record(so)
@@ -605,11 +621,13 @@ class FusedTrainStep(object):
                     self._wgrad(cb['d_z1'], cb['h'], Bs, ff.dense_1.weight.grad, None, fork, wg)
                     self._wgrad(cb['d_hz'], cb['ctx'], Bs, aa.dense.weight.grad, None, fork, wg)
                 else:
-                    self._post_attn_bwd(layer, cb, cb, dc_out, cb['x'], C, C, Bs, Bs, cb['d_x'], cb['d_ctx'], p_h, rngp, base, act_id, st, fork, wg)
+                    self._post_attn_bwd(layer, cb, cb, dc_out, cb['x'], C, C, Bs, Bs, cb['d_x'], cb['d_ctx'], p_h, rngp, base, act_id, st, fork, wg,
+                                        dops=b['dense_bwd_ops'].get(l))
                     LIB.call('acsr_gather_last_bwd', _p(cb['d_ctx']), _p(ln, torch.int64), Bs, L, d, _p(b['d_ctx'][:T]), _p(b['d_ctx'][T:]), st)
                     LIB.call('acsr_gather_last_bwd', _p(cb['d_x']), _p(ln, torch.int64), Bs, L, d, _p(d_x[:T]), _p(d_x[T:]), st)
             else:
-                self._post_attn_bwd(layer, lb, lb, d_out, x, T2, P, T, T, d_x, b['d_ctx'], p_h, rngp, base, act_id, st, fork, wg, b=b)
+                self._post_attn_bwd(layer, lb, lb, d_out, x, T2, P, T, T, d_x, b['d_ctx'], p_h, rngp, base, act_id, st, fork, wg, b=b,
+                                    dops=b['dense_bwd_ops'].get(l))
             if wg and self.split_wgrad and (l == 0 or self.split_wgrad > 1):
                 # the out-projection / feed-forward weight gradients are complete here: their launch runs on the side stream
                 # under the attention backward, so the launch left for the end of the layer (the projections') is short --
@@ -687,14 +705,29 @@ class FusedTrainStep(object):
         if side is not None:
             main.wait_stream(side)                            # join: every weight gradient of this branch landed
 
-    def _post_attn_bwd(self, layer, bf, gb, d_out, x_res, R2, P, res_rows, w_rows, d_xres, d_ctx, p_h, rngp, base, act_id, st, fork, wg, b=None):
+    def _post_attn_bwd(self, layer, bf, gb, d_out, x_res, R2, P, res_rows, w_rows, d_xres, d_ctx, p_h, rngp, base, act_id, st, fork, wg, b=None,
+                       dops=None):
         """backward of _post_attn_fwd over R2 cotangent rows ([stream 0 ; stream 1]); the saved forward tensors of bf repeat
         with period P, the residual x_res with period res_rows; rows [0, w_rows) (stream 0) feed the parameter gradients.
         Writes the gradient of the attention context to d_ctx and of the residual input to d_xres; weight-gradient problems
-        are appended to wg (launched together at the end of the layer)."""
+        are appended to wg (launched together at the end of the layer).  dops: the layer's weights prepared by acsr_dense_bwd_prep
+        (the whole chain as one launch)."""
         m = self.m
         d, I = m.hidden_size, m.inner_size
         aa, ff = layer.attack_attention, layer.feed_forward
+        if dops is not None:
+            # only rows [0, w_rows) of d_z2 / d_z1 / d_hz leave the SM; the three bias gradients are their column sums, taken by
+            # the weight-gradient launch
+            LIB.call('acsr_dense_bwd', _p(d_out), R2, P, res_rows, w_rows, d, I, act_id, _p(dops), _p(bf['z2']), _p(ff.dense_2.bias),
+                     _p(bf['h']), _p(ff.LayerNorm.weight), _p(bf['st_f']), _p(bf['z1']), _p(ff.dense_1.bias), _p(bf['hz']),
+                     _p(aa.dense.bias), _p(x_res), _p(aa.LayerNorm.weight), _p(bf['st_a']), p_h, _p(bf['m_a']), _p(bf['m_f']), rngp,
+                     base + 3, base + 5, _p(gb['d_z2']), _p(gb['d_z1']), _p(gb['d_hz']), _p(d_xres), _p(d_ctx),
+                     _p(ff.LayerNorm.weight.grad), _p(ff.LayerNorm.bias.grad), _p(aa.LayerNorm.weight.grad),
+                     _p(aa.LayerNorm.bias.grad), self.passes, st)
+            self._wgrad(gb['d_z2'], bf['a1'], w_rows, ff.dense_2.weight.grad, ff.dense_2.bias.grad, fork, wg)
+            self._wgrad(gb['d_z1'], bf['h'], w_rows, ff.dense_1.weight.grad, ff.dense_1.bias.grad, fork, wg)
+            self._wgrad(gb['d_hz'], bf['ctx'], w_rows, aa.dense.weight.grad, aa.dense.bias.grad, fork, wg)
+            return
         d_h = gb['d_h'] if b is None else b['d_h']
         d_a1 = gb['d_a1'] if b is None else b['d_a1']
         gp, ps = ops.gemm_problem, self.passes
@@ -773,6 +806,15 @@ class FusedTrainStep(object):
             # written once per step by acsr_dense_prep, complete (event dependency) before its reader starts: static for the PDL chain
             LIB.query('acsr_register_static', t.data_ptr(), t.numel() * 4)
             self.buf[key] = dict(ops=t)
+        return self.buf[key]
+
+    def _dense_bwd_ops_buffer(self, l, s, dev):
+        key = ('dense_bwd_ops', l, s)
+        if key not in self.buf:
+            t = torch.empty(LIB.query('acsr_dense_bwd_prep_floats', int(self.m.inner_size)), dtype=torch.float32, device=dev)
+            # written once per step by acsr_dense_bwd_prep, complete before its reader starts: static for the PDL chain
+            LIB.query('acsr_register_static', t.data_ptr(), t.numel() * 4)
+            self.buf[key] = t
         return self.buf[key]
 
     def _stacked(self, l):

@@ -436,6 +436,25 @@ int acsr_dense_fwd(const float* ctx, const float* res, int64_t rows, int64_t res
                    const void* rng, uint32_t stream_a, uint32_t stream_f, float* hz, float* st_a, float* h, float* z1, float* a1,
                    float* z2, float* st_f, float* out, int passes, void* stream);
 
+/* ---- backward of that dense part as ONE tcgen05 kernel (hidden size 64, inner size a multiple of 64 up to 256), the chain of two
+ * acsr_bias_dropout_res_ln_bwd calls, acsr_bias_act_bwd and three input-gradient GEMMs:
+ *   d_pre_f = LN_f backward of d_out ; d_z2 = d_pre_f * mask_f ; d_z1 = (d_z2.W2) * act'(z1 + b1) ; d_h = d_pre_f + d_z1.W1 ;
+ *   d_xres = LN_a backward of d_h ; d_hz = d_xres * mask_a ; d_ctx = d_hz.Wo
+ * with the argument meaning of those calls: `rows` cotangent rows; the saved tensors z2, h, st_f, z1 [., I], hz, st_a (and the
+ * explicit masks [., 64]) repeat with period act_rows, x_res with period res_rows; rows < param_rows feed the parameter gradients.
+ * `ops` = the weights pre-split by acsr_dense_bwd_prep (acsr_dense_bwd_prep_floats(I) floats).  Writes d_xres and d_ctx
+ * [rows, 64] (overwritten) and rows < param_rows of d_z2, d_hz [., 64] and d_z1 [., I]; ADDS the LayerNorm weight / bias gradients
+ * of both norms into g_ln*.  The bias gradients of dense_2, dense_1 and the out-projection are left to the weight-gradient launch
+ * (column sums of d_z2, d_z1, d_hz).  Dropout: masks or Philox streams as acsr_bias_dropout_res_ln_bwd. */
+int64_t acsr_dense_bwd_prep_floats(int I);
+int acsr_dense_bwd_prep(const float* Wo, const float* W1, const float* W2, int d, int I, float* ops, void* stream);
+int acsr_dense_bwd(const float* d_out, int64_t rows, int64_t act_rows, int64_t res_rows, int64_t param_rows, int d, int I, int act,
+                   const float* ops, const float* z2, const float* b2, const float* h, const float* lnF_w, const float* st_f,
+                   const float* z1, const float* b1, const float* hz, const float* bo, const float* x_res, const float* lnA_w,
+                   const float* st_a, float p_drop, const float* mask_a, const float* mask_f, const void* rng, uint32_t stream_a,
+                   uint32_t stream_f, float* d_z2, float* d_z1, float* d_hz, float* d_xres, float* d_ctx, float* g_lnF_w,
+                   float* g_lnF_b, float* g_lnA_w, float* g_lnA_b, int passes, void* stream);
+
 /* ---- loss_type BPR (model/sequential_recommender/acsasrec.py:109-116, model/loss.py:21-47) ----
  * x_m = out_m . (E[pos_m] - E[neg_m]); row_loss[m] = -log(gamma + sigmoid(x_m)); loss[g] = mean over row group g
  * (M rows in n_groups equal groups: [calibrated ; attacked] in the fused step).  row_x [M] is saved for the backward. */
