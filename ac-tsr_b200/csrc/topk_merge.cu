@@ -9,9 +9,12 @@
 namespace acsr {
 
 constexpr int kMergeThreads = 256;
-constexpr int kMergeMaxCand = 56 * 1024;      // 32-bit keys of one row in shared memory (224 KB)
 constexpr int kMergeMaxK = 64;
 constexpr int kFastCap = 512;        // candidates the fast path sorts (P/2 <= 256 threads)
+// The 32-bit keys of one row (dynamic shared memory) and the kernel's static arrays (histograms, scan, fast-path candidates:
+// 15,904 bytes by ptxas -v) share the 227 KB a block may use; a key count beyond that cannot be launched at all.
+constexpr int kMergeStaticBytes = 16 * 1024;
+constexpr int kMergeMaxCand = (227 * 1024 - kMergeStaticBytes) / 4;     // 54,016 keys
 
 __device__ __forceinline__ unsigned f2key(float v) {        // larger float <-> larger unsigned
   const unsigned u = __float_as_uint(v);

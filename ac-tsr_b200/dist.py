@@ -18,7 +18,7 @@ Two storage modes:
               tile inside the two kernels (acsr_ce_bwd_dout / _dtable: no gradient matrix in HBM); reduce-scatter(sum) of
               d_out; dE_shard needs no traffic.
   evaluation: all-gather `out` -> fused top-k on the shard (indices offset by the shard start, column 0 skipped on shard 0)
-              -> all-gather of the partial lists -> merge of the rank's own rows.
+              -> merge of the shard's chunk lists into one list per row -> all-gather of those lists -> merge of the rank's own rows.
 
 The collective plumbing is backend-agnostic: `compute` supplies the local kernels (CUDA ops by default; the gloo CPU tests
 inject torch restatements), so world_size-2 tests run without a GPU.  Nothing here allocates by value from the host inside the
@@ -202,17 +202,14 @@ class VocabParallel(object):
 
     # ------------------------------------------------------------------------------------------
     def full_sort_topk(self, out_local, table, k, positive_local=None):
-        """all-gather of partial top-k lists (north_star eval path) -> (val [R,k], idx [R,k], rec|None)."""
+        """all-gather of partial top-k lists (north_star eval path) -> (val [R,k], idx [R,k], rec|None).  Each rank first merges
+        its shard's per-chunk lists into one list per row, so the final merge sees W*k candidates however many chunks a shard
+        runs (W * 148 chunk lists of k would exceed the merge's capacity)."""
         R, d = out_local.shape
         out_all = self._all_gather(out_local).view(self.world * R, d)
-        E_s = self.shard(table)
-        pv, pi = self.compute.topk_partial(out_all, E_s, k, self.lo, self.lo == 0)   # [W*R, nc, k]
-        ncmax = self._ncmax(self.world * R)
-        if pv.shape[1] < ncmax:
-            padn = ncmax - pv.shape[1]
-            pv = torch.cat((pv, pv.new_full((pv.shape[0], padn, k), -float('inf'))), 1)
-            pi = torch.cat((pi, pi.new_full((pi.shape[0], padn, k), -1)), 1)
+        pv, pi = self.compute.topk_partial(out_all, self.shard(table), k, self.lo, self.lo == 0)   # [W*R, nc, k]
+        sv, si, _ = self.compute.topk_merge(pv, pi, k, None)                                      # [W*R, k]
         sl = slice(self.rank * R, (self.rank + 1) * R)
-        mv = self._all_gather(pv)[:, sl].permute(1, 0, 2, 3).reshape(R, self.world * ncmax, k).contiguous()
-        mi = self._all_gather(pi)[:, sl].permute(1, 0, 2, 3).reshape(R, self.world * ncmax, k).contiguous()
+        mv = self._all_gather(sv)[:, sl].permute(1, 0, 2).contiguous()                             # [R, W, k]
+        mi = self._all_gather(si)[:, sl].permute(1, 0, 2).contiguous()
         return self.compute.topk_merge(mv, mi, k, positive_local)
