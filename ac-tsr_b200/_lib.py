@@ -201,11 +201,17 @@ def _ab_candidate_rank(a):
     return 4 * M * d + M * C * (8 + 4 * d) + 4 * M * (kmax + 1) + (4 * M * C if a[9] else 0)
 
 
+def _ab_candidate_rank_counts(a):
+    # (out, table, V, d, cand, M, n_cand, kmax, rec, scores, counts, stream): acsr_candidate_rank + three counts per row out
+    return _ab_candidate_rank(a) + 12 * a[5]
+
+
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
 ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_ragged': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl, 'acsr_dense_fwd': _ab_dense_fwd, 'acsr_linear_tok_actbwd': _ab_linear_tok_actbwd,
               'acsr_proj_input_grad': _ab_proj_input_grad, 'acsr_dense_bwd': _ab_dense_bwd,
               'acsr_linear_wgrad': _ab_linear_wgrad, 'acsr_linear_wgrad_batched': _ab_linear_wgrad_batched,
-              'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank}
+              'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank,
+              'acsr_candidate_rank_counts': _ab_candidate_rank_counts}
 
 
 class KernelTimer:

@@ -228,16 +228,19 @@ class AcBERT4Rec(SequentialRecommender):
         B = att.shape[0]
         return both[:B], both[B:]
 
-    def full_sort_topk(self, interaction, k, positive=None):
-        """fused scores -> scores[:,0] = -inf -> top-k -> hit flags of the calibrated stream (trainer.py:941-942, collector.py:145-153)"""
+    def full_sort_topk(self, interaction, k, positive=None, counts=False):
+        """fused scores -> scores[:,0] = -inf -> top-k -> hit flags of the calibrated stream (trainer.py:941-942, collector.py:145-153);
+        counts=True: + the positive's rank counts [B, 2] (ops.full_sort_topk)"""
         _, cal = self._test_outputs(interaction)
-        return ops.full_sort_topk(cal.contiguous(), self.item_embedding.weight[:self.n_items], k, positive, self.logits_passes)
+        return ops.full_sort_topk(cal.contiguous(), self.item_embedding.weight[:self.n_items], k, positive, self.logits_passes,
+                                  counts=counts)
 
-    def sampled_topk(self, interaction, candidates, k, positive=None):
+    def sampled_topk(self, interaction, candidates, k, positive=None, counts=False):
         """sampled-candidate ranking of the calibrated stream (candidates [B, 1+N], positive in column 0, written there from
-        `positive` when given) over the table without the mask-token row -> (scores [B, 1+N], rec_topk [B, k+1])"""
+        `positive` when given) over the table without the mask-token row -> (scores [B, 1+N], rec_topk [B, k+1]) (+ counts [B, 3]
+        of ops.candidate_rank with counts=True)"""
         if positive is not None:
             candidates[:, 0].copy_(positive)
         _, cal = self._test_outputs(interaction)
-        rec, scores = ops.candidate_rank(cal, self.item_embedding.weight[:self.n_items], candidates, k, want_scores=True)
-        return scores, rec
+        r = ops.candidate_rank(cal, self.item_embedding.weight[:self.n_items], candidates, k, want_scores=True, want_counts=counts)
+        return (r[1], r[0]) + tuple(r[2:])

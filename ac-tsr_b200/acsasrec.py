@@ -207,9 +207,10 @@ class ACSASRec(SequentialRecommender):
         scores = ops.logits_scores(out, self.item_embedding.weight, self.logits_passes)
         return None, scores
 
-    def full_sort_topk(self, interaction, k, positive=None):
+    def full_sort_topk(self, interaction, k, positive=None, counts=False):
         """Fused replacement of full_sort_predict + `scores[:,0]=-inf` + topk + hit flags
-        (trainer.py:941-942, collector.py:145-153): -> (topk_scores[B,k], topk_idx[B,k], rec_topk[B,k+1]|None)."""
+        (trainer.py:941-942, collector.py:145-153): -> (topk_scores[B,k], topk_idx[B,k], rec_topk[B,k+1]|None), and with
+        counts=True the positive's rank counts [B, 2] (ops.full_sort_topk) as a fourth entry."""
         item_seq = interaction[self.ITEM_SEQ]
         item_seq_len = interaction[self.ITEM_SEQ_LEN]
         # programmatic dependent launch between the eval kernels (prologues overlap the previous kernel's tail), as in the training step
@@ -218,17 +219,17 @@ class ACSASRec(SequentialRecommender):
             out, _ = self._encode(item_seq, item_seq_len, need_attacked=False)
             vp = getattr(self, '_vp', None)
             if vp is not None:                        # vocab-parallel: partial top-k per shard, all-gather, merge (dist.py)
-                return vp.full_sort_topk(out, self.item_embedding.weight, k, positive)
-            return ops.full_sort_topk(out, self.item_embedding.weight, k, positive, self.logits_passes)
+                return vp.full_sort_topk(out, self.item_embedding.weight, k, positive, counts=counts)
+            return ops.full_sort_topk(out, self.item_embedding.weight, k, positive, self.logits_passes, counts=counts)
         finally:
             if was is not None:
                 ops.LIB.query('acsr_set_pdl', was)
 
-    def sampled_topk(self, interaction, candidates, k, positive=None):
+    def sampled_topk(self, interaction, candidates, k, positive=None, counts=False):
         """Sampled-candidate ranking (`eval_args.mode: uniN / popN`; trainer.py _neg_sample_batch_eval + collector.py
         eval_batch_collect): candidates [B, 1+N] int64 with the positive in column 0 (written there from `positive` when
         given).  Encodes each sequence once (the reference predicts on the interaction repeated 1+N times) and ranks the
-        calibrated scores -> (scores [B, 1+N], rec_topk [B, k+1])."""
+        calibrated scores -> (scores [B, 1+N], rec_topk [B, k+1]), and with counts=True the counts [B, 3] of ops.candidate_rank."""
         vp = getattr(self, '_vp', None)
         if vp is not None and vp.sharded:
             raise ValueError('sampled evaluation is not implemented for a vocab-sharded item table')
@@ -237,8 +238,8 @@ class ACSASRec(SequentialRecommender):
         was = ops.LIB.query('acsr_set_pdl', 1) if self._eval_pdl else None
         try:
             out, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], need_attacked=False)
-            rec, scores = ops.candidate_rank(out, self.item_embedding.weight, candidates, k, want_scores=True)
-            return scores, rec
+            r = ops.candidate_rank(out, self.item_embedding.weight, candidates, k, want_scores=True, want_counts=counts)
+            return (r[1], r[0]) + tuple(r[2:])
         finally:
             if was is not None:
                 ops.LIB.query('acsr_set_pdl', was)

@@ -201,22 +201,23 @@ class ACSSEPT(SequentialRecommender):
         both += self._user_term(out, torch.cat((ut, ut))).view(-1, 1)
         return both[:B], both[B:]
 
-    def full_sort_topk(self, interaction, k, positive=None):
+    def full_sort_topk(self, interaction, k, positive=None, counts=False):
         """fused scores -> scores[:,0] = -inf -> top-k -> hit flags of the calibrated stream (trainer.py:941-942,
-        collector.py:145-153).  The user term is added to the k returned scores; it cannot change their order."""
+        collector.py:145-153).  The user term is added to the k returned scores; it cannot change their order.  counts=True: + the
+        positive's rank counts [B, 2] (ops.full_sort_topk), taken on the item part of the score for the same reason."""
         item_seq = interaction[self.ITEM_SEQ]
         user_id = interaction[self.USER_ID]
         cal, _ = self._encode(item_seq, interaction[self.ITEM_SEQ_LEN], user_id, need_attacked=False)
-        val, idx, rec = ops.full_sort_topk(self._item_part(cal), self.item_embedding.weight, k, positive, self.logits_passes)
-        return val + self._user_term(cal, self.user_test_embedding(user_id)).view(-1, 1), idx, rec
+        r = ops.full_sort_topk(self._item_part(cal), self.item_embedding.weight, k, positive, self.logits_passes, counts=counts)
+        return (r[0] + self._user_term(cal, self.user_test_embedding(user_id)).view(-1, 1),) + tuple(r[1:])
 
-    def sampled_topk(self, interaction, candidates, k, positive=None):
+    def sampled_topk(self, interaction, candidates, k, positive=None, counts=False):
         """sampled-candidate ranking of the calibrated stream (candidates [B, 1+N], positive in column 0, written there from
         `positive` when given) -> (scores [B, 1+N], rec_topk [B, k+1]).  The user term is added to the returned scores; it is
-        the same for every candidate of a row and cannot change the rank."""
+        the same for every candidate of a row and cannot change the rank.  counts=True: + counts [B, 3] of ops.candidate_rank."""
         if positive is not None:
             candidates[:, 0].copy_(positive)
         user_id = interaction[self.USER_ID]
         cal, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], user_id, need_attacked=False)
-        rec, scores = ops.candidate_rank(self._item_part(cal), self.item_embedding.weight, candidates, k, want_scores=True)
-        return scores + self._user_term(cal, self.user_test_embedding(user_id)).view(-1, 1), rec
+        r = ops.candidate_rank(self._item_part(cal), self.item_embedding.weight, candidates, k, want_scores=True, want_counts=counts)
+        return (r[1] + self._user_term(cal, self.user_test_embedding(user_id)).view(-1, 1), r[0]) + tuple(r[2:])

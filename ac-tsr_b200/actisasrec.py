@@ -162,19 +162,20 @@ class ACTiSASRec(SequentialRecommender):
         both = ops.logits_scores(out, self.item_embedding.weight, self.logits_passes)
         return both[:B], both[B:]
 
-    def full_sort_topk(self, interaction, k, positive=None):
-        """fused scores -> scores[:,0] = -inf -> top-k -> hit flags of the calibrated stream (trainer.py:941-942, collector.py:145-153)"""
+    def full_sort_topk(self, interaction, k, positive=None, counts=False):
+        """fused scores -> scores[:,0] = -inf -> top-k -> hit flags of the calibrated stream (trainer.py:941-942, collector.py:145-153);
+        counts=True: + the positive's rank counts [B, 2] (ops.full_sort_topk)"""
         item_seq = interaction[self.ITEM_SEQ]
         time_matrix = self.get_time_matrix(interaction[self.timestamp])
         cal, _ = self._encode(item_seq, interaction[self.ITEM_SEQ_LEN], time_matrix, need_attacked=False)
-        return ops.full_sort_topk(cal.contiguous(), self.item_embedding.weight, k, positive, self.logits_passes)
+        return ops.full_sort_topk(cal.contiguous(), self.item_embedding.weight, k, positive, self.logits_passes, counts=counts)
 
-    def sampled_topk(self, interaction, candidates, k, positive=None):
+    def sampled_topk(self, interaction, candidates, k, positive=None, counts=False):
         """sampled-candidate ranking of the calibrated stream (candidates [B, 1+N], positive in column 0, written there from
-        `positive` when given) -> (scores [B, 1+N], rec_topk [B, k+1])"""
+        `positive` when given) -> (scores [B, 1+N], rec_topk [B, k+1]) (+ counts [B, 3] of ops.candidate_rank with counts=True)"""
         if positive is not None:
             candidates[:, 0].copy_(positive)
         time_matrix = self.get_time_matrix(interaction[self.timestamp])
         cal, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], time_matrix, need_attacked=False)
-        rec, scores = ops.candidate_rank(cal, self.item_embedding.weight, candidates, k, want_scores=True)
-        return scores, rec
+        r = ops.candidate_rank(cal, self.item_embedding.weight, candidates, k, want_scores=True, want_counts=counts)
+        return (r[1], r[0]) + tuple(r[2:])

@@ -14,7 +14,8 @@ constexpr int kTcThreads = 320;
 constexpr int kTmemCols = 128;         // 2 accumulator stages x 64 columns
 constexpr int kMaxTopK = 64;
 
-enum { MODE_STORE = 0, MODE_CE = 1, MODE_GRAD = 2, MODE_TOPK = 3, MODE_LINEAR = 4 };
+// MODE_TOPK_RANK: MODE_TOPK that also counts, per row, the scores above and equal to the positive's (GAUC's average rank)
+enum { MODE_STORE = 0, MODE_CE = 1, MODE_GRAD = 2, MODE_TOPK = 3, MODE_LINEAR = 4, MODE_TOPK_RANK = 5 };
 
 struct LogitsParams {
   const float* out;      // [M,64]
@@ -44,6 +45,11 @@ struct LogitsParams {
   const float* bias;
   int accumulate;
   long long b_out, b_table, b_bias, b_C;   // per-problem strides of a batched launch (blockIdx.y)
+  // TOPK_RANK: per (row, chunk) the number of items scoring > rank_score[row] and == rank_score[row], columns 0 (when skipped) and
+  // rank_pos[row] - idx_offset excluded -> rank_counts [M, n_slots, 2]
+  const long long* rank_pos;
+  const float* rank_score;
+  int* rank_counts;
 };
 
 // grid plan shared by both paths: [m_tile(128 rows), n_chunk] CTAs, about one per SM

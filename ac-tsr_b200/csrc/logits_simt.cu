@@ -49,6 +49,7 @@ template <int MODE>
 __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const LogitsParams p, const int d) {
   pdl_launch_dependents();
   pdl_wait();
+  constexpr bool kTopk = MODE == MODE_TOPK || MODE == MODE_TOPK_RANK, kRank = MODE == MODE_TOPK_RANK;
   extern __shared__ __align__(16) float smem_f[];
   SimtSmem sm;
   sm.As = smem_f;
@@ -56,7 +57,7 @@ __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const Logi
   sm.pair = sm.Bs + kSimtKC * kBN;
   sm.cnts = reinterpret_cast<int*>(sm.pair + 2 * kBM);
   sm.lval = reinterpret_cast<float*>(sm.cnts + kBM);
-  sm.lidx = reinterpret_cast<int*>(sm.lval + (MODE == MODE_TOPK ? p.k * kSimtThreads : 0));
+  sm.lidx = reinterpret_cast<int*>(sm.lval + (kTopk ? p.k * kSimtThreads : 0));
 
   const int tid = threadIdx.x;
   const int row = tid & (kBM - 1), half = tid >> 7;
@@ -74,6 +75,10 @@ __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const Logi
   long long g_tgt = -1;
   int cnt = 0, minpos = 0;                      // MODE_TOPK
   float thr = -INFINITY;
+  float r_s = INFINITY;                         // MODE_TOPK_RANK: the positive's score, its local column, this thread's counts
+  long long r_pl = -1;
+  int r_gt = 0, r_eq = 0;
+  if (kRank && row_ok) { r_s = p.rank_score[grow]; r_pl = p.rank_pos[grow] - p.idx_offset; }
   if (MODE == MODE_GRAD && row_ok) { g_lse = p.lse[grow]; g_scale = p.row_scale[grow]; g_tgt = p.target[grow]; }
 
   float4 pa[4], pb[2];
@@ -177,8 +182,16 @@ __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const Logi
         run_s = run_s * __expf(run_m - nm) + s;
         run_m = nm;
       }
-    } else {   // MODE_TOPK
+    } else {   // MODE_TOPK / MODE_TOPK_RANK
       const int k = p.k;
+      if (kRank) {
+#pragma unroll
+        for (int i = 0; i < 32; ++i) {
+          const bool ok = i < nvalid && !(p.skip_col0 && c0 + i == 0) && c0 + i != r_pl;
+          r_gt += ok && acc[i] > r_s;
+          r_eq += ok && acc[i] == r_s;
+        }
+      }
 #pragma unroll
       for (int i = 0; i < 32; ++i) {
         const float x = acc[i];
@@ -201,10 +214,15 @@ __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const Logi
       o[0] = nm; o[1] = s;
     }
   }
-  if (MODE == MODE_TOPK) {
-    if (half == 1) sm.cnts[row] = cnt;
+  if (kTopk) {
+    int* rpair = reinterpret_cast<int*>(sm.pair);   // MODE_TOPK_RANK: half 1's two counts (the CE hand-over slots are free here)
+    if (half == 1) {
+      sm.cnts[row] = cnt;
+      if (kRank) { rpair[2 * row] = r_gt; rpair[2 * row + 1] = r_eq; }
+    }
     __syncthreads();
     if (half == 0) {
+      if (kRank) { r_gt += rpair[2 * row]; r_eq += rpair[2 * row + 1]; }
       const int k = p.k, oc = sm.cnts[row], oslot = tid + kBM;
       for (int s = 0; s < oc; ++s) {
         const float x = sm.lval[s * kSimtThreads + oslot];
@@ -223,6 +241,12 @@ __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const Logi
           long long* pi = p.pidx + ((long long)grow * p.n_slots + c) * k;
           for (int s = 0; s < k; ++s) { pv[s] = -INFINITY; pi[s] = -1; }
         }
+        if (kRank) {
+          int* rc = p.rank_counts + (long long)grow * p.n_slots * 2;
+          rc[2 * chunk] = r_gt;
+          rc[2 * chunk + 1] = r_eq;
+          for (int c = p.n_chunks + chunk; c < p.n_slots; c += p.n_chunks) { rc[2 * c] = 0; rc[2 * c + 1] = 0; }
+        }
       }
     }
   }
@@ -231,9 +255,10 @@ __global__ void __launch_bounds__(kSimtThreads, 1) logits_simt_kernel(const Logi
 template <int MODE>
 static int launch_simt(LogitsParams& p, int d, cudaStream_t st, const char* who) {
   logits_plan(p);
-  if (MODE == MODE_TOPK) logits_plan_topk(p);
+  constexpr bool kTopk = MODE == MODE_TOPK || MODE == MODE_TOPK_RANK;
+  if (kTopk) logits_plan_topk(p);
   size_t smem = (size_t)(kSimtKC * kBM + kSimtKC * kBN + 2 * kBM + kBM) * 4;
-  if (MODE == MODE_TOPK) smem += (size_t)2 * p.k * kSimtThreads * 4;
+  if (kTopk) smem += (size_t)2 * p.k * kSimtThreads * 4;
   cudaError_t e = cudaFuncSetAttribute(logits_simt_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) { set_error("%s: smem attr: %s", who, cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
   launch_pdl(logits_simt_kernel<MODE>, dim3(p.m_tiles * p.n_chunks), dim3(kSimtThreads), smem, st, p, d);
@@ -250,6 +275,7 @@ int launch_logits_simt(int mode, LogitsParams& p, int d, cudaStream_t st, const 
     case MODE_CE: return launch_simt<MODE_CE>(p, d, st, who);
     case MODE_GRAD: return launch_simt<MODE_GRAD>(p, d, st, who);
     case MODE_TOPK: return launch_simt<MODE_TOPK>(p, d, st, who);
+    case MODE_TOPK_RANK: return launch_simt<MODE_TOPK_RANK>(p, d, st, who);
   }
   set_error("%s: bad mode", who);
   return ACSR_ERR_ARG;

@@ -24,13 +24,14 @@ namespace acsr {
 
 template <int MODE>
 struct TcCfg {
-  static constexpr int kStages = MODE == MODE_TOPK ? 2 : 4;
+  static constexpr bool kTopkMode = MODE == MODE_TOPK || MODE == MODE_TOPK_RANK;
+  static constexpr int kStages = kTopkMode ? 2 : 4;
   static constexpr int kAbytes = kBM * kD * 4;          // 32 KB per (hi|lo)
   static constexpr int kBbytes = kBN * kD * 4;          // 16 KB per (hi|lo) per buffer
   // MODE_TOPK keeps the stationary tile of `out` in TENSOR MEMORY (hi / lo halves written once with tcgen05.st; the MMAs take
   // it as their A operand, TS form): its shared memory goes to a second set of candidate lists, so that the top-k epilogue --
   // the bottleneck of the kernel, one thread per logits row -- runs on eight warps like the CE epilogue.
-  static constexpr bool kATmem = MODE == MODE_TOPK;
+  static constexpr bool kATmem = kTopkMode;
   static constexpr int kOffAhi = 0;
   static constexpr int kOffAlo = kOffAhi + (kATmem ? 0 : kAbytes);
   static constexpr int kOffBhi = kOffAlo + (kATmem ? 0 : kAbytes);      // [2]
@@ -38,16 +39,17 @@ struct TcCfg {
   static constexpr int kOffStg = kOffBlo + 2 * kBbytes;  // [kStages]
   static constexpr int kOffTopk = kOffStg + kStages * kBbytes;
   static constexpr int kListBytes = 2 * kMaxTopK * kBM * 4;              // values + indices of one warp set: 64 KB
-  static constexpr int kTopkBytes = MODE == MODE_TOPK ? 2 * kListBytes : 0;
+  static constexpr int kTopkBytes = kTopkMode ? 2 * kListBytes : 0;
   // MODE_CE / MODE_TOPK: the epilogue is instruction-issue / latency bound (one thread per logits row), so it runs on EIGHT warps,
   // two per TMEM lane quarter, each owning one 32-column half of every tile; the halves meet once, at the end, through kOffPair
-  static constexpr int kEpiWarps = (MODE == MODE_CE || MODE == MODE_TOPK) ? 8 : 4;
+  static constexpr int kEpiWarps = (MODE == MODE_CE || kTopkMode) ? 8 : 4;
   // Two MMA-issuing threads (warp 1: even tiles, the last warp: odd tiles -- each owns one operand buffer and one accumulator
   // stage): a thread issues one 128 x 64 x 8 TF32 MMA every ~90 cycles against a 32-cycle tensor floor (scripts/umma_rate.py)
   static constexpr int kIssuer2 = 6 + kEpiWarps;
   static constexpr int kThreads = 192 + 32 * kEpiWarps + 32;
   static constexpr int kOffPair = kOffTopk + kTopkBytes;
-  static constexpr int kPairBytes = (MODE == MODE_CE || MODE == MODE_TOPK) ? kBM * 8 : 0;
+  // MODE_TOPK_RANK also hands the upper warp set's two rank counts over: [128] candidate counts, then [128] int2
+  static constexpr int kPairBytes = MODE == MODE_TOPK_RANK ? kBM * 12 : (MODE == MODE_CE || kTopkMode) ? kBM * 8 : 0;
   static constexpr int kOffBar = kOffPair + kPairBytes;
   static constexpr int kNumBars = 2 * kStages + 2 + 2 + 2 + 2;
   static constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 16;
@@ -89,6 +91,7 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
   pdl_launch_dependents();
   pdl_wait();
   using Cfg = TcCfg<MODE>;
+  constexpr bool kTopk = Cfg::kTopkMode, kRank = MODE == MODE_TOPK_RANK;
   extern __shared__ __align__(128) uint8_t smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m_tile = blockIdx.x % p.m_tiles;
@@ -261,13 +264,18 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
     float run_m = -INFINITY, run_s = 0.f;         // MODE_CE
     float g_lse = 0.f, g_scale = 0.f;             // MODE_GRAD
     long long g_tgt = -1;
-    const int lhalf = MODE == MODE_TOPK ? half : 0;                          // MODE_TOPK: each warp set keeps its own candidate lists
+    const int lhalf = kTopk ? half : 0;                          // MODE_TOPK: each warp set keeps its own candidate lists
     float* lval = reinterpret_cast<float*>(smem + Cfg::kOffTopk + lhalf * Cfg::kListBytes);           // [k][128]
     int* lidx = reinterpret_cast<int*>(smem + Cfg::kOffTopk + lhalf * Cfg::kListBytes + kMaxTopK * kBM * 4);
     int cnt = 0, minpos = 0, npend = 0;
     float thr = -INFINITY;
     float gb = -INFINITY;                         // MODE_TOPK: lower bound of the row's overall k-th best score, from p.row_bound
     float rmax = -INFINITY, rmax_pub = -INFINITY;  // best score of this CTA's stream for the row, and the value last published
+    // MODE_TOPK_RANK: the positive's score (+inf on rows past M: nothing counted), its local column, and this stream's counts
+    float r_s = INFINITY;
+    long long r_pl = -1;
+    int r_gt = 0, r_eq = 0;
+    if (kRank && row_ok) { r_s = p.rank_score[grow]; r_pl = p.rank_pos[grow] - p.idx_offset; }
     if (MODE == MODE_GRAD && row_ok) { g_lse = p.lse[grow]; g_scale = p.row_scale[grow]; g_tgt = p.target[grow]; }
     float lin_bias = 0.f;
     if (MODE == MODE_LINEAR && row_ok && p.bias != nullptr) lin_bias = p.bias[blockIdx.y * p.b_bias + grow];
@@ -277,7 +285,7 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
       const long long n0 = (long long)(chunk + it * p.n_chunks) * kBN;
       mbar_wait(tm_full + ob, ph);
       tc_fence_after();
-      if (MODE == MODE_TOPK && p.row_bound != nullptr && row_ok && (it < 8 ? (it & 3) == 1 : (it & 31) == 9)) {
+      if (kTopk && p.row_bound != nullptr && row_ok && (it < 8 ? (it & 3) == 1 : (it & 31) == 9)) {
         // Every warp set of every CTA of this row tile publishes the best score of its own stream (slot [2 chunk + half][row]).
         // Those are 2 n_chunks DIFFERENT catalogue items, so once >= k of them are known, their minimum is a lower bound of the row's overall k-th best:
         // a score at or below it cannot make the top-k and never touches the candidate list.  (Each stream's own k-th best is a far
@@ -389,6 +397,17 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
 #pragma unroll
           for (int i = 1; i < 32; ++i) cmax = fmaxf(cmax, v[i]);
           rmax = fmaxf(rmax, cmax);
+          if (kRank && cmax >= r_s) {
+            // every score of every tile is counted here, before the bound / threshold tests below may skip the tile; excluded
+            // columns are -inf already.  A chunk whose maximum is below s_pos holds nothing to count.
+#pragma unroll
+            for (int i = 0; i < 32; ++i) { r_gt += v[i] > r_s; r_eq += v[i] == r_s; }
+            if (r_pl >= c0 && r_pl < c0 + 32) {                  // the positive's own score, however this path rounded it
+#pragma unroll
+              for (int i = 0; i < 32; ++i)
+                if (c0 + i == r_pl) { r_gt -= v[i] > r_s; r_eq -= v[i] == r_s; }
+            }
+          }
           auto drain = [&]() {
             while (__any_sync(0xffffffffu, npend > 0)) {
               if (npend > 0) {
@@ -430,7 +449,7 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
       }
       tc_fence_before();
       mbar_arrive(tm_empty + ob);
-      if (MODE == MODE_TOPK && p.row_bound != nullptr && row_ok && rmax > rmax_pub) {
+      if (kTopk && p.row_bound != nullptr && row_ok && rmax > rmax_pub) {
         __stcg(p.row_bound + (long long)(2 * chunk + half) * p.M + grow, bound_enc(rmax));
         rmax_pub = rmax;
       }
@@ -450,12 +469,17 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
         o[0] = nm; o[1] = s;
       }
     }
-    if (MODE == MODE_TOPK) {
+    if (kTopk) {
       // the two warp sets of a row meet once: the upper set's candidates are inserted into the lower set's list
       int* pcnt = reinterpret_cast<int*>(smem + Cfg::kOffPair);
-      if (half == 1) pcnt[row] = cnt;
+      int2* prank = reinterpret_cast<int2*>(smem + Cfg::kOffPair + kBM * 4);
+      if (half == 1) {
+        pcnt[row] = cnt;
+        if (kRank) prank[row] = make_int2(r_gt, r_eq);
+      }
       asm volatile("bar.sync 1, %0;" ::"n"(32 * Cfg::kEpiWarps) : "memory");
       if (half == 0) {
+        if (kRank) { const int2 o = prank[row]; r_gt += o.x; r_eq += o.y; }
         const int cnt1 = pcnt[row];
         const float* oval = reinterpret_cast<const float*>(smem + Cfg::kOffTopk + Cfg::kListBytes);
         const int* oidx = reinterpret_cast<const int*>(smem + Cfg::kOffTopk + Cfg::kListBytes + kMaxTopK * kBM * 4);
@@ -465,7 +489,7 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
         }
       }
     }
-    if (MODE == MODE_TOPK && row_ok && half == 0) {
+    if (kTopk && row_ok && half == 0) {
       float* ov = p.pval + ((long long)grow * p.n_slots + chunk) * p.k;
       long long* oi = p.pidx + ((long long)grow * p.n_slots + chunk) * p.k;
       for (int s = 0; s < p.k; ++s) {
@@ -478,6 +502,12 @@ __global__ void __launch_bounds__(TcCfg<MODE>::kThreads, 1) logits_tc_kernel(con
         float* pv = p.pval + ((long long)grow * p.n_slots + c) * p.k;
         long long* pi = p.pidx + ((long long)grow * p.n_slots + c) * p.k;
         for (int s = 0; s < p.k; ++s) { pv[s] = -INFINITY; pi[s] = -1; }
+      }
+      if (kRank) {                                   // plain stores, one slot per (row, chunk): no atomics, deterministic
+        int* rc = p.rank_counts + (long long)grow * p.n_slots * 2;
+        rc[2 * chunk] = r_gt;
+        rc[2 * chunk + 1] = r_eq;
+        for (int c = p.n_chunks + chunk; c < p.n_slots; c += p.n_chunks) { rc[2 * c] = 0; rc[2 * c + 1] = 0; }
       }
     }
   }
@@ -515,6 +545,24 @@ __global__ void __launch_bounds__(256) ce_rows_kernel(const float* __restrict__ 
     for (int j = lane; j < d; j += 32) dot = fmaf(out[(long long)m * d + j], table[t * d + j], dot);
   dot = warp_sum(dot);
   if (lane == 0) { lse[m] = l; tgt_logit[m] = dot; row_loss[m] = l - dot; }
+}
+
+// dot[m] = out[m] . table[ids[m] - idx_offset] when that row lives in this table (shard), else 0: the target logit of ce_rows_kernel
+// on its own, in the same fixed fp32 order (lane-strided FMAs, then the warp sum), so the shards' answers can be summed
+__global__ void __launch_bounds__(256) row_dot_kernel(const float* __restrict__ out, const float* __restrict__ table,
+                                                      const long long* __restrict__ ids, int M, int d, long long V, long long idx_offset,
+                                                      float* __restrict__ dot) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int m = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (m >= M) return;
+  const long long t = ids[m] - idx_offset;
+  float acc = 0.f;
+  if (t >= 0 && t < V)
+    for (int j = lane; j < d; j += 32) acc = fmaf(out[(long long)m * d + j], table[t * d + j], acc);
+  acc = warp_sum(acc);
+  if (lane == 0) dot[m] = acc;
 }
 
 __global__ void __launch_bounds__(256) ce_mean_kernel(const float* __restrict__ row_loss, int M, int n_groups, float* __restrict__ loss) {
@@ -634,7 +682,7 @@ static int launch_tc(LogitsParams& p, cudaStream_t st, const char* who, int batc
   using Cfg = TcCfg<MODE>;
   static_assert(Cfg::kSmemBytes <= 227 * 1024, "shared memory budget");
   logits_plan(p, batch);
-  if (MODE == MODE_TOPK) logits_plan_topk(p);
+  if (Cfg::kTopkMode) logits_plan_topk(p);
   cudaError_t e = cudaFuncSetAttribute(logits_tc_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
   if (e != cudaSuccess) { set_error("%s: smem attr: %s", who, cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
   launch_pdl(logits_tc_kernel<MODE>, dim3(p.m_tiles * p.n_chunks, batch), dim3(Cfg::kThreads), Cfg::kSmemBytes, st, p);
@@ -781,6 +829,40 @@ int acsr_logits_topk_partial_ws(const float* out, const float* table, int M, int
     }
   }
   return launch_tc<MODE_TOPK>(p, (cudaStream_t)stream, "logits_topk_partial");
+}
+
+int acsr_row_dot(const float* out, const float* table, const int64_t* ids, int M, int d, int64_t V, int64_t idx_offset, float* dot,
+                 void* stream) {
+  ACSR_REQUIRE(out && table && ids && dot, "row_dot: NULL pointer");
+  ACSR_REQUIRE(M > 0 && V > 0 && d > 0, "row_dot: bad sizes M=%d V=%lld d=%d", M, (long long)V, d);
+  launch_pdl(row_dot_kernel, dim3((M + 7) / 8), dim3(256), 0, (cudaStream_t)stream, out, table, (const long long*)ids, M, d, (long long)V,
+             (long long)idx_offset, dot);
+  return check_launch("row_dot");
+}
+
+int acsr_logits_topk_rank_partial(const float* out, const float* table, int M, int64_t V, int d, int passes, int k, int64_t idx_offset,
+                                  int skip_col0, const int64_t* positive, const float* pos_score, float* partial_val,
+                                  int64_t* partial_idx, int32_t* partial_counts, int32_t* row_bound, void* stream) {
+  int rc = validate_common(out, table, M, V, d, passes, "logits_topk_rank_partial");
+  if (rc) return rc;
+  ACSR_REQUIRE(partial_val && partial_idx && positive && pos_score && partial_counts, "logits_topk_rank_partial: NULL pointer");
+  if (k < 1 || k > kMaxTopK) { set_error("logits_topk_rank_partial: k=%d unsupported (1..%d)", k, kMaxTopK); return ACSR_ERR_UNSUPPORTED; }
+  LogitsParams p = {};
+  p.out = out; p.table = table; p.M = M; p.V = V; p.passes = passes;
+  p.k = k; p.idx_offset = idx_offset; p.skip_col0 = skip_col0; p.pval = partial_val; p.pidx = (long long*)partial_idx;
+  p.rank_pos = (const long long*)positive; p.rank_score = pos_score; p.rank_counts = partial_counts;
+  if (d != kD) return launch_logits_simt(MODE_TOPK_RANK, p, d, (cudaStream_t)stream, "logits_topk_rank_partial");
+  {
+    LogitsParams q = p;                    // the shared bound as in acsr_logits_topk_partial_ws
+    logits_plan(q);
+    logits_plan_topk(q);
+    p.row_bound = (row_bound != nullptr && 2 * q.n_chunks >= k) ? row_bound : nullptr;
+    if (p.row_bound != nullptr) {
+      cudaError_t e = cudaMemsetAsync(row_bound, 0x80, (size_t)M * 2 * q.n_chunks * sizeof(int32_t), (cudaStream_t)stream);
+      if (e != cudaSuccess) { set_error("logits_topk_rank_partial: memset: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
+    }
+  }
+  return launch_tc<MODE_TOPK_RANK>(p, (cudaStream_t)stream, "logits_topk_rank_partial");
 }
 
 }  // extern "C"

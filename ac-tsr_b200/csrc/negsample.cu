@@ -123,20 +123,22 @@ __device__ __forceinline__ float group_dot(const float4* __restrict__ o4, const 
   return acc;
 }
 
-template <int G>
+// COUNT: every candidate id enters the hash set (the positive's first), and counts[m] = (distinct negatives scoring above the
+// positive = the rank, distinct negatives tied with it, distinct candidates = the finite entries of the scattered score row)
+template <int G, bool COUNT>
 __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const float* __restrict__ out, const float* __restrict__ table,
                                                                       long long V, int d, const long long* __restrict__ cand, int C,
                                                                       int kmax, int hash_size, int* __restrict__ rec,
-                                                                      float* __restrict__ scores) {
+                                                                      float* __restrict__ scores, int* __restrict__ counts) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float4* o4 = reinterpret_cast<float4*>(smem_raw);
   long long* hset = reinterpret_cast<long long*>(smem_raw + (size_t)d * 4);
   __shared__ float s_pos;
-  __shared__ int s_rank;
+  __shared__ int s_rank, s_eq, s_distinct;
   pdl_launch_dependents();
   const int m = blockIdx.x, tid = threadIdx.x;
   for (int i = tid; i < hash_size; i += kRankThreads) hset[i] = -1;
-  if (tid == 0) s_rank = 0;
+  if (tid == 0) { s_rank = 0; s_eq = 0; s_distinct = 1; }
   pdl_wait();
   const int d4 = d >> 2;
   const float4* orow = reinterpret_cast<const float4*>(out + (long long)m * d);
@@ -153,9 +155,12 @@ __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const floa
       if (scores != nullptr) scores[(long long)m * C] = s;
     }
   }
+  const unsigned mask = (unsigned)hash_size - 1;
+  long long pos_id = crow[0];
+  pos_id = pos_id < 0 ? 0 : (pos_id >= V ? V - 1 : pos_id);
+  if (COUNT && tid == 0) hset[hash_slot(pos_id, mask)] = pos_id;     // a negative equal to the positive collapses into it
   __syncthreads();
   const float s0 = s_pos;
-  const unsigned mask = (unsigned)hash_size - 1;
   const int groups = kRankThreads / G;
   for (int c = 1 + tid / G; c - (tid / G) < C; c += groups) {          // every lane of a warp iterates the same number of times
     const bool live = c < C;
@@ -164,7 +169,21 @@ __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const floa
     const float s = group_dot<G>(o4, reinterpret_cast<const float4*>(table + id * d), d4, sub);
     if (live && sub == 0) {
       if (scores != nullptr) scores[(long long)m * C + c] = s;
-      if (s > s0) {                                                    // ties count in the positive's favour
+      if (COUNT) {
+        unsigned h = hash_slot(id, mask);
+        while (true) {
+          const long long prev = (long long)atomicCAS(reinterpret_cast<unsigned long long*>(hset + h), (unsigned long long)-1ll,
+                                                      (unsigned long long)id);
+          if (prev == -1) {                                            // first copy of this item among all candidates
+            atomicAdd(&s_distinct, 1);
+            if (s > s0) atomicAdd(&s_rank, 1);
+            else if (s == s0) atomicAdd(&s_eq, 1);
+            break;
+          }
+          if (prev == id) break;
+          h = (h + 1) & mask;
+        }
+      } else if (s > s0) {                                             // ties count in the positive's favour
         unsigned h = hash_slot(id, mask);
         while (true) {
           const long long prev = (long long)atomicCAS(reinterpret_cast<unsigned long long*>(hset + h), (unsigned long long)-1ll,
@@ -180,6 +199,11 @@ __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const floa
   const int rank = s_rank;
   int* rrow = rec + (long long)m * (kmax + 1);
   for (int i = tid; i <= kmax; i += kRankThreads) rrow[i] = (i == kmax) ? 1 : (i == rank ? 1 : 0);
+  if (COUNT && tid == 0) {
+    counts[3 * m] = rank;
+    counts[3 * m + 1] = s_eq;
+    counts[3 * m + 2] = s_distinct;
+  }
 }
 
 }  // namespace acsr
@@ -210,8 +234,8 @@ int acsr_neg_sample(const int64_t* users, const int64_t* positives, const int64_
 
 int acsr_candidate_rank_max_candidates(void) { return kRankMaxCand; }
 
-int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
-                        int32_t* rec, float* scores, void* stream) {
+static int candidate_rank_impl(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
+                               int32_t* rec, float* scores, int32_t* counts, void* stream) {
   ACSR_REQUIRE(out && table && cand && rec, "candidate_rank: NULL pointer");
   ACSR_REQUIRE(M > 0 && V > 0 && n_cand >= 1 && kmax >= 1, "candidate_rank: bad sizes");
   ACSR_REQUIRE(d > 0 && d % 4 == 0, "candidate_rank: hidden size %d must be a positive multiple of 4", d);
@@ -230,10 +254,17 @@ int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, 
   cudaStream_t st = (cudaStream_t)stream;
 #define ACSR_RANK_LAUNCH(G)                                                                                                  \
   do {                                                                                                                       \
-    cudaError_t e = cudaFuncSetAttribute(candidate_rank_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    if (e != cudaSuccess) { set_error("candidate_rank: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }      \
-    launch_pdl(candidate_rank_kernel<G>, dim3(M), dim3(kRankThreads), smem, st, out, table, (long long)V, d,               \
-               (const long long*)cand, n_cand, kmax, hash_size, (int*)rec, scores);                                         \
+    if (counts != nullptr) {                                                                                                 \
+      cudaError_t e = cudaFuncSetAttribute(candidate_rank_kernel<G, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+      if (e != cudaSuccess) { set_error("candidate_rank: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }    \
+      launch_pdl(candidate_rank_kernel<G, true>, dim3(M), dim3(kRankThreads), smem, st, out, table, (long long)V, d,       \
+                 (const long long*)cand, n_cand, kmax, hash_size, (int*)rec, scores, (int*)counts);                         \
+    } else {                                                                                                                 \
+      cudaError_t e = cudaFuncSetAttribute(candidate_rank_kernel<G, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+      if (e != cudaSuccess) { set_error("candidate_rank: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }    \
+      launch_pdl(candidate_rank_kernel<G, false>, dim3(M), dim3(kRankThreads), smem, st, out, table, (long long)V, d,      \
+                 (const long long*)cand, n_cand, kmax, hash_size, (int*)rec, scores, (int*)nullptr);                        \
+    }                                                                                                                        \
   } while (0)
   if (d4 > 16) ACSR_RANK_LAUNCH(32);
   else if (d4 > 8) ACSR_RANK_LAUNCH(16);
@@ -241,6 +272,17 @@ int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, 
   else ACSR_RANK_LAUNCH(4);
 #undef ACSR_RANK_LAUNCH
   return check_launch("candidate_rank");
+}
+
+int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
+                        int32_t* rec, float* scores, void* stream) {
+  return candidate_rank_impl(out, table, V, d, cand, M, n_cand, kmax, rec, scores, nullptr, stream);
+}
+
+int acsr_candidate_rank_counts(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
+                               int32_t* rec, float* scores, int32_t* counts, void* stream) {
+  ACSR_REQUIRE(counts, "candidate_rank_counts: NULL counts");
+  return candidate_rank_impl(out, table, V, d, cand, M, n_cand, kmax, rec, scores, counts, stream);
 }
 
 }  // extern "C"

@@ -21,10 +21,15 @@ __device__ __forceinline__ unsigned f2key(float v) {        // larger float <-> 
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
+// RANK: counts[row] = (#items scoring > s_pos, #items scoring == s_pos) with s_pos = pos_score[row].  Dense rows count their own
+// scores, the excluded position 0 and the positive's own column left out; candidate lists sum the n_count_parts (greater, equal)
+// pairs pcounts[row, :] the producers of the lists counted.
+template <bool RANK>
 __global__ void __launch_bounds__(kMergeThreads)
 topk_merge_kernel(const float* __restrict__ pval, const long long* __restrict__ pidx, int n_cand, long long ld, int k,
                   int skip_first, long long idx_offset, const long long* __restrict__ positive, float* __restrict__ oval,
-                  long long* __restrict__ oidx, int* __restrict__ rec) {
+                  long long* __restrict__ oidx, int* __restrict__ rec, const float* __restrict__ pos_score,
+                  const int* __restrict__ pcounts, int n_count_parts, int* __restrict__ counts) {
   // pidx != NULL: candidate lists (value, item id; id < 0 = padding).  pidx == NULL: a dense score row, item id = position +
   // idx_offset, position 0 excluded when skip_first (trainer.py:942: scores[:, 0] = -inf).
   pdl_launch_dependents();
@@ -40,10 +45,29 @@ topk_merge_kernel(const float* __restrict__ pval, const long long* __restrict__ 
   const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const float* rv = pval + (long long)row * ld;
   const long long* ri = pidx ? pidx + (long long)row * ld : nullptr;
-  for (int i = tid; i < n_cand; i += kMergeThreads) {
-    const bool valid = ri ? ri[i] >= 0 : !(skip_first && i == 0);
-    keys[i] = valid ? f2key(rv[i]) : 0u;                  // padding entries sort last
+  int r_gt = 0, r_eq = 0;                                // RANK: this thread's share of the row's counts
+  __shared__ int s_gt, s_eq;
+  const float r_s = RANK && pidx == nullptr ? pos_score[row] : 0.f;
+  const long long r_pl = RANK && pidx == nullptr ? positive[row] - idx_offset : -1;
+  if (RANK && pidx == nullptr) {                         // dense row: each score is read once for its key and its count
+    for (int i = tid; i < n_cand; i += kMergeThreads) {
+      const bool valid = !(skip_first && i == 0);
+      const float x = rv[i];
+      keys[i] = valid ? f2key(x) : 0u;
+      if (valid && i != r_pl) { r_gt += x > r_s; r_eq += x == r_s; }
+    }
+  } else {
+    for (int i = tid; i < n_cand; i += kMergeThreads) {
+      const bool valid = ri ? ri[i] >= 0 : !(skip_first && i == 0);
+      keys[i] = valid ? f2key(rv[i]) : 0u;                // padding entries sort last
+    }
   }
+  if (RANK && pidx != nullptr)
+    for (int i = tid; i < n_count_parts; i += kMergeThreads) {
+      r_gt += pcounts[((long long)row * n_count_parts + i) * 2];
+      r_eq += pcounts[((long long)row * n_count_parts + i) * 2 + 1];
+    }
+  if (RANK && tid == 0) { s_gt = 0; s_eq = 0; }
   if (tid == 0) { s_prefix = 0u; s_need = k; s_cnt = 0; }
   if (tid < kMergeMaxK) sel[tid] = 0ull;
   // ---- fast path: a lower bound T0 of the k-th largest key from the threads' local maxima (at least k keys are >= the k-th
@@ -200,6 +224,13 @@ topk_merge_kernel(const float* __restrict__ pval, const long long* __restrict__ 
   }
   }   // radix-select path
   __syncthreads();
+  if (RANK) {                                            // s_gt / s_eq were zeroed before the barriers above
+    r_gt = __reduce_add_sync(0xffffffffu, r_gt);
+    r_eq = __reduce_add_sync(0xffffffffu, r_eq);
+    if (lane == 0) { atomicAdd(&s_gt, r_gt); atomicAdd(&s_eq, r_eq); }
+    __syncthreads();
+    if (tid == 0) { counts[2 * row] = s_gt; counts[2 * row + 1] = s_eq; }
+  }
   const long long pos_item = positive ? positive[row] : -1;
   for (int j = tid; j < k; j += kMergeThreads) {
     const unsigned long long e = sel[j];
@@ -226,11 +257,29 @@ extern "C" int acsr_topk_merge(const float* partial_val, const int64_t* partial_
   ACSR_REQUIRE(n_cand >= k, "topk_merge: fewer candidates than k");
   if (k > kMergeMaxK) { set_error("topk_merge: k=%d unsupported (1..%d)", k, kMergeMaxK); return ACSR_ERR_UNSUPPORTED; }
   const size_t smem = (size_t)n_cand * 4;
-  cudaError_t e = cudaFuncSetAttribute(topk_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(topk_merge_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) { set_error("topk_merge: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
-  launch_pdl(topk_merge_kernel, dim3(M), dim3(kMergeThreads), smem, (cudaStream_t)stream, partial_val, (const long long*)partial_idx, n_cand,
-             (long long)n_cand, k, 0, 0ll, (const long long*)positive, topk_val, (long long*)topk_idx, rec_topk);
+  launch_pdl(topk_merge_kernel<false>, dim3(M), dim3(kMergeThreads), smem, (cudaStream_t)stream, partial_val, (const long long*)partial_idx, n_cand,
+             (long long)n_cand, k, 0, 0ll, (const long long*)positive, topk_val, (long long*)topk_idx, rec_topk, (const float*)nullptr,
+             (const int*)nullptr, 0, (int*)nullptr);
   return check_launch("topk_merge");
+}
+
+extern "C" int acsr_topk_merge_rank(const float* partial_val, const int64_t* partial_idx, int M, int n_parts, int k,
+                                    const int64_t* positive, const int32_t* partial_counts, int n_count_parts, float* topk_val,
+                                    int64_t* topk_idx, int32_t* rec_topk, int32_t* counts, void* stream) {
+  ACSR_REQUIRE(partial_val && partial_idx && topk_val && topk_idx && partial_counts && counts, "topk_merge_rank: NULL pointer");
+  ACSR_REQUIRE(M > 0 && n_parts > 0 && k > 0 && n_count_parts > 0, "topk_merge_rank: bad sizes");
+  const int n_cand = n_parts * k;
+  if (n_cand > kMergeMaxCand) { set_error("topk_merge_rank: %d candidates per row exceed %d", n_cand, kMergeMaxCand); return ACSR_ERR_UNSUPPORTED; }
+  if (k > kMergeMaxK) { set_error("topk_merge_rank: k=%d unsupported (1..%d)", k, kMergeMaxK); return ACSR_ERR_UNSUPPORTED; }
+  const size_t smem = (size_t)n_cand * 4;
+  cudaError_t e = cudaFuncSetAttribute(topk_merge_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) { set_error("topk_merge_rank: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
+  launch_pdl(topk_merge_kernel<true>, dim3(M), dim3(kMergeThreads), smem, (cudaStream_t)stream, partial_val, (const long long*)partial_idx,
+             n_cand, (long long)n_cand, k, 0, 0ll, (const long long*)positive, topk_val, (long long*)topk_idx, rec_topk,
+             (const float*)nullptr, (const int*)partial_counts, n_count_parts, (int*)counts);
+  return check_launch("topk_merge_rank");
 }
 
 extern "C" int acsr_topk_select_max_items(void) { return kMergeMaxCand; }
@@ -243,9 +292,27 @@ extern "C" int acsr_topk_select(const float* scores, int M, int64_t V, int64_t l
   if (k > kMergeMaxK) { set_error("topk_select: k=%d unsupported (1..%d)", k, kMergeMaxK); return ACSR_ERR_UNSUPPORTED; }
   ACSR_REQUIRE(V - (skip_col0 ? 1 : 0) >= k, "topk_select: fewer items than k");
   const size_t smem = (size_t)V * 4;
-  cudaError_t e = cudaFuncSetAttribute(topk_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(topk_merge_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) { set_error("topk_select: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
-  launch_pdl(topk_merge_kernel, dim3(M), dim3(kMergeThreads), smem, (cudaStream_t)stream, scores, (const long long*)nullptr, (int)V, (long long)ld, k,
-             skip_col0 ? 1 : 0, (long long)idx_offset, (const long long*)positive, topk_val, (long long*)topk_idx, rec_topk);
+  launch_pdl(topk_merge_kernel<false>, dim3(M), dim3(kMergeThreads), smem, (cudaStream_t)stream, scores, (const long long*)nullptr, (int)V, (long long)ld, k,
+             skip_col0 ? 1 : 0, (long long)idx_offset, (const long long*)positive, topk_val, (long long*)topk_idx, rec_topk,
+             (const float*)nullptr, (const int*)nullptr, 0, (int*)nullptr);
   return check_launch("topk_select");
+}
+
+extern "C" int acsr_topk_select_rank(const float* scores, int M, int64_t V, int64_t ld, int k, int skip_col0, int64_t idx_offset,
+                                     const int64_t* positive, const float* pos_score, float* topk_val, int64_t* topk_idx,
+                                     int32_t* rec_topk, int32_t* counts, void* stream) {
+  ACSR_REQUIRE(scores && topk_val && topk_idx && positive && pos_score && counts, "topk_select_rank: NULL pointer");
+  ACSR_REQUIRE(M > 0 && V > 0 && k > 0 && ld >= V, "topk_select_rank: bad sizes");
+  if (V > kMergeMaxCand) { set_error("topk_select_rank: %lld items per row exceed %d (use the fused top-k)", (long long)V, kMergeMaxCand); return ACSR_ERR_UNSUPPORTED; }
+  if (k > kMergeMaxK) { set_error("topk_select_rank: k=%d unsupported (1..%d)", k, kMergeMaxK); return ACSR_ERR_UNSUPPORTED; }
+  ACSR_REQUIRE(V - (skip_col0 ? 1 : 0) >= k, "topk_select_rank: fewer items than k");
+  const size_t smem = (size_t)V * 4;
+  cudaError_t e = cudaFuncSetAttribute(topk_merge_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) { set_error("topk_select_rank: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
+  launch_pdl(topk_merge_kernel<true>, dim3(M), dim3(kMergeThreads), smem, (cudaStream_t)stream, scores, (const long long*)nullptr, (int)V,
+             (long long)ld, k, skip_col0 ? 1 : 0, (long long)idx_offset, (const long long*)positive, topk_val, (long long*)topk_idx,
+             rec_topk, pos_score, (const int*)nullptr, 0, (int*)counts);
+  return check_launch("topk_select_rank");
 }

@@ -71,6 +71,15 @@ class CudaCompute(object):
     def topk_merge(self, pv, pi, k, positive):
         return self.ops.topk_merge(pv, pi, k, positive)
 
+    def row_dot(self, out, table, ids, idx_offset):
+        return self.ops.row_dot(out, table, ids, idx_offset)
+
+    def topk_rank_partial(self, out, table, k, positive, pos_score, idx_offset, skip_col0):
+        return self.ops.logits_topk_rank_partial(out, table, k, positive, pos_score, idx_offset, skip_col0, self.passes)
+
+    def topk_merge_rank(self, pv, pi, k, pc, positive):
+        return self.ops.topk_merge_rank(pv, pi, k, pc, positive)
+
     def gather_rows(self, ids, shard, lo, hi):
         out = torch.empty((ids.numel(), shard.shape[1]), dtype=torch.float32, device=shard.device)
         self.LIB.call('acsr_shard_gather_rows', self.ops._p(ids, torch.int64), ids.numel(), self.ops._p(shard), lo, hi, shard.shape[1],
@@ -201,12 +210,26 @@ class VocabParallel(object):
         return self._reduce_scatter(d_out_all, R)
 
     # ------------------------------------------------------------------------------------------
-    def full_sort_topk(self, out_local, table, k, positive_local=None):
+    def full_sort_topk(self, out_local, table, k, positive_local=None, counts=False):
         """all-gather of partial top-k lists (north_star eval path) -> (val [R,k], idx [R,k], rec|None).  Each rank first merges
         its shard's per-chunk lists into one list per row, so the final merge sees W*k candidates however many chunks a shard
-        runs (W * 148 chunk lists of k would exceed the merge's capacity)."""
+        runs (W * 148 chunk lists of k would exceed the merge's capacity).  counts=True: also counts [R, 2] int32 (GAUC's rank
+        inputs, ops.full_sort_topk) -- every shard counts its own items against the positive's score, which the owner of the
+        positive's row computes (the others contribute 0 to a sum, like the CE target logit), and the per-row counts are summed."""
         R, d = out_local.shape
         out_all = self._all_gather(out_local).view(self.world * R, d)
+        if counts:
+            E_s = self.shard(table)
+            pos_all = self._all_gather(positive_local.reshape(R)).view(self.world * R)
+            s_pos = self.compute.row_dot(out_all, E_s, pos_all, self.lo)
+            dist.all_reduce(s_pos, group=self.group)
+            pv, pi, pc = self.compute.topk_rank_partial(out_all, E_s, k, pos_all, s_pos, self.lo, self.lo == 0)
+            sv, si, _, sc = self.compute.topk_merge_rank(pv, pi, k, pc, None)                     # [W*R, k], [W*R, 2]
+            sl = slice(self.rank * R, (self.rank + 1) * R)
+            mv = self._all_gather(sv)[:, sl].permute(1, 0, 2).contiguous()                         # [R, W, k]
+            mi = self._all_gather(si)[:, sl].permute(1, 0, 2).contiguous()
+            mc = self._all_gather(sc)[:, sl].permute(1, 0, 2).contiguous()                         # [R, W, 2]
+            return self.compute.topk_merge_rank(mv, mi, k, mc, positive_local)
         pv, pi = self.compute.topk_partial(out_all, self.shard(table), k, self.lo, self.lo == 0)   # [W*R, nc, k]
         sv, si, _ = self.compute.topk_merge(pv, pi, k, None)                                      # [W*R, k]
         sl = slice(self.rank * R, (self.rank + 1) * R)

@@ -848,16 +848,96 @@ def topk_select(scores, k, positive=None, skip_col0=True, idx_offset=0):
     return val, idx, rec
 
 
+def _check_positive(positive, M, who):
+    if positive is None or positive.dim() != 1 or positive.shape[0] != M:
+        raise AcsrError('%s: positive must be a 1-D tensor of %d item ids (got %s)' % (who, M, None if positive is None else tuple(positive.shape)))
+    return positive.contiguous()
+
+
+def row_dot(out, table, ids, idx_offset=0):
+    """dot [M] = out[m] . table[ids[m] - idx_offset] in fp32 (0 where that row is not in this table / shard), the positive's score
+    the rank counts are taken against (acsr_row_dot)"""
+    out, table = out.contiguous(), table.contiguous()
+    M, d = out.shape
+    if table.dim() != 2 or table.shape[1] != d:
+        raise AcsrError('row_dot: out %s and table %s disagree' % (tuple(out.shape), tuple(table.shape)))
+    ids = _check_positive(ids, M, 'row_dot')
+    dot = torch.empty(M, dtype=torch.float32, device=out.device)
+    LIB.call('acsr_row_dot', _p(out), _p(table), _p(ids, torch.int64), M, d, table.shape[0], int(idx_offset), _p(dot), _stream())
+    return dot
+
+
+def logits_topk_rank_partial(out, table, k, positive, pos_score, idx_offset=0, skip_col0=True, passes=3, share_bound=True):
+    """logits_topk_partial + per-(row, chunk) counts [M, nc, 2] int32 of the scores above / equal to pos_score (GAUC)"""
+    out, table = out.contiguous(), table.contiguous()
+    M, d = out.shape
+    V = table.shape[0]
+    positive = _check_positive(positive, M, 'logits_topk_rank_partial')
+    if pos_score.shape != (M,):
+        raise AcsrError('logits_topk_rank_partial: pos_score must be [%d] (got %s)' % (M, tuple(pos_score.shape)))
+    nc = logits_num_chunks(M, V)
+    pv = torch.empty((M, nc, k), dtype=torch.float32, device=out.device)
+    pi = torch.empty((M, nc, k), dtype=torch.int64, device=out.device)
+    pc = torch.empty((M, nc, 2), dtype=torch.int32, device=out.device)
+    rb = torch.empty(2 * M * nc, dtype=torch.int32, device=out.device) if share_bound else None
+    LIB.call('acsr_logits_topk_rank_partial', _p(out), _p(table), M, V, d, passes, k, idx_offset, int(skip_col0),
+             _p(positive, torch.int64), _p(pos_score.contiguous()), _p(pv), _p(pi, torch.int64), _p(pc, torch.int32),
+             _p(rb, torch.int32), _stream())
+    return pv, pi, pc
+
+
+def topk_merge_rank(pv, pi, k, pc, positive=None):
+    """topk_merge + the sum of the per-part counts pc [M, n, 2] -> (val, idx, rec | None, counts [M, 2] int32)"""
+    M = pv.shape[0]
+    pv = pv.reshape(M, -1, k).contiguous()
+    pi = pi.reshape(M, -1, k).contiguous()
+    pc = pc.reshape(M, -1, 2).contiguous()
+    dev = pv.device
+    val = torch.empty((M, k), dtype=torch.float32, device=dev)
+    idx = torch.empty((M, k), dtype=torch.int64, device=dev)
+    rec = torch.empty((M, k + 1), dtype=torch.int32, device=dev) if positive is not None else None
+    counts = torch.empty((M, 2), dtype=torch.int32, device=dev)
+    LIB.call('acsr_topk_merge_rank', _p(pv), _p(pi, torch.int64), M, pv.shape[1], k,
+             _p(positive.contiguous(), torch.int64) if positive is not None else None, _p(pc, torch.int32), pc.shape[1],
+             _p(val), _p(idx, torch.int64), _p(rec, torch.int32), _p(counts, torch.int32), _stream())
+    return val, idx, rec, counts
+
+
+def topk_select_rank(scores, k, positive, pos_score, skip_col0=True, idx_offset=0):
+    """topk_select + counts [M, 2] int32 of the row's scores above / equal to pos_score (the positive's column left out)"""
+    M, V = scores.shape
+    dev = scores.device
+    if not scores.is_cuda or scores.dtype != torch.float32 or scores.stride(1) != 1:
+        raise AcsrError('topk_select_rank: scores must be a float32 CUDA matrix with unit column stride (rows may be strided)')
+    positive = _check_positive(positive, M, 'topk_select_rank')
+    val = torch.empty((M, k), dtype=torch.float32, device=dev)
+    idx = torch.empty((M, k), dtype=torch.int64, device=dev)
+    rec = torch.empty((M, k + 1), dtype=torch.int32, device=dev)
+    counts = torch.empty((M, 2), dtype=torch.int32, device=dev)
+    LIB.call('acsr_topk_select_rank', scores.data_ptr(), M, V, scores.stride(0), k, int(skip_col0), idx_offset,
+             _p(positive, torch.int64), _p(pos_score.contiguous()), _p(val), _p(idx, torch.int64), _p(rec, torch.int32),
+             _p(counts, torch.int32), _stream())
+    return val, idx, rec, counts
+
+
 _SELECT_MAX = []
 
 
-def full_sort_topk(out, table, k, positive=None, passes=3):
+def full_sort_topk(out, table, k, positive=None, passes=3, counts=False):
     """scores -> scores[:,0]=-inf -> top-k -> hit flags (trainer.py:941-942, collector.py:147-153).  Small catalogues
     (one row of scores fits in shared memory): tensor-core scores, L2-resident, + radix select; large ones: the fused
-    logits + streaming top-k kernel and a merge of its per-chunk lists (the scores never exist)."""
+    logits + streaming top-k kernel and a merge of its per-chunk lists (the scores never exist).
+    counts=True (needs positive): also -> counts [M, 2] int32 = (#items scoring above, #items tied with) the positive's fp32 score
+    (row_dot), column 0 and the positive itself not counted -- GAUC's average rank without sorting the catalogue."""
     if not _SELECT_MAX:
         _SELECT_MAX.append(LIB.query('acsr_topk_select_max_items'))
     V = table.shape[0]
+    if counts:
+        s_pos = row_dot(out, table, _check_positive(positive, out.shape[0], 'full_sort_topk'))
+        if V <= _SELECT_MAX[0] and V - 1 >= k:
+            return topk_select_rank(logits_scores(out, table, passes), k, positive, s_pos)
+        pv, pi, pc = logits_topk_rank_partial(out, table, k, positive, s_pos, 0, True, passes)
+        return topk_merge_rank(pv, pi, k, pc, positive)
     if V <= _SELECT_MAX[0] and V - 1 >= k:
         return topk_select(logits_scores(out, table, passes), k, positive)
     pv, pi = logits_topk_partial(out, table, k, 0, True, passes)
@@ -894,9 +974,10 @@ def neg_sample(users, n_neg, used_offsets, used_items, n_items, rng, rng_stream,
     return out
 
 
-def candidate_rank(out, table, cand, k, want_scores=False):
+def candidate_rank(out, table, cand, k, want_scores=False, want_counts=False):
     """rank of column 0 of cand [M, 1+N] among the distinct other candidates by out[m] . table[c] (fp32), as the hit-flag
-    matrix rec [M, k+1] int32 of the evaluator (acsr_candidate_rank) -> (rec, scores [M, 1+N] | None)"""
+    matrix rec [M, k+1] int32 of the evaluator (acsr_candidate_rank) -> (rec, scores [M, 1+N] | None); want_counts: -> (rec,
+    scores | None, counts [M, 3] int32 = distinct negatives above / tied with the positive, distinct candidates)"""
     out, table, cand = out.contiguous(), table.contiguous(), cand.contiguous()
     if out.dim() != 2 or table.dim() != 2 or cand.dim() != 2:
         raise AcsrError('candidate_rank: out [M, d], table [V, d] and cand [M, 1+N] must be matrices')
@@ -906,6 +987,11 @@ def candidate_rank(out, table, cand, k, want_scores=False):
                                                                                             tuple(cand.shape), int(k)))
     rec = torch.empty((M, k + 1), dtype=torch.int32, device=out.device)
     scores = torch.empty(cand.shape, dtype=torch.float32, device=out.device) if want_scores else None
+    if want_counts:
+        counts = torch.empty((M, 3), dtype=torch.int32, device=out.device)
+        LIB.call('acsr_candidate_rank_counts', _p(out), _p(table), table.shape[0], d, _p(cand, torch.int64), M, cand.shape[1], int(k),
+                 _p(rec, torch.int32), _p(scores), _p(counts, torch.int32), _stream())
+        return rec, scores, counts
     LIB.call('acsr_candidate_rank', _p(out), _p(table), table.shape[0], d, _p(cand, torch.int64), M, cand.shape[1], int(k),
              _p(rec, torch.int32), _p(scores), _stream())
     return rec, scores

@@ -215,6 +215,9 @@ class ACSASRecTrainer(object):
         # BPR with `neg_sampling` on host-side batches: the ops.NegSampler that draws each step's negatives on the device
         # (set from the training loader by _train_epoch; a DeviceTrainDataLoader draws inside its own gather instead)
         self.train_neg_sampler = None
+        # training rows per target item (RecBole's data.count_items, collected from the training data by fit / set_item_counts):
+        # AveragePopularity and TailPercentage read it
+        self.item_counts = None
         self.logger.info('use attack trainer!!!')
 
     # ------------------------------------------------------------------------------------------
@@ -578,8 +581,22 @@ class ACSASRecTrainer(object):
         self.optimizer.load_state_dict(checkpoint['optimizer'], scatter=scatter)
         self.logger.info('Checkpoint loaded. Resume training from epoch {}'.format(self.start_epoch))
 
+    def set_item_counts(self, train_data):
+        """record the training item counts the popularity metrics need (collector.py data_collect(train_data): data.count_items)
+        from a training loader or dataset (its inter_feat item ids), or take them as an array indexed by item id"""
+        ds = getattr(train_data, 'dataset', train_data)
+        feat = getattr(ds, 'inter_feat', None)
+        if feat is not None:
+            ids = feat[ds.iid_field]
+            ids = (ids.cpu() if torch.is_tensor(ids) else torch.as_tensor(ids)).to(torch.int64).reshape(-1)
+            n = int(getattr(ds, 'item_num', 0) or 0)
+            self.item_counts = np.bincount(ids.numpy(), minlength=n).astype(np.int64)
+        else:
+            self.item_counts = np.asarray(train_data, dtype=np.int64)
+
     def fit(self, train_data, valid_data=None, verbose=True, saved=True, show_progress=False, callback_fn=None):
         """trainer.py:809-924 (epoch range 2*epochs, eval every eval_step, early stopping, checkpoint on improvement)."""
+        self.set_item_counts(train_data)
         if saved and self.start_epoch >= self.epochs:
             self._save_checkpoint(-1, verbose=verbose)
         for epoch_idx in range(self.start_epoch, 2 * self.epochs):
@@ -628,33 +645,54 @@ class ACSASRecTrainer(object):
             scores[history_index] = -np.inf
         return interaction, scores, positive_u, positive_i
 
-    def eval_batch(self, batched_data, rec_out=None, neg_sampler=None, neg_num=0):
+    def eval_batch(self, batched_data, rec_out=None, neg_sampler=None, neg_num=0, need=None):
         """-> rec_topk [B, kmax+1] int32 on the device (collector.py:145-153 'rec.topk'); with rec_out (a pinned host tensor)
         the graphed path copies the result straight into it (no device-side clone) and returns rec_out.  With neg_sampler (the
         batch of a data.NegSampleEvalDataLoader, `eval_args.mode: uniN / popN`): the positive is ranked against neg_num
-        negatives drawn on the device (trainer.py _neg_sample_batch_eval, collector.py eval_batch_collect)."""
+        negatives drawn on the device (trainer.py _neg_sample_batch_eval, collector.py eval_batch_collect).
+        need = (counts, items) with either set (what GAUC / the item-distribution metrics read): -> (rec, counts [B, 2] int32 | None,
+        user_len [B] int32 | None, items [B, kmax] int32 | None) instead, all on the device (collector.py rec.meanrank / rec.items)."""
         interaction, history_index, positive_u, positive_i = batched_data
         kmax = max(self.topk)
+        need = tuple(bool(x) for x in need) if need is not None and any(need) else None
         if neg_sampler is not None:
-            return self._sampled_eval(interaction, positive_i, neg_sampler, int(neg_num), kmax, rec_out)
+            return self._sampled_eval(interaction, positive_i, neg_sampler, int(neg_num), kmax, rec_out, need)
         if self.fused_topk and history_index is None:
             if kmax > 64:                      # the fused top-k keeps at most 64 candidates per row: materialised scores + torch.topk
-                return self._eval_materialised(batched_data, kmax, rec_out)
+                return self._eval_materialised(batched_data, kmax, rec_out, need)
             if self.use_graph and not self.model.training and not self._host_schedule():
-                return self._graphed_eval(interaction, positive_i, kmax, rec_out)
+                return self._graphed_eval(interaction, positive_i, kmax, rec_out, need)
             inter = interaction.to(self.device)
             pos = inter[self.model.POS_ITEM_ID] if positive_i is interaction.interaction.get(self.model.POS_ITEM_ID) else \
                 positive_i.to(self.device, non_blocking=True)
+            if need is not None:
+                return self._collect_full(self.model.full_sort_topk(inter, kmax, pos, counts=need[0]), need, rec_out)
             _, _, rec = self.model.full_sort_topk(inter, kmax, pos)
         else:
-            return self._eval_materialised(batched_data, kmax, rec_out)
+            return self._eval_materialised(batched_data, kmax, rec_out, need)
         if rec_out is not None:
             rec_out.copy_(rec, non_blocking=True)
             return rec_out
         return rec
 
-    def _eval_materialised(self, batched_data, kmax, rec_out=None):
-        """trainer.py:926-945 + collector.py:145-153 on materialised scores (API-compatible path)."""
+    def _n_items(self):
+        return int(self.tot_item_num or self.model.n_items)
+
+    def _collect_full(self, res, need, rec_out=None):
+        """(val, idx, rec[, counts]) of a full-sort top-k -> (rec, counts, user_len, items) of eval_batch(need=...).  Every
+        score but column 0 is finite in full sort, so user_len = n_items - 1 (collector.py: argmin of the sorted row)."""
+        rec = res[2]
+        if rec_out is not None:
+            rec_out.copy_(rec, non_blocking=True)
+            rec = rec_out
+        counts = res[3] if need[0] else None
+        user_len = torch.full((rec.shape[0],), self._n_items() - 1, dtype=torch.int32, device=res[1].device) if need[0] else None
+        items = res[1].to(torch.int32) if need[1] else None
+        return rec, counts, user_len, items
+
+    def _eval_materialised(self, batched_data, kmax, rec_out=None, need=None):
+        """trainer.py:926-945 + collector.py:145-153 on materialised scores (API-compatible path).  need: the rank counts are
+        taken on the scores this path holds (the positive's own column left out), the ids are torch.topk's."""
         interaction, scores, positive_u, positive_i = self._full_sort_batch_eval(batched_data)
         _, topk_idx = torch.topk(scores, kmax, dim=-1)
         pos = positive_i.to(self.device)
@@ -662,16 +700,23 @@ class ACSASRecTrainer(object):
         rec = torch.cat((flags, torch.ones_like(flags[:, :1])), dim=1)
         if rec_out is not None:
             rec_out.copy_(rec, non_blocking=True)
-            return rec_out
-        return rec
+            rec = rec_out
+        if need is None:
+            return rec
+        counts = user_len = None
+        if need[0]:
+            s_pos = scores.gather(1, pos.view(-1, 1))
+            counts = torch.stack(((scores > s_pos).sum(1), (scores == s_pos).sum(1) - 1), 1).to(torch.int32)
+            user_len = torch.isfinite(scores).sum(1).to(torch.int32)
+        return rec, counts, user_len, (topk_idx.to(torch.int32) if need[1] else None)
 
     @torch.no_grad()
-    def _graphed_eval(self, interaction, positive_i, kmax, rec_out=None):
-        """forward + fused logits/top-k + hit flags of one eval batch as a CUDA-graph replay (one graph per batch shape).
-        The batch (host or device) is copied into static buffers; the returned rec tensor is a fresh copy."""
+    def _graphed_eval(self, interaction, positive_i, kmax, rec_out=None, need=None):
+        """forward + fused logits/top-k + hit flags of one eval batch as a CUDA-graph replay (one graph per batch shape, and per
+        `need` of eval_batch).  The batch (host or device) is copied into static buffers; the returned tensors are fresh copies."""
         m = self.model
         fields = list(getattr(m, 'EVAL_FIELDS', None) or [m.ITEM_SEQ, m.ITEM_SEQ_LEN])      # ACSSEPT also reads the user id
-        key = tuple(tuple(interaction[k].shape) for k in fields) + (kmax,)
+        key = tuple(tuple(interaction[k].shape) for k in fields) + (kmax,) + ((need,) if need is not None else ())
         g = self._eval_graphs.get(key)
         if g is None:
             dev = self.device
@@ -689,14 +734,20 @@ class ACSASRecTrainer(object):
             pos.copy_(positive_i)
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
+            def body():
+                if need is None:
+                    return m.full_sort_topk(inter, kmax, pos)[2], None
+                return None, self._collect_full(m.full_sort_topk(inter, kmax, pos, counts=need[0]), need)
             with torch.cuda.stream(side):
                 for _ in range(2):
-                    m.full_sort_topk(inter, kmax, pos)
+                    body()
             torch.cuda.current_stream().wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                _, _, rec = m.full_sort_topk(inter, kmax, pos)
-            g = dict(graph=graph, static=static, pos=pos, rec=rec, inter=inter)
+                rec, extra = body()
+            if extra is not None:
+                rec = extra[0]
+            g = dict(graph=graph, static=static, pos=pos, rec=rec, inter=inter, extra=extra)
             self._eval_graphs[key] = g
         if getattr(interaction, 'layout', None) == getattr(g['inter'], 'layout', ()) and positive_i is interaction.interaction.get(m.POS_ITEM_ID):
             g['inter'].packed.copy_(interaction.packed, non_blocking=True)
@@ -705,24 +756,41 @@ class ACSASRecTrainer(object):
                 g['static'][k].copy_(interaction[k], non_blocking=True)
             g['pos'].copy_(positive_i, non_blocking=True)
         g['graph'].replay()
+        return self._graph_result(g, rec_out)
+
+    @staticmethod
+    def _graph_result(g, rec_out):
+        """copies of a replayed eval graph's outputs: rec (into rec_out when given), and with a `need` the other three of eval_batch"""
         if rec_out is not None:
             rec_out.copy_(g['rec'], non_blocking=True)
-            return rec_out
-        return g['rec'].clone()
+            rec = rec_out
+        else:
+            rec = g['rec'].clone()
+        if g.get('extra') is None:
+            return rec
+        return (rec,) + tuple(t.clone() if t is not None else None for t in g['extra'][1:])
 
-    def _sampled_body(self, inter, pos, cand, sampler, kmax):
-        """negatives into cand[:, 1:] (the sampler's state advances), the positive into column 0, rank -> rec [B, kmax+1]"""
+    def _sampled_body(self, inter, pos, cand, sampler, kmax, need=None):
+        """negatives into cand[:, 1:] (the sampler's state advances), the positive into column 0, rank -> rec [B, kmax+1];
+        need (counts only: the item-distribution metrics are not defined here): -> (rec, counts [B, 2], user_len [B], None)"""
         m = self.model
         N = cand.shape[1] - 1
         sampler.draw(inter[m.USER_ID], N, positives=pos, out=cand[:, 1:], ld=N + 1)
-        _, rec = m.sampled_topk(inter, cand, kmax, pos)
-        return rec
+        if need is None:
+            _, rec = m.sampled_topk(inter, cand, kmax, pos)
+            return rec
+        _, rec, counts = m.sampled_topk(inter, cand, kmax, pos, counts=True)
+        return rec, counts[:, :2], counts[:, 2], None
 
     @torch.no_grad()
-    def _sampled_eval(self, interaction, positive_i, sampler, N, kmax, rec_out=None):
+    def _sampled_eval(self, interaction, positive_i, sampler, N, kmax, rec_out=None, need=None):
         """one batch of sampled-candidate evaluation: sampler -> encoder -> acsr_candidate_rank, eagerly or as a CUDA-graph
-        replay (one graph per batch shape; every replay draws fresh negatives)"""
+        replay (one graph per batch shape and `need`; every replay draws fresh negatives)"""
         m = self.model
+        if need is not None and need[1]:
+            raise NotImplementedError('the item-distribution metrics (ItemCoverage, AveragePopularity, GiniIndex, ShannonEntropy, '
+                                      'TailPercentage) are not available in sampled evaluation (eval_args.mode uniN / popN): '
+                                      'use full-sort evaluation for them')
         if self._sharded():
             raise ValueError('sampled evaluation (eval_args.mode uniN / popN) needs the replicated item table; '
                              'it is not implemented for a vocab-sharded table')
@@ -734,17 +802,18 @@ class ACSASRecTrainer(object):
             inter = interaction.to(dev)
             pos = positive_i.to(dev)
             cand = torch.empty((pos.shape[0], N + 1), dtype=torch.int64, device=dev)
-            rec = self._sampled_body(inter, pos, cand, sampler, kmax)
+            res = self._sampled_body(inter, pos, cand, sampler, kmax, need)
+            rec = res if need is None else res[0]
             if rec_out is not None:
                 rec_out.copy_(rec, non_blocking=True)
-                return rec_out
-            return rec
+                rec = rec_out
+            return rec if need is None else (rec,) + tuple(res[1:])
         fields = list(getattr(m, 'EVAL_FIELDS', None) or [m.ITEM_SEQ, m.ITEM_SEQ_LEN])
         if m.USER_ID not in fields:
             fields.append(m.USER_ID)
         # the graph captures the sampler's device state (used sets, alias table, Philox state): one graph per sampler, which the
         # record keeps alive so its id cannot be reused by another
-        key = ('sampled', id(sampler), N, kmax) + tuple(tuple(interaction[k].shape) for k in fields)
+        key = ('sampled', id(sampler), N, kmax) + tuple(tuple(interaction[k].shape) for k in fields) + ((need,) if need is not None else ())
         g = self._eval_graphs.get(key)
         own = getattr(interaction, 'layout', None) is not None and positive_i is interaction.interaction.get(m.POS_ITEM_ID)
         if g is None:
@@ -767,13 +836,14 @@ class ACSASRecTrainer(object):
             with torch.cuda.stream(side):      # warm-up; the sampler's state is put back so the graph starts where eager would
                 snap = sampler.rng.state.clone()
                 for _ in range(2):
-                    self._sampled_body(inter, pos, cand, sampler, kmax)
+                    self._sampled_body(inter, pos, cand, sampler, kmax, need)
                 sampler.rng.state.copy_(snap)
             torch.cuda.current_stream().wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                rec = self._sampled_body(inter, pos, cand, sampler, kmax)
-            g = dict(graph=graph, pos=pos, rec=rec, inter=inter, cand=cand, fields=fields, sampler=sampler)
+                res = self._sampled_body(inter, pos, cand, sampler, kmax, need)
+            rec, extra = (res, None) if need is None else (res[0], res)
+            g = dict(graph=graph, pos=pos, rec=rec, inter=inter, cand=cand, fields=fields, sampler=sampler, extra=extra)
             self._eval_graphs[key] = g
         assert g['sampler'] is sampler
         if own and interaction.layout == getattr(g['inter'], 'layout', ()):
@@ -783,10 +853,7 @@ class ACSASRecTrainer(object):
                 g['inter'][k].copy_(interaction[k], non_blocking=True)
             g['pos'].copy_(positive_i, non_blocking=True)
         g['graph'].replay()
-        if rec_out is not None:
-            rec_out.copy_(g['rec'], non_blocking=True)
-            return rec_out
-        return g['rec'].clone()
+        return self._graph_result(g, rec_out)
 
     @torch.no_grad()
     def evaluate(self, eval_data, load_best_model=True, model_file=None, show_progress=False):
@@ -802,9 +869,23 @@ class ACSASRecTrainer(object):
         self.model.eval()
         self.tot_item_num = eval_data.dataset.item_num
         sampler = getattr(eval_data, 'neg_sampler', None)      # data.NegSampleEvalDataLoader: sampled-candidate evaluation
-        recs = [self.eval_batch(b, neg_sampler=sampler, neg_num=getattr(eval_data, 'neg_num', 0)) for b in eval_data]
-        rec = torch.cat(recs, dim=0).cpu().numpy()
-        return self.evaluator.evaluate(rec)
+        ev = self.evaluator
+        if ev.need_items and sampler is not None:
+            raise NotImplementedError('the item-distribution metrics (ItemCoverage, AveragePopularity, GiniIndex, ShannonEntropy, '
+                                      'TailPercentage) are not available in sampled evaluation (eval_args.mode uniN / popN): '
+                                      'use full-sort evaluation for them')
+        if ev.need_item_counts and self.item_counts is None:
+            raise ValueError('AveragePopularity / TailPercentage need the training item counts: call fit(train_data) first, or '
+                             'trainer.set_item_counts(train_data) (a training loader, its dataset, or an array of counts by item id)')
+        if not (ev.need_counts or ev.need_items):
+            recs = [self.eval_batch(b, neg_sampler=sampler, neg_num=getattr(eval_data, 'neg_num', 0)) for b in eval_data]
+            rec = torch.cat(recs, dim=0).cpu().numpy()
+            return ev.evaluate(rec)
+        need = (ev.need_counts, ev.need_items)
+        parts = [self.eval_batch(b, neg_sampler=sampler, neg_num=getattr(eval_data, 'neg_num', 0), need=need) for b in eval_data]
+        cat = [torch.cat([p[i] for p in parts], dim=0).cpu().numpy() if parts[0][i] is not None else None for i in range(4)]
+        rec, counts, user_len, items = cat
+        return ev.evaluate(rec, counts=counts, user_len=user_len, items=items, n_items=self._n_items(), item_counts=self.item_counts)
 
 
 class AcBERT4RecTrainer(ACSASRecTrainer):

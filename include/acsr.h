@@ -267,6 +267,25 @@ int acsr_logits_topk_partial_ws(const float* out, const float* table, int M, int
 int acsr_topk_merge(const float* partial_val, const int64_t* partial_idx, int M, int n_parts, int k,
                     const int64_t* positive, float* topk_val, int64_t* topk_idx, int32_t* rec_topk, void* stream);
 
+/* ---- rank counts of the positive for GAUC (evaluator/metrics.py GAUC, collector.py rec.meanrank) ----
+ * The reference sorts the whole [B, V] score matrix to find the positive's average rank.  Here the top-k kernels count, per row,
+ * G = #items scoring strictly above s_pos and E = #items scoring equal to it, column 0 (when skipped) and the positive's own column
+ * excluded, so the counts do not depend on how a path rounds the positive's own score.  s_pos = pos_score[m] comes from
+ * acsr_row_dot (one fp32 dot in a fixed order, as the CE target logit); the 1-based average rank is G + (E + 2) / 2.
+ * acsr_row_dot: dot[m] = out[m] . table[ids[m] - idx_offset] when 0 <= ids[m] - idx_offset < V, else 0 (the shards' answers sum). */
+int acsr_row_dot(const float* out, const float* table, const int64_t* ids, int M, int d, int64_t V, int64_t idx_offset, float* dot,
+                 void* stream);
+/* acsr_logits_topk_partial_ws that also writes partial_counts [M, acsr_logits_num_chunks(M, V), 2] int32 = (G, E) of each chunk
+ * (zero for the lists no CTA produces); positive [M] = item ids (idx_offset is subtracted, as for the output ids).  Plain stores:
+ * deterministic.  Every score is counted, including tiles the shared bound lets skip the candidate bookkeeping. */
+int acsr_logits_topk_rank_partial(const float* out, const float* table, int M, int64_t V, int d, int passes, int k, int64_t idx_offset,
+                                  int skip_col0, const int64_t* positive, const float* pos_score, float* partial_val,
+                                  int64_t* partial_idx, int32_t* partial_counts, int32_t* row_bound, void* stream);
+/* acsr_topk_merge that also sums partial_counts [M, n_count_parts, 2] into counts [M, 2]; positive may be NULL (no rec_topk). */
+int acsr_topk_merge_rank(const float* partial_val, const int64_t* partial_idx, int M, int n_parts, int k,
+                         const int64_t* positive, const int32_t* partial_counts, int n_count_parts, float* topk_val,
+                         int64_t* topk_idx, int32_t* rec_topk, int32_t* counts, void* stream);
+
 /* dense variant for catalogues of at most acsr_topk_select_max_items() items (one row's scores as 32-bit keys in shared
  * memory): top-k of every row of scores [M, ld] (first V columns) by a 4-pass radix select + a sort of the k winners.
  * skip_col0 excludes column 0 (trainer.py:942); item id = column + idx_offset.  Together with acsr_logits_store this is the
@@ -275,6 +294,11 @@ int acsr_topk_merge(const float* partial_val, const int64_t* partial_idx, int M,
 int acsr_topk_select_max_items(void);
 int acsr_topk_select(const float* scores, int M, int64_t V, int64_t ld, int k, int skip_col0, int64_t idx_offset,
                      const int64_t* positive, float* topk_val, int64_t* topk_idx, int32_t* rec_topk, void* stream);
+/* acsr_topk_select that also counts counts [M, 2] = (G, E) against pos_score over the row in shared memory (see acsr_row_dot);
+ * positive is required (its column, id - idx_offset, is not counted). */
+int acsr_topk_select_rank(const float* scores, int M, int64_t V, int64_t ld, int k, int skip_col0, int64_t idx_offset,
+                          const int64_t* positive, const float* pos_score, float* topk_val, int64_t* topk_idx, int32_t* rec_topk,
+                          int32_t* counts, void* stream);
 
 /* Fold the attack transforms into the first projections (layers.py:658-659, 687-689) so that the five projections of a layer
  * read the same input and run as ONE batched GEMM: out_W [5,d,d] / out_b [5,d] = {Wq, Wk, Wv, Waq.Wq, Wak.Wk} and
@@ -511,6 +535,10 @@ int acsr_neg_sample(const int64_t* users, const int64_t* positives, const int64_
 int acsr_candidate_rank_max_candidates(void);
 int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
                         int32_t* rec, float* scores, void* stream);
+/* the same plus counts [M, 3] int32 = (distinct negatives scoring above the positive, distinct negatives tied with it, distinct
+ * candidates including the positive): GAUC's rank inputs and user_len, the number of finite entries of the scattered row. */
+int acsr_candidate_rank_counts(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
+                               int32_t* rec, float* scores, int32_t* counts, void* stream);
 
 /* ---- K13: fused Adam over one flat fp32 buffer (trainer/trainer.py:614-615,687) ---------
  * torch.optim.Adam semantics (no amsgrad); step_count device int64[1], incremented by the call. */
