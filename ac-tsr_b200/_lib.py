@@ -129,18 +129,6 @@ def _ab_linear_tok(a):
     return 4 * batch * (rows * K + rows * N * (2 if acc else 1) + N * K)
 
 
-def _ab_linear_tok_actbwd(a):
-    # (X, ldx, rows, K, W, w_sn, w_sk, wkb, N, Z, z_rows, ...): X, W, Z in; Y out
-    rows, K, N = a[2], a[3], a[8]
-    return 4 * (rows * K + N * K + 2 * rows * N)
-
-
-def _ab_dense_fwd(a):
-    # (ctx, res, rows, res_rows, d, I, ...): ctx + residual in; hz, h, z2, out [rows,64], z1, a1 [rows,I], stats out; weights in
-    rows, res_rows, d, I = a[2], a[3], a[4], a[5]
-    return 4 * (rows * d + min(rows, res_rows) * d + 4 * rows * d + 2 * rows * I + 4 * rows + d * d + 2 * d * I)
-
-
 def _ab_dense_bwd(a):
     # (d_out, rows, act_rows, res_rows, param_rows, d, I, ...): d_out, the saved z2 / h / hz [., 64], z1 [., I], stats and the residual
     # in; d_xres, d_ctx [rows, 64] out, d_z2 / d_hz [param_rows, 64] and d_z1 [param_rows, I] out; weights in
@@ -207,7 +195,7 @@ def _ab_candidate_rank_counts(a):
 
 
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
-ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_ragged': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl, 'acsr_dense_fwd': _ab_dense_fwd, 'acsr_linear_tok_actbwd': _ab_linear_tok_actbwd,
+ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl,
               'acsr_proj_input_grad': _ab_proj_input_grad, 'acsr_dense_bwd': _ab_dense_bwd,
               'acsr_linear_wgrad': _ab_linear_wgrad, 'acsr_linear_wgrad_batched': _ab_linear_wgrad_batched,
               'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank,

@@ -1,4 +1,4 @@
-// Backward of an encoder layer's dense part after its attention (the reverse of dense_fwd.cu's chain) as ONE tcgen05 launch,
+// Backward of an encoder layer's dense part after its attention (layers.py:676-684, 790-798) as ONE tcgen05 launch,
 // hidden size 64, inner size a multiple of 64 up to 256.  Per 128-token tile:
 //   1. FFN LayerNorm backward: d_out -> d_pre_f (the residual part of d_h) and d_z2 = d_pre_f * mask_f
 //   2. per 64-wide chunk c of the inner axis: acc_c = d_z2.W2[:, c] ; d_z1_c = acc_c * act'(z1_c + b1_c) ; acc_h += d_z1_c.W1[c, :]
@@ -8,7 +8,7 @@
 // critical path of every non-last layer's backward, and d_a1 / d_z1 ([rows, I] each) made round trips through L2 although only
 // rows < param_rows of d_z2 / d_z1 / d_hz are read afterwards (by the weight gradients).  Here the intermediates stay in TENSOR
 // MEMORY: each epilogue leaves its result split into hi / lo TF32 halves with tcgen05.st and the next MMA reads it as its A
-// operand (TS form, as in dense_fwd.cu / proj_bwd.cu).  Bias gradients are not computed here: the weight-gradient launch takes
+// operand (TS form, as in logits_bwd.cu / proj_bwd.cu).  Bias gradients are not computed here: the weight-gradient launch takes
 // them as column sums of its left operand (d_z2, d_z1, d_hz).
 //
 // TMEM columns (128 lanes x 512, one CTA per SM):

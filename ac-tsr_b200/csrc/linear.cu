@@ -131,15 +131,12 @@ linear_wgrad_kernel(const float* __restrict__ dY, const float* __restrict__ X, i
 constexpr int kFoldRows = 8;       // output rows per CTA
 __global__ void __launch_bounds__(256) fold_attack_weights_kernel(const float* __restrict__ Wqkv, const float* __restrict__ bqkv,
                                                                   const float* __restrict__ Waqk, const float* __restrict__ baqk, int d,
-                                                                  const float* __restrict__ Wg, const float* __restrict__ bg, int Lg,
                                                                   float* __restrict__ out_W, float* __restrict__ out_b) {
   extern __shared__ float fsm[];                    // B [d][d], A rows [kFoldRows][d], b1 [d]
   // (no early programmatic-launch trigger: the folded weights it writes are registered as static, see acsr_register_static)
   pdl_wait();
-  // slot 5 (optional): the gate of combine_option 'gate' (layers.py:887: gate(mixed_q)) folded the same way, Wg.Wq [Lg, d] and
-  // Wg.bq + bg, so the gate logits are a sixth (Lg-feature) problem of the projection launch
   const int slot = blockIdx.y, r0 = blockIdx.x * kFoldRows;
-  const int nr = min(kFoldRows, (slot == 5 ? Lg : d) - r0);
+  const int nr = min(kFoldRows, d - r0);
   if (nr <= 0) return;
   float* oW = out_W + (long long)slot * d * d + (long long)r0 * d;
   float* ob = out_b + (long long)slot * d + r0;
@@ -151,9 +148,9 @@ __global__ void __launch_bounds__(256) fold_attack_weights_kernel(const float* _
   float* sB = fsm;
   float* sA = sB + d * d;
   float* sb1 = sA + kFoldRows * d;
-  const int first = slot == 5 ? 0 : slot - 3;                                     // the projection folded in: Wq (slots 3, 5) or Wk (slot 4)
-  const float* A = (slot == 5 ? Wg : Waqk + (long long)(slot - 3) * d * d) + (long long)r0 * d;     // rows r0.. of the second linear map
-  const float* b2 = slot == 5 ? bg : baqk + (slot - 3) * d;
+  const int first = slot - 3;                                                     // the projection folded in: Wq (slot 3) or Wk (slot 4)
+  const float* A = Waqk + (long long)first * d * d + (long long)r0 * d;           // rows r0.. of the second linear map
+  const float* b2 = baqk + first * d;
   const float* Bm = Wqkv + (long long)first * d * d;
   for (int e = threadIdx.x; e < d * d; e += blockDim.x) sB[e] = Bm[e];
   for (int e = threadIdx.x; e < nr * d; e += blockDim.x) sA[e] = A[e];
@@ -179,21 +176,15 @@ using namespace acsr;
 
 extern "C" int acsr_fold_attack_weights(const float* Wqkv, const float* bqkv, const float* Waqk, const float* baqk, int d, float* out_W,
                                         float* out_b, void* stream) {
-  return acsr_fold_projection_weights(Wqkv, bqkv, Waqk, baqk, d, nullptr, nullptr, 0, out_W, out_b, stream);
-}
-
-extern "C" int acsr_fold_projection_weights(const float* Wqkv, const float* bqkv, const float* Waqk, const float* baqk, int d,
-                                            const float* Wg, const float* bg, int Lg, float* out_W, float* out_b, void* stream) {
   ACSR_REQUIRE(Wqkv && bqkv && Waqk && baqk && out_W && out_b && d > 0 && d <= 1024, "fold_attack_weights: bad arguments");
-  ACSR_REQUIRE(Lg == 0 || (Wg && bg && Lg > 0 && Lg <= d), "fold_projection_weights: gate width %d (1..%d)", Lg, d);
   ACSR_REQUIRE(d <= 128, "fold_attack_weights: hidden size %d > 128", d);
   const size_t smem = (size_t)(d * d + kFoldRows * d + d) * sizeof(float);
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(fold_attack_weights_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) { set_error("fold_attack_weights: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
   }
-  launch_pdl(fold_attack_weights_kernel, dim3((d + kFoldRows - 1) / kFoldRows, Lg > 0 ? 6 : 5), dim3(256), smem, (cudaStream_t)stream, Wqkv,
-             bqkv, Waqk, baqk, d, Wg, bg, Lg, out_W, out_b);
+  launch_pdl(fold_attack_weights_kernel, dim3((d + kFoldRows - 1) / kFoldRows, 5), dim3(256), smem, (cudaStream_t)stream, Wqkv, bqkv,
+             Waqk, baqk, d, out_W, out_b);
   return check_launch("fold_attack_weights");
 }
 

@@ -1,7 +1,7 @@
 // Encoder GEMMs  Y[T,N] = epilogue(X[T,K] . W^T)  on the 5th-gen tensor cores (tcgen05), 3xTF32.
 //
 // Replaces the nn.Linear forward / input-gradient GEMMs of layers.py:658-659, 680, 687-689, 791-794, 887
-// and fuses what follows them in the reference: the bias add, bias + activation (layers.py:776-792) and
+// and fuses what follows them in the reference: the bias add and
 // bias + dropout + residual + LayerNorm (layers.py:681-683, 794-796).
 //
 // Token rows are the UMMA M axis: a 128-token tile of X is split by four loader warps into (hi, lo)
@@ -11,7 +11,7 @@
 // is split once per CTA and stays in shared memory.  One thread issues tcgen05.mma.kind::tf32
 // 128 x N x 8 for {lo.hi, hi.lo, hi.hi} (3xTF32: fp32-level accuracy) into a double-buffered TMEM
 // accumulator; four epilogue warps read it back with tcgen05.ld 32x32b, so ONE THREAD OWNS ONE TOKEN
-// ROW: bias, activation, dropout, residual and the LayerNorm statistics are thread-private (no
+// ROW: bias, dropout, residual and the LayerNorm statistics are thread-private (no
 // shuffles), and the row is written with 16-byte stores.  CTAs are persistent over token tiles; the
 // X operand is double buffered when shared memory allows, so loading/splitting tile t+1 overlaps the
 // MMAs and the epilogue of tile t.
@@ -26,7 +26,7 @@ constexpr int kLtKB = 64;            // K block (floats) held per A buffer
 constexpr int kLtABytes = kLtBM * kLtKB * 4;     // 32 KB per (hi | lo)
 constexpr int kLtTmemCols = 256;     // 2 accumulator stages x <= 128 columns
 
-enum { EPI_PLAIN = 0, EPI_ACT = 1, EPI_BDRL = 2, EPI_ACTBWD = 3 };
+enum { EPI_PLAIN = 0, EPI_BDRL = 2 };
 
 struct LinTokParams {
   const float* X; long long ldx, xkb; long long rows; int K;       // element (r, k) = X[(k / 64) * xkb + r * ldx + k % 64]
@@ -35,15 +35,12 @@ struct LinTokParams {
   float* Y; long long ldy; int accumulate;
   int batch; long long bx, bw, bb, by;                               // per-problem strides of a batched launch (blockIdx.z)
   int passes, epi;
-  // EPI_ACT
-  int act; float* Y2;
   // EPI_BDRL
   const float* res; long long res_rows; const float *ln_w, *ln_b; float eps, p; const float* mask;
   const RngState* rng; uint32_t rng_stream; float* out; float* stats;
   // plan
   int m_tiles, n_blocks, NB, KBn, nbuf;                              // NB: features per CTA (multiple of 16), KBn = ceil(K/64)
   int w_static;                                                      // W / bias are registered parameters (acsr_register_static): staged before griddepcontrol.wait
-  int last_n; long long last_ldy;                                    // > 0: the LAST problem of a batched launch has this many features / this row stride of Y
 };
 
 struct LtSmem {
@@ -80,9 +77,6 @@ __global__ void __launch_bounds__(kLtThreads, 1) linear_tok_kernel(const LinTokP
   const float* biasp = p.bias ? p.bias + bz * p.bb : nullptr;
   float* Yp = p.Y + bz * p.by;
   const int NB = p.NB, KBn = p.KBn, nbuf = p.nbuf;
-  const bool is_last = p.last_n > 0 && bz == p.batch - 1;
-  const int Neff = is_last ? p.last_n : p.N;                      // (the gate logits ride along with the five projections: 50 features, row stride 50)
-  const long long ldy_eff = is_last ? p.last_ldy : p.ldy;
   const int b_bytes = NB * KBn * kLtKB * 4;
   uint8_t* sBhi = smem;
   uint8_t* sBlo = smem + b_bytes;
@@ -144,7 +138,7 @@ __global__ void __launch_bounds__(kLtThreads, 1) linear_tok_kernel(const LinTokP
         const int n = item % NB, kc = item / NB;
         const int kb = kc / (kLtKB / 4), kcl = kc % (kLtKB / 4);
         const int k0 = kb * kLtKB + kcl * 4;
-        if (n0 + n < Neff && k0 < p.K) {
+        if (n0 + n < p.N && k0 < p.K) {
           const float* w = Wp + kb * p.wkb + (long long)(n0 + n) * p.w_sn + (long long)(kcl * 4) * p.w_sk;
           if (vec_ok && k0 + 4 <= p.K) xs[u] = __ldg(reinterpret_cast<const float4*>(w));
           else {
@@ -164,7 +158,7 @@ __global__ void __launch_bounds__(kLtThreads, 1) linear_tok_kernel(const LinTokP
         lt_split_store(Bhi + off, Blo + off, xs[u]);
       }
     }
-    for (int i = sid; i < 128; i += kStagers) sBias[i] = (biasp != nullptr && n0 + i < Neff) ? biasp[n0 + i] : 0.f;
+    for (int i = sid; i < 128; i += kStagers) sBias[i] = (biasp != nullptr && n0 + i < p.N) ? biasp[n0 + i] : 0.f;
   }
   if (stage_early) pdl_wait();
   fence_proxy_async();
@@ -253,7 +247,7 @@ __global__ void __launch_bounds__(kLtThreads, 1) linear_tok_kernel(const LinTokP
     const int quarter = warp & 3;                 // TMEM lane quarter this warp may access
     const int row = quarter * 32 + lane;
     const uint32_t t_lane = tmem_base + ((uint32_t)(quarter * 32) << 16);
-    const int ncols = min(NB, Neff - n0);         // valid features of this block
+    const int ncols = min(NB, p.N - n0);          // valid features of this block
     int it = 0;
     for (int tile = blockIdx.x; tile < p.m_tiles; tile += gridDim.x, ++it) {
       const int ts = it & 1;
@@ -322,61 +316,30 @@ __global__ void __launch_bounds__(kLtThreads, 1) linear_tok_kernel(const LinTokP
           tmem_ld32(t_lane + ts * NB + cc * 32, v);
           const int nvalid = min(32, ncols - cc * 32);
           if (row_ok) {
-            float* y = Yp + grow * ldy_eff + n0 + cc * 32;
+            float* y = Yp + grow * p.ldy + n0 + cc * 32;
             const bool vec = nvalid == 32 && ((reinterpret_cast<uintptr_t>(y) & 15) == 0);
-            if (EPI == EPI_ACTBWD) {
-              // Y = acc * act'(Z + bias): the activation backward (layers.py:776-792) applied to the input gradient d_a1 = d_z2.W2
-              // while it is still in registers; Z = the saved pre-activation GEMM output (p.res, rows repeat with period res_rows)
-              const float* z = p.res + (grow % p.res_rows) * p.ldy + n0 + cc * 32;
-              if (vec && ((reinterpret_cast<uintptr_t>(z) & 15) == 0)) {
+            if (vec) {
+              float4 old[8];
+              if (p.accumulate) {
 #pragma unroll
-                for (int i = 0; i < 32; i += 4) {
-                  const float4 z4 = __ldg(reinterpret_cast<const float4*>(z + i));
-                  *reinterpret_cast<float4*>(y + i) = make_float4(v[i] * act_bwd(p.act, z4.x + sBias[cc * 32 + i]), v[i + 1] * act_bwd(p.act, z4.y + sBias[cc * 32 + i + 1]),
-                                                                  v[i + 2] * act_bwd(p.act, z4.z + sBias[cc * 32 + i + 2]), v[i + 3] * act_bwd(p.act, z4.w + sBias[cc * 32 + i + 3]));
-                }
-              } else {
-#pragma unroll
-                for (int i = 0; i < 32; ++i) if (i < nvalid) y[i] = v[i] * act_bwd(p.act, __ldg(z + i) + sBias[cc * 32 + i]);
+                for (int i = 0; i < 8; ++i) old[i] = *reinterpret_cast<const float4*>(y + 4 * i);
               }
-            } else if (EPI == EPI_ACT) {
-              // Y = raw GEMM output (pre-bias, saved for the backward), Y2 = act(Y + bias)
-              float* y2 = p.Y2 + bz * p.by + grow * p.ldy + n0 + cc * 32;
-              if (vec) {
 #pragma unroll
-                for (int i = 0; i < 32; i += 4) {
-                  *reinterpret_cast<float4*>(y + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
-                  *reinterpret_cast<float4*>(y2 + i) = make_float4(act_fwd(p.act, v[i] + sBias[cc * 32 + i]), act_fwd(p.act, v[i + 1] + sBias[cc * 32 + i + 1]),
-                                                                   act_fwd(p.act, v[i + 2] + sBias[cc * 32 + i + 2]), act_fwd(p.act, v[i + 3] + sBias[cc * 32 + i + 3]));
-                }
-              } else {
-#pragma unroll
-                for (int i = 0; i < 32; ++i) if (i < nvalid) { y[i] = v[i]; y2[i] = act_fwd(p.act, v[i] + sBias[cc * 32 + i]); }
+              for (int i = 0; i < 8; ++i) {
+                float4 o = make_float4(v[4 * i] + sBias[cc * 32 + 4 * i], v[4 * i + 1] + sBias[cc * 32 + 4 * i + 1],
+                                       v[4 * i + 2] + sBias[cc * 32 + 4 * i + 2], v[4 * i + 3] + sBias[cc * 32 + 4 * i + 3]);
+                if (p.accumulate) { o.x += old[i].x; o.y += old[i].y; o.z += old[i].z; o.w += old[i].w; }
+                *reinterpret_cast<float4*>(y + 4 * i) = o;
               }
             } else {
-              if (vec) {
-                float4 old[8];
-                if (p.accumulate) {
+              float old[32];
+              if (p.accumulate) {
 #pragma unroll
-                  for (int i = 0; i < 8; ++i) old[i] = *reinterpret_cast<const float4*>(y + 4 * i);
-                }
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                  float4 o = make_float4(v[4 * i] + sBias[cc * 32 + 4 * i], v[4 * i + 1] + sBias[cc * 32 + 4 * i + 1],
-                                         v[4 * i + 2] + sBias[cc * 32 + 4 * i + 2], v[4 * i + 3] + sBias[cc * 32 + 4 * i + 3]);
-                  if (p.accumulate) { o.x += old[i].x; o.y += old[i].y; o.z += old[i].z; o.w += old[i].w; }
-                  *reinterpret_cast<float4*>(y + 4 * i) = o;
-                }
-              } else {
-                float old[32];
-                if (p.accumulate) {
-#pragma unroll
-                  for (int i = 0; i < 32; ++i) old[i] = i < nvalid ? y[i] : 0.f;
-                }
-#pragma unroll
-                for (int i = 0; i < 32; ++i)
-                  if (i < nvalid) y[i] = v[i] + sBias[cc * 32 + i] + (p.accumulate ? old[i] : 0.f);
+                for (int i = 0; i < 32; ++i) old[i] = i < nvalid ? y[i] : 0.f;
               }
+#pragma unroll
+              for (int i = 0; i < 32; ++i)
+                if (i < nvalid) y[i] = v[i] + sBias[cc * 32 + i] + (p.accumulate ? old[i] : 0.f);
             }
           }
         }
@@ -433,17 +396,8 @@ extern "C" {
 int acsr_linear_tok(const float* X, int64_t ldx, int64_t x_kblock_stride, int64_t rows, int K, const float* W, int64_t w_stride_n,
                     int64_t w_stride_k, int64_t w_kblock_stride, int N, const float* bias, int accumulate, float* Y, int64_t ldy,
                     int batch, int64_t stride_x, int64_t stride_w, int64_t stride_bias, int64_t stride_y, int passes, void* stream) {
-  return acsr_linear_tok_ragged(X, ldx, x_kblock_stride, rows, K, W, w_stride_n, w_stride_k, w_kblock_stride, N, bias, accumulate, Y, ldy,
-                                batch, stride_x, stride_w, stride_bias, stride_y, 0, 0, passes, stream);
-}
-
-int acsr_linear_tok_ragged(const float* X, int64_t ldx, int64_t x_kblock_stride, int64_t rows, int K, const float* W, int64_t w_stride_n,
-                           int64_t w_stride_k, int64_t w_kblock_stride, int N, const float* bias, int accumulate, float* Y, int64_t ldy,
-                           int batch, int64_t stride_x, int64_t stride_w, int64_t stride_bias, int64_t stride_y, int last_n,
-                           int64_t last_ldy, int passes, void* stream) {
   ACSR_REQUIRE(X && W && Y, "linear_tok: NULL pointer");
   ACSR_REQUIRE(rows >= 0 && N > 0 && K > 0 && batch > 0 && batch < 65536 && ldy >= N, "linear_tok: bad sizes");
-  ACSR_REQUIRE(last_n == 0 || (last_n > 0 && last_n <= N && last_ldy >= last_n && batch > 1), "linear_tok: bad ragged last problem");
   ACSR_REQUIRE(passes == 1 || passes == 3, "linear_tok: passes must be 1 or 3");
   if (rows == 0) return ACSR_OK;
   LinTokParams p = {};
@@ -451,42 +405,9 @@ int acsr_linear_tok_ragged(const float* X, int64_t ldx, int64_t x_kblock_stride,
   p.W = W; p.w_sn = w_stride_n; p.w_sk = w_stride_k; p.wkb = w_kblock_stride; p.N = N;
   p.bias = bias; p.accumulate = accumulate; p.Y = Y; p.ldy = ldy;
   p.batch = batch; p.bx = stride_x; p.bw = stride_w; p.bb = stride_bias; p.by = stride_y;
-  p.passes = passes; p.epi = EPI_PLAIN; p.last_n = last_n; p.last_ldy = last_ldy;
+  p.passes = passes; p.epi = EPI_PLAIN;
   p.w_static = is_static_memory(p.W) && (p.bias == nullptr || is_static_memory(p.bias));
   return lt_launch<EPI_PLAIN>(p, (cudaStream_t)stream, "linear_tok");
-}
-
-int acsr_linear_tok_act(const float* X, int64_t ldx, int64_t rows, int K, const float* W, int N, const float* bias, int act,
-                        float* Z, float* A, int64_t ldy, int passes, void* stream) {
-  ACSR_REQUIRE(X && W && Z && A, "linear_tok_act: NULL pointer");
-  ACSR_REQUIRE(rows >= 0 && N > 0 && K > 0 && ldy >= N, "linear_tok_act: bad sizes");
-  ACSR_REQUIRE(act >= 0 && act <= 4, "linear_tok_act: unknown activation %d", act);
-  ACSR_REQUIRE(passes == 1 || passes == 3, "linear_tok_act: passes must be 1 or 3");
-  if (rows == 0) return ACSR_OK;
-  LinTokParams p = {};
-  p.X = X; p.ldx = ldx; p.xkb = kLtKB; p.rows = rows; p.K = K;
-  p.W = W; p.w_sn = K; p.w_sk = 1; p.wkb = kLtKB; p.N = N;
-  p.bias = bias; p.Y = Z; p.Y2 = A; p.ldy = ldy; p.act = act;
-  p.batch = 1; p.passes = passes; p.epi = EPI_ACT;
-  p.w_static = is_static_memory(p.W) && (p.bias == nullptr || is_static_memory(p.bias));
-  return lt_launch<EPI_ACT>(p, (cudaStream_t)stream, "linear_tok_act");
-}
-
-int acsr_linear_tok_actbwd(const float* X, int64_t ldx, int64_t rows, int K, const float* W, int64_t w_stride_n, int64_t w_stride_k,
-                           int64_t w_kblock_stride, int N, const float* Z, int64_t z_rows, const float* bias, int act, float* Y,
-                           int passes, void* stream) {
-  ACSR_REQUIRE(X && W && Z && Y, "linear_tok_actbwd: NULL pointer");
-  ACSR_REQUIRE(rows >= 0 && N > 0 && K > 0 && z_rows > 0, "linear_tok_actbwd: bad sizes");
-  ACSR_REQUIRE(act >= 0 && act <= 4, "linear_tok_actbwd: unknown activation %d", act);
-  ACSR_REQUIRE(passes == 1 || passes == 3, "linear_tok_actbwd: passes must be 1 or 3");
-  if (rows == 0) return ACSR_OK;
-  LinTokParams p = {};
-  p.X = X; p.ldx = ldx; p.xkb = kLtKB; p.rows = rows; p.K = K;
-  p.W = W; p.w_sn = w_stride_n; p.w_sk = w_stride_k; p.wkb = w_kblock_stride; p.N = N;
-  p.bias = bias; p.Y = Y; p.ldy = N; p.act = act; p.res = Z; p.res_rows = z_rows;
-  p.batch = 1; p.passes = passes; p.epi = EPI_ACTBWD;
-  p.w_static = is_static_memory(p.W) && (p.bias == nullptr || is_static_memory(p.bias));
-  return lt_launch<EPI_ACTBWD>(p, (cudaStream_t)stream, "linear_tok_actbwd");
 }
 
 int acsr_linear_tok_bdrl(const float* X, int64_t ldx, int64_t rows, int K, const float* W, const float* bias, const float* res,

@@ -62,21 +62,10 @@ static inline void logits_plan(LogitsParams& p, int batch = 1) {
   p.n_chunks = nc;
 }
 
-// top-k mode: pval / pidx hold n_slots = acsr_logits_num_chunks lists per row; the kernel may fill fewer (n_chunks <= n_slots,
-// ACSR_TOPK_MIN_TILES catalogue tiles per CTA at least) and pads the rest.  Measured on B200 (scripts/topk_micro.py): the first
-// tile of a CTA (filling the k-best lists) costs as much as many later ones, so spreading over all SMs (1) wins at every size.
-static inline void logits_plan_topk(LogitsParams& p) {
-  p.n_slots = p.n_chunks;
-  static int min_tiles = 0;
-  if (min_tiles == 0) {
-    const char* e = getenv("ACSR_TOPK_MIN_TILES");       // tuning knob
-    min_tiles = e ? atoi(e) : 1;
-    if (min_tiles < 1) min_tiles = 1;
-  }
-  int nc = (p.n_tiles + min_tiles - 1) / min_tiles;
-  if (nc < 1) nc = 1;
-  if (nc < p.n_chunks) p.n_chunks = nc;
-}
+// top-k mode: pval / pidx hold n_slots = acsr_logits_num_chunks lists per row, one per CTA of the row tile.  The CTAs spread over
+// all SMs even when that leaves few catalogue tiles each: measured on B200 (scripts/topk_micro.py), a CTA's first tile (filling the
+// k-best lists) costs as much as many later ones, so fewer, longer CTAs lose at every size.
+static inline void logits_plan_topk(LogitsParams& p) { p.n_slots = p.n_chunks; }
 
 // gemm_ks.cu: logits for hidden sizes other than 64 on the K-streamed tcgen05 GEMM (mode = ACSR_EPI_STORE / _CE / _CE_GRAD)
 int gemm_logits(int mode, const float* out, const float* table, int M, long long V, int d, int passes, float* C, long long ldc,

@@ -9,7 +9,7 @@
 //   stage 1: acc_q = d_aq.Waq (+ d_gl.Wg), acc_k = d_ak.Wak (3xTF32, in TMEM); the epilogue adds d_mq / d_mk in exact fp32 (the
 //            add of linear_tok's accumulate epilogue), writes rows < rows_keep back into d_qkv (the Q / K weight gradients read
 //            them) and leaves the sums, split into hi / lo, in TMEM with tcgen05.st;
-//   stage 2: d_x += [d_mq | d_mk | d_mv] . [Wq; Wk; Wv], the A operand read from TMEM (TS form, as in logits_bwd.cu / dense_fwd.cu).
+//   stage 2: d_x += [d_mq | d_mk | d_mv] . [Wq; Wk; Wv], the A operand read from TMEM (TS form, as in logits_bwd.cu / dense_bwd.cu).
 // The A operands of stage 1 are streamed through TMEM too: the six weight blocks (read transposed, split into hi / lo, canonical
 // K-major UMMA layout) fill 192 KB of shared memory and leave no room for an A tile there.
 //

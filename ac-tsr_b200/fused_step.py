@@ -46,45 +46,23 @@ class FusedTrainStep(object):
         self.m, self.opt = model, optimizer
         self.buf = {}
         self.vp = None            # dist.VocabParallel when the logits are sharded over ranks
-        # d == 64: every encoder GEMM runs on the tcgen05 token-tile kernel (3xTF32) with its epilogue fused;
-        # other widths stay library GEMMs + the row-wise epilogue kernels
-        self.tc = (bool(getattr(model, 'tc_linear', True)) and model.hidden_size == 64 and model.inner_size <= 256
-                   and model.inner_size % 4 == 0)
-        # every other width (d = 128 of the shipped yelp / sports / toys configs, d = 256 of BASELINE config #5): the K-streamed
-        # tcgen05 kernel (gemm_ks.cu) through problem lists.  At every width the weight gradients of a layer go through it as
-        # ONE launch (token axis on K, split over the CTAs).  No library GEMM is left on the step.
-        self.tc_wgrad = bool(getattr(model, 'tc_wgrad', True))
+        # d == 64: every encoder GEMM runs on the tcgen05 token-tile kernel (3xTF32) with its epilogue fused.  Every other width
+        # (d = 128 of the shipped yelp / sports / toys configs, d = 256 of BASELINE config #5): the K-streamed tcgen05 kernel
+        # (gemm_ks.cu) through problem lists.  At every width the weight gradients of a layer go through it as ONE launch (token
+        # axis on K, split over the CTAs).  No library GEMM is left on the step.
+        self.tc = model.hidden_size == 64 and model.inner_size <= 256 and model.inner_size % 4 == 0
         self.passes = 3                                   # encoder GEMMs: 3xTF32 (fp32-level accuracy)
-        self.overlap_wgrad = bool(getattr(model, 'overlap_wgrad', True))
+        self.overlap_wgrad = True                         # weight gradients on a second stream next to the input-gradient chain
         self.n_branches = int(getattr(model, 'step_branches', 1))
         self._streams = {}
-        self.compact_last = bool(getattr(model, 'compact_last', True))   # last layer's dense part on the len-1 rows only
-        import os
-        self.order_side = os.environ.get('ACSR_ORDER_SIDE', '1') == '1'     # sequence ordering next to, not in front of, the embedding
-        self.fold_attack = os.environ.get('ACSR_FOLD_ATTACK', '1') == '1'   # attack transforms folded into the Q/K/V launch (forward)
-        # ... and the gate logits as a sixth problem of that launch: correct (tests run it), but measured no faster on B200 (0.742 vs
-        # 0.735 ms per C2 step: the sixth problem adds a round to the persistent CTAs, the separate 100-CTA launch hides under PDL) -> off
-        self.fold_gate = os.environ.get('ACSR_FOLD_GATE', '0') == '1'
-        self.pdl = bool(getattr(model, 'pdl', True))            # programmatic dependent launch between the step's kernels
-        # last layer's dense part on the compact rows as ONE launch per direction (acsr_tail_fwd / _bwd); ACSR_TAIL_FUSED=0: six launches
-        self.tail_fused = (self.tc and model.inner_size % 16 == 0 and os.environ.get('ACSR_TAIL_FUSED', '1') == '1')
-        # activation backward inside the d_a1 GEMM's TMEM epilogue (acsr_linear_tok_actbwd): correct (tests run it) but SLOWER on B200 --
-        # 65 us against 22 + 21 us for GEMM + row-wise kernel: four epilogue warps (one thread per token row) cannot issue the erf
-        # derivative of 128 x 256 elements fast enough -> off
-        self.fuse_act_bwd = os.environ.get('ACSR_FUSE_ACT_BWD', '0') == '1'
-        # out-projection + LayerNorm + feed-forward + LayerNorm of a token tile as ONE tcgen05 kernel (acsr_dense_fwd: activations stay
-        # in tensor memory between the GEMMs).  Correct (tests run it) and two launches fewer, but NOT faster on B200: 54.7 us against
-        # 13 + 17 + 5 + 24 us for the four launches it replaces, step 0.7233 vs 0.7177 ms.  ncu (profiles/r02_ncu_full_dense.txt): IPC
-        # 0.37, 17 % warps active -- the chain load -> MMA -> LayerNorm epilogue -> 4 x (MMA -> erf epilogue -> MMA) -> LayerNorm epilogue
-        # is serial inside a tile and each per-row epilogue (Philox + LayerNorm / erf, one warp per SM sub-partition) costs microseconds;
-        # separate launches spread the same epilogues over more CTAs.  Off by default (ACSR_DENSE_FUSED=1 turns it on).
-        self.dense_fused = (self.tc and model.inner_size % 64 == 0 and os.environ.get('ACSR_DENSE_FUSED', '0') == '1')
+        self.pdl = True                                   # programmatic dependent launch between the step's kernels
+        # last layer's dense part on the compact rows as ONE launch per direction (acsr_tail_fwd / _bwd); other inner sizes: six launches
+        self.tail_fused = self.tc and model.inner_size % 16 == 0
         # backward of a layer's dense part (two LayerNorm backwards, the activation backward, three input-gradient GEMMs) as ONE
-        # tcgen05 launch (acsr_dense_bwd: d_a1 / d_z1 stay in tensor memory); ACSR_DENSE_BWD=0: the six launches
-        self.dense_bwd = (self.tc and model.inner_size % 64 == 0 and os.environ.get('ACSR_DENSE_BWD', '1') == '1')
-        self.split_wgrad = int(os.environ.get('ACSR_SPLIT_WGRAD', '1'))       # 1: two weight-gradient launches for the first layer (see _backward_branch); 2: every layer
-        # CE backward without the [2B,V] gradient matrix (acsr_ce_bwd_dout / _dtable, hidden size 64); ACSR_CE_FUSED_BWD=0 keeps Gt
-        self.ce_fused_bwd = model.hidden_size == 64 and os.environ.get('ACSR_CE_FUSED_BWD', '1') == '1'
+        # tcgen05 launch (acsr_dense_bwd: d_a1 / d_z1 stay in tensor memory); other inner sizes: the six launches
+        self.dense_bwd = self.tc and model.inner_size % 64 == 0
+        # CE backward without the [2B,V] gradient matrix (acsr_ce_bwd_dout / _dtable); other widths go through Gt
+        self.ce_fused_bwd = model.hidden_size == 64
 
     # ------------------------------------------------------------------------------------------
     def _stream_for(self, dev, key):
@@ -105,19 +83,20 @@ class FusedTrainStep(object):
             return torch.empty(s, dtype=torch.float32, device=dev)
         b = dict(T=T, x0=f(T, d), st_e=f(T, 2), layers=[], order=torch.empty(Bs, dtype=torch.int32, device=dev))
         for l in range(N):
-            R = 2 * T if l == N - 1 else T
-            # mixed_q, mixed_k, mixed_v, attack_q, attack_k (+ the gate logits [T, L] in a sixth slot): one batched GEMM writes all
-            qkv5 = f(6, T, d)
-            qkv, aqk = qkv5[:3], qkv5[3:5]
-            Rp = 1 if (l == N - 1 and self.compact_last) else R      # the compact last layer keeps its dense part in b['c']
-            lb = dict(qkv5=qkv5, qkv=qkv, aqk=aqk, mq=qkv[0], mk=qkv[1], mv=qkv[2], aq=aqk[0], ak=aqk[1],
-                      gl=(qkv5[5].view(-1)[:T * L].view(T, L) if L <= d else f(T, L)), ctx=f(R, d),
-                      hz=f(Rp, d), st_a=f(Rp, 2), h=f(Rp, d), z1=f(Rp, I), a1=f(Rp, I), z2=f(Rp, d), st_f=f(Rp, 2), out=f(Rp, d))
+            last = l == N - 1
+            # mixed_q, mixed_k, mixed_v, attack_q, attack_k: one batched GEMM writes all
+            qkv5 = f(5, T, d)
+            qkv, aqk = qkv5[:3], qkv5[3:]
+            lb = dict(qkv5=qkv5, qkv=qkv, aqk=aqk, mq=qkv[0], mk=qkv[1], mv=qkv[2], aq=aqk[0], ak=aqk[1], gl=f(T, L),
+                      ctx=f(2 * T if last else T, d))
+            if not last:                       # the last layer's dense part runs on the compact rows of b['c']
+                lb.update(hz=f(T, d), st_a=f(T, 2), h=f(T, d), z1=f(T, I), a1=f(T, I), z2=f(T, d), st_f=f(T, 2), out=f(T, d))
             # buffers read by the weight-gradient kernels are per layer: the side stream may still be reading layer l's
             # while the branch stream already writes layer l-1's
             if grads:
-                for n, w in (('d_z2', d), ('d_z1', I), ('d_hz', d), ('d_gl', L)):
-                    lb[n] = f(2 * T if (Rp > 1 or n == 'd_gl') else 1, w)
+                lb['d_gl'] = f(2 * T, L)
+                if not last:
+                    lb['d_z2'], lb['d_z1'], lb['d_hz'] = f(2 * T, d), f(2 * T, I), f(2 * T, d)
                 lb['d_qkv'], lb['d_aqk'] = f(3, 2 * T, d), f(2, 2 * T, d)
                 lb['d_mq'], lb['d_mk'], lb['d_mv'] = lb['d_qkv'][0], lb['d_qkv'][1], lb['d_qkv'][2]
                 lb['d_aq'], lb['d_ak'] = lb['d_aqk'][0], lb['d_aqk'][1]
@@ -204,11 +183,8 @@ class FusedTrainStep(object):
                     bb = br['buf']
                     if self._sharded():
                         self._shard_buffers(bb, dev)['d_xrows'].zero_()
-                    if self.compact_last:
-                        bb['d_ctx'].zero_()
-                        bb['d_x'].zero_()
-                    else:
-                        bb['d_out'].zero_()
+                    bb['d_ctx'].zero_()
+                    bb['d_x'].zero_()
                     for l, layer in enumerate(m.trm_encoder.layer):
                         if layer.combine_option == 'gate':
                             bb['layers'][l]['d_gl'].zero_()
@@ -280,10 +256,8 @@ class FusedTrainStep(object):
                 jb['Gt'] = torch.empty((V, 2 * B), dtype=torch.float32, device=dev)
             LIB.call('acsr_logits_ce_grad', _p(jb['out2']), _p(E), _p(jb['lse']), _p(jb['target2'], torch.int64),
                      _p(jb['row_scale']), 2 * B, V, d, passes, _p(jb['Gt']), 2 * B, st)
-            if self.tc_wgrad:          # d_out2 [2B,d] += Gt^T . E : contraction over the catalogue, split over the CTAs
-                ops.gemm_batch([ops.wgrad_problem(jb['Gt'], E, V, 2 * B, d, jb['d_out2'])])
-            else:
-                LIB.call('acsr_linear_wgrad', _p(jb['Gt']), _p(E), V, 2 * B, d, _p(jb['d_out2']), None, st)
+            # d_out2 [2B,d] += Gt^T . E : contraction over the catalogue, split over the CTAs
+            ops.gemm_batch([ops.wgrad_problem(jb['Gt'], E, V, 2 * B, d, jb['d_out2'])])
         for br in branches:
             if br['stream'] is not main:
                 br['stream'].wait_stream(main)
@@ -297,9 +271,7 @@ class FusedTrainStep(object):
             with torch.cuda.stream(dE_stream):
                 if self.ce_fused_bwd:     # dE += G[:B]^T . out[:B], G recomputed (table rows on the UMMA M axis)
                     ops.ce_bwd_dtable(jb['out2'][:B], E, jb['lse'][:B], jb['target2'][:B], jb['row_scale'][:B], E.grad, passes)
-                elif self.tc and B <= 256:
-                    ops.linear_tok(jb['Gt'], V, B, jb['out2'], d, E.grad, d, ldx=2 * B, w_sn=1, w_sk=d, wkb=64 * d, accumulate=True)
-                else:                   # dE [V,d] += Gt[:, :B] . out[:B]  (rows of the table on the M axis, K = B)
+                else:                  # dE [V,d] += Gt[:, :B] . out[:B]  (rows of the table on the M axis, K = B)
                     ops.gemm_batch([ops.gemm_problem(jb['Gt'], jb['out2'], E.grad, V, d, B, a_strides=(2 * B, 1, 0, B),
                                                      b_strides=(1, d, 0, B), accumulate=True)])
         else:
@@ -342,47 +314,26 @@ class FusedTrainStep(object):
         # longest sequences first: order of the attention CTAs of this batch (forward and backward).  Only the attention
         # kernels read it, so the single-CTA sort runs next to the embedding and the first projections, not in front of them.
         cur = torch.cuda.current_stream()
-        so = self._stream_for(seq.device, ('order', s)) if self.order_side else cur
-        if so is not cur:
-            so.wait_stream(cur)
+        so = self._stream_for(seq.device, ('order', s))
+        so.wait_stream(cur)
         folded = {}
-        if self.tc and self.fold_attack:                  # first on the side stream: the first projection launch needs layer 0's
+        if self.tc:                                       # first on the side stream: the first projection launch needs layer 0's
             for l in range(N):
                 st3 = self._stacked(l)
                 if st3 is None:
                     continue
                 fw = self._folded_buffers(l, seq.device)
-                lay = m.trm_encoder.layer[l]
-                # combine_option 'gate': gate(mixed_q) = x.(Wg.Wq)^T + (Wg.bq + bg) rides along as a sixth, L-feature problem
-                fw['gate'] = lay.combine_option == 'gate' and lay.gate.out_features == L and L <= d and self.fold_gate
-                LIB.call('acsr_fold_projection_weights', _p(st3['Wqkv']), _p(st3['bqkv']), _p(st3['Waqk']), _p(st3['baqk']), d,
-                         _p(lay.gate.weight) if fw['gate'] else None, _p(lay.gate.bias) if fw['gate'] else None, L if fw['gate'] else 0,
+                LIB.call('acsr_fold_attack_weights', _p(st3['Wqkv']), _p(st3['bqkv']), _p(st3['Waqk']), _p(st3['baqk']), d,
                          _p(fw['W']), _p(fw['b']), so.cuda_stream)
                 fw['done'] = torch.cuda.Event()
                 fw['done'].record(so)
                 folded[l] = fw
-        dense_ops = {}
-        if self.dense_fused:
-            # the layers' dense weights as pre-split (hi, lo) TF32 operands, once per step next to the embedding kernel.  The last
-            # layer's dense part runs on the compact rows (acsr_tail_fwd) and needs none.
-            for l in range(N):
-                if l == N - 1 and self.compact_last and self.tail_fused:
-                    continue
-                lay = m.trm_encoder.layer[l]
-                dbuf = self._dense_ops_buffer(l, seq.device)
-                LIB.call('acsr_dense_prep', _p(lay.attack_attention.dense.weight), _p(lay.feed_forward.dense_1.weight),
-                         _p(lay.feed_forward.dense_2.weight), d, I, _p(dbuf['ops']), so.cuda_stream)
-                dbuf['done'] = torch.cuda.Event()
-                dbuf['done'].record(so)
-                dense_ops[l] = dbuf
-        b['dense_ops'] = dense_ops
         bwd_ops = {}
-        if self.dense_bwd and training and not self.fuse_act_bwd:
-            # the same weights transposed for acsr_dense_bwd.  Enqueued ahead of the sequence ordering, whose event the first
-            # attention launch waits for: complete before any backward kernel starts (and static for its PDL chain)
-            for l in range(N):
-                if l == N - 1 and self.compact_last and self.tail_fused:
-                    continue
+        if self.dense_bwd and training:
+            # the layers' dense weights transposed for acsr_dense_bwd (the last layer's dense part runs on the compact rows, see
+            # acsr_tail_bwd).  Enqueued ahead of the sequence ordering, whose event the first attention launch waits for: complete
+            # before any backward kernel starts (and static for its PDL chain)
+            for l in range(N - 1):
                 lay = m.trm_encoder.layer[l]
                 dbuf = self._dense_bwd_ops_buffer(l, s, seq.device)
                 LIB.call('acsr_dense_bwd_prep', _p(lay.attack_attention.dense.weight), _p(lay.feed_forward.dense_1.weight),
@@ -407,27 +358,16 @@ class FusedTrainStep(object):
         act_id = ops.ACT_IDS[m.hidden_act]
         for l, layer in enumerate(m.trm_encoder.layer):
             last = l == N - 1 and need_att                 # the attacked branch only matters on the last layer (and not in eval)
-            R = 2 * T if last else T
             lb = b['layers'][l]
             aa, ff = layer.attack_attention, layer.feed_forward
             base = soff + 16 * (l + 1)
             b['xs'].append(x)
-            st3 = self._stacked(l)
-            if l in folded and so is not cur:
-                cur.wait_event(folded[l]['done'])  # this layer's folded weights (side stream) are ready
-            if st3 is not None and self.tc and self.fold_attack:
+            fw = folded.get(l)
+            if fw is not None:
                 # all five projections read x: one batched tcgen05 launch over the folded weights (prepared at the start of the
                 # step on the ordering stream, next to the embedding kernel)
-                fw = folded[l]
-                if fw['gate']:
-                    ops.linear_tok(x, T, d, fw['W'], d, lb['qkv5'], d, bias=fw['b'], batch=6, sx=0, sw=d * d, sb=d, sy=T * d,
-                                   last_n=L, last_ldy=L)
-                else:
-                    ops.linear_tok(x, T, d, fw['W'], d, lb['qkv5'], d, bias=fw['b'], batch=5, sx=0, sw=d * d, sb=d, sy=T * d)
-            elif st3 is not None and self.tc:                 # stacked Q/K/V and attack pair: two batched tcgen05 launches
-                ops.linear_tok(x, T, d, st3['Wqkv'], d, lb['qkv'], d, bias=st3['bqkv'], batch=3, sx=0, sw=d * d, sb=d, sy=T * d)
-                ops.linear_tok(lb['qkv'], T, d, st3['Waqk'], d, lb['aqk'], d, bias=st3['baqk'], batch=2, sx=T * d, sw=d * d,
-                               sb=d, sy=T * d)
+                cur.wait_event(fw['done'])
+                ops.linear_tok(x, T, d, fw['W'], d, lb['qkv5'], d, bias=fw['b'], batch=5, sx=0, sw=d * d, sb=d, sy=T * d)
             else:
                 # any width: Q / K / V in one launch of the K-streamed tcgen05 kernel, then the attack pair (+ the gate logits,
                 # which read mixed_q as well) in a second one
@@ -446,7 +386,7 @@ class FusedTrainStep(object):
             if gate:
                 if layer.gate.out_features != L:
                     raise ValueError('gate width %d != sequence length %d' % (layer.gate.out_features, L))
-                if self.tc and not (l in folded and folded[l].get('gate')):
+                if self.tc:
                     ops.linear_tok(lb['mq'], T, d, layer.gate.weight, L, lb['gl'], L, bias=layer.gate.bias)
             elif layer.combine_option == 'annealing':
                 comb_scalar = math.exp(-layer.anneal_step / 100000)
@@ -455,13 +395,13 @@ class FusedTrainStep(object):
             p_attn = aa.attn_dropout.p if training else 0.0
             lb['attn_args'] = self._attn_args(layer, lb, seq, Bs, L, H, dh, comb_scalar, p_attn, rand, l, rngp, base)
             ctx_cal, ctx_att = lb['ctx'][:T], (lb['ctx'][T:] if last else None)
-            if l == 0 and so is not cur:
+            if l == 0:
                 cur.wait_event(order_done)         # sequence order (side stream) is ready
             LIB.call('acsr_attn_calib_fwd', *lb['attn_args'], _p(ctx_att), _p(ctx_cal),
                      jb['pen'][l:].data_ptr() if need_att else None, None, _p(b['order'], torch.int32),
-                     _p(ln, torch.int64) if (l == N - 1 and self.compact_last) else None, st)
+                     _p(ln, torch.int64) if l == N - 1 else None, st)
             m_a, m_f = mask2(l, 'D5', 'D4', last), mask2(l, 'D7', 'D6', last)
-            if l == N - 1 and self.compact_last:
+            if l == N - 1:
                 # ---- last layer: gather position len-1 of every sequence, then the dense part on the compact rows ----
                 cb = b['c']
                 C = 2 * Bs if need_att else Bs
@@ -492,38 +432,21 @@ class FusedTrainStep(object):
                         jb['out2'][B + lo:B + lo + Bs].copy_(cb['out'][Bs:C])
                 return
             lb['m_a'], lb['m_f'] = m_a, m_f
-            dops = dense_ops.get(l)
-            if dops is not None and so is not cur:
-                cur.wait_event(dops['done'])
-            self._post_attn_fwd(layer, lb, x, T, R, lb['out'], p_h, rngp, base, act_id, st, dops)
-            x = lb['out'][:T]
-        last_out = b['layers'][N - 1]['out']
-        # rows [0,B) of out2 calibrated, [B,2B) attacked; this branch owns the rows of its sequences in both halves
-        lo = br['sl'].start
-        LIB.call('acsr_gather_last_fwd', None, _p(last_out[:T]), _p(ln, torch.int64), Bs, L, d, _p(jb['out2'][lo:lo + Bs]), st)
-        if need_att:
-            LIB.call('acsr_gather_last_fwd', None, _p(last_out[T:]), _p(ln, torch.int64), Bs, L, d, _p(jb['out2'][B + lo:B + lo + Bs]), st)
+            self._post_attn_fwd(layer, lb, x, T, T, lb['out'], p_h, rngp, base, act_id, st)
+            x = lb['out']
 
-    def _post_attn_fwd(self, layer, bf, x_res, res_rows, R, out, p_h, rngp, base, act_id, st, dops=None):
+    def _post_attn_fwd(self, layer, bf, x_res, res_rows, R, out, p_h, rngp, base, act_id, st):
         """out-projection + dropout + residual + LayerNorm, then the feed-forward block, on R rows of bf['ctx']
         (layers.py:676-684, 790-798).  x_res [res_rows, d] is the layer input (residual)."""
         m = self.m
         d, I = m.hidden_size, m.inner_size
         aa, ff = layer.attack_attention, layer.feed_forward
-        if dops is not None:
-            LIB.call('acsr_dense_fwd', _p(bf['ctx']), _p(x_res), R, res_rows, d, I, act_id, _p(dops['ops']), _p(aa.dense.bias),
-                     _p(aa.LayerNorm.weight), _p(aa.LayerNorm.bias), aa.LayerNorm.eps, _p(ff.dense_1.bias), _p(ff.dense_2.bias),
-                     _p(ff.LayerNorm.weight), _p(ff.LayerNorm.bias), ff.LayerNorm.eps, p_h, _p(bf['m_a']), _p(bf['m_f']), rngp, base + 3,
-                     base + 5, _p(bf['hz']), _p(bf['st_a']), _p(bf['h']), _p(bf['z1']), _p(bf['a1']), _p(bf['z2']), _p(bf['st_f']), _p(out),
-                     self.passes, st)
-            return
         if self.tc:
             # out-projection + bias + dropout + residual + LayerNorm in one kernel; FFN: GEMM, bias + activation, then
             # GEMM + bias + dropout + residual + LayerNorm
             ops.linear_tok_bdrl(bf['ctx'], R, d, aa.dense.weight, aa.dense.bias, x_res, res_rows, aa.LayerNorm.weight,
                                 aa.LayerNorm.bias, aa.LayerNorm.eps, p_h, bf['m_a'], rngp, base + 3, bf['hz'], bf['h'], bf['st_a'])
-            # (the fused bias+activation epilogue, acsr_linear_tok_act, is slower than GEMM + the row-wise kernel at I=256:
-            # four epilogue warps per SM cannot hide the erf latency)
+            # (a bias + activation epilogue on the GEMM measured slower at I=256: four epilogue warps cannot hide the erf latency)
             ops.linear_tok(bf['h'], R, d, ff.dense_1.weight, I, bf['z1'], I)
             LIB.call('acsr_bias_act_fwd', _p(bf['z1']), _p(ff.dense_1.bias), R, I, act_id, _p(bf['a1']), st)
             ops.linear_tok_bdrl(bf['a1'], R, I, ff.dense_2.weight, ff.dense_2.bias, bf['h'], R, ff.LayerNorm.weight,
@@ -583,13 +506,8 @@ class FusedTrainStep(object):
         d_out, d_x = b['d_out'], b['d_x']
         lo = br['sl'].start
         T2 = 2 * T
-        compact = self.compact_last
-        if not compact:
-            LIB.call('acsr_gather_last_bwd', _p(jb['d_out2'][lo:lo + Bs]), _p(ln, torch.int64), Bs, L, d, None, _p(d_out[:T]), st)
-            LIB.call('acsr_gather_last_bwd', _p(jb['d_out2'][B + lo:B + lo + Bs]), _p(ln, torch.int64), Bs, L, d, None, _p(d_out[T:]), st)
         for l in reversed(range(N)):
             last = l == N - 1
-            P = T2 if last else T                               # period of the saved forward tensors
             lb = b['layers'][l]
             layer = m.trm_encoder.layer[l]
             aa, ff = layer.attack_attention, layer.feed_forward
@@ -597,7 +515,7 @@ class FusedTrainStep(object):
             x = b['xs'][l]
             gate = layer.combine_option == 'gate'
             wg = []                                          # weight-gradient problems of this layer (one launch at its end)
-            if last and compact:
+            if last:
                 # the dense part of the last layer on the 2*Bs rows that carry a cotangent, then scatter into the zeroed
                 # token-major buffers the attention backward (d_ctx) and the layer below (residual path, d_x) read
                 cb = b['c']
@@ -617,18 +535,17 @@ class FusedTrainStep(object):
                              _p(cb['d_z2']), _p(cb['d_z1']), _p(cb['d_hz']), _p(d_x[:T]), _p(d_x[T:]), _p(b['d_ctx'][:T]),
                              _p(b['d_ctx'][T:]), g(aa.dense.bias), g(aa.LayerNorm.weight), g(aa.LayerNorm.bias), g(ff.dense_1.bias),
                              g(ff.dense_2.bias), g(ff.LayerNorm.weight), g(ff.LayerNorm.bias), st)
-                    self._wgrad(cb['d_z2'], cb['a1'], Bs, ff.dense_2.weight.grad, None, fork, wg)
-                    self._wgrad(cb['d_z1'], cb['h'], Bs, ff.dense_1.weight.grad, None, fork, wg)
-                    self._wgrad(cb['d_hz'], cb['ctx'], Bs, aa.dense.weight.grad, None, fork, wg)
+                    self._wgrad(cb['d_z2'], cb['a1'], Bs, ff.dense_2.weight.grad, None, wg)
+                    self._wgrad(cb['d_z1'], cb['h'], Bs, ff.dense_1.weight.grad, None, wg)
+                    self._wgrad(cb['d_hz'], cb['ctx'], Bs, aa.dense.weight.grad, None, wg)
                 else:
-                    self._post_attn_bwd(layer, cb, cb, dc_out, cb['x'], C, C, Bs, Bs, cb['d_x'], cb['d_ctx'], p_h, rngp, base, act_id, st, fork, wg,
-                                        dops=b['dense_bwd_ops'].get(l))
+                    self._post_attn_bwd(layer, cb, cb, dc_out, cb['x'], C, C, Bs, Bs, cb['d_x'], cb['d_ctx'], p_h, rngp, base, act_id, st, wg)
                     LIB.call('acsr_gather_last_bwd', _p(cb['d_ctx']), _p(ln, torch.int64), Bs, L, d, _p(b['d_ctx'][:T]), _p(b['d_ctx'][T:]), st)
                     LIB.call('acsr_gather_last_bwd', _p(cb['d_x']), _p(ln, torch.int64), Bs, L, d, _p(d_x[:T]), _p(d_x[T:]), st)
             else:
-                self._post_attn_bwd(layer, lb, lb, d_out, x, T2, P, T, T, d_x, b['d_ctx'], p_h, rngp, base, act_id, st, fork, wg, b=b,
+                self._post_attn_bwd(layer, lb, lb, d_out, x, T2, T, T, T, d_x, b['d_ctx'], p_h, rngp, base, act_id, st, wg, b=b,
                                     dops=b['dense_bwd_ops'].get(l))
-            if wg and self.split_wgrad and (l == 0 or self.split_wgrad > 1):
+            if wg and l == 0:
                 # the out-projection / feed-forward weight gradients are complete here: their launch runs on the side stream
                 # under the attention backward, so the launch left for the end of the layer (the projections') is short --
                 # the first layer's is the tail of the step's critical path
@@ -647,16 +564,16 @@ class FusedTrainStep(object):
             LIB.call('acsr_attn_calib_bwd2', _p(dc[:T]), None, _p(d_att1), _p(d_cal1), _p(dpen[l:l + 1]), *lb['attn_args'],
                      _p(lb['d_mq']), _p(lb['d_mk']), _p(lb['d_mv']), _p(lb['d_aq']), _p(lb['d_ak']),
                      _p(lb['d_gl']) if gate else None, _p(g(ow)), _p(g(ob_)), _p(g(dw)), _p(g(db_)), _p(g(sc)), _p(g(rr)),
-                     _p(b['order'], torch.int32), _p(ln, torch.int64) if (last and compact) else None, st)
+                     _p(b['order'], torch.int32), _p(ln, torch.int64) if last else None, st)
             # projections: input gradients for both streams, weight gradients from the owning stream
             aqt, akt = aa.attack_query_transform, aa.attack_key_transform
             # weight gradients of the projections: attack transforms are trained by the attacked-loss stream (rows [T,2T)), the
             # gate by both halves of d_gl's stream-0 rows, Q / K / V by the calibrated-loss stream.  (A third launch for the attack pair
             # + gate, whose operands are final right after the attention backward, measured no further gain: 0.7162 vs 0.7179 ms.)
-            self._wgrad(lb['d_aq'][T:], lb['mq'], T, aqt.weight.grad, aqt.bias.grad, fork, wg)
-            self._wgrad(lb['d_ak'][T:], lb['mk'], T, akt.weight.grad, akt.bias.grad, fork, wg)
+            self._wgrad(lb['d_aq'][T:], lb['mq'], T, aqt.weight.grad, aqt.bias.grad, wg)
+            self._wgrad(lb['d_ak'][T:], lb['mk'], T, akt.weight.grad, akt.bias.grad, wg)
             if gate:
-                self._wgrad(lb['d_gl'], lb['mq'], T, layer.gate.weight.grad, layer.gate.bias.grad, fork, wg)
+                self._wgrad(lb['d_gl'], lb['mq'], T, layer.gate.weight.grad, layer.gate.bias.grad, wg)
 
             st3 = self._stacked(l)
             gp = ops.gemm_problem
@@ -685,7 +602,7 @@ class FusedTrainStep(object):
                         ops.gemm_batch([gp(lb[dk], lin.weight, d_x, rows_x, d, d, b_strides=(1, d, 0, d), accumulate=True)],
                                        passes=self.passes)
             for lin, dk in ((aa.query, 'd_mq'), (aa.key, 'd_mk'), (aa.value, 'd_mv')):
-                self._wgrad(lb[dk], x, T, lin.weight.grad, lin.bias.grad, fork, wg)
+                self._wgrad(lb[dk], x, T, lin.weight.grad, lin.bias.grad, wg)
             if wg:                                           # all weight gradients of the layer: ONE launch on the side stream
                 ops.gemm_batch(wg, passes=self.passes, stream=fork())
             if l > 0:
@@ -705,7 +622,7 @@ class FusedTrainStep(object):
         if side is not None:
             main.wait_stream(side)                            # join: every weight gradient of this branch landed
 
-    def _post_attn_bwd(self, layer, bf, gb, d_out, x_res, R2, P, res_rows, w_rows, d_xres, d_ctx, p_h, rngp, base, act_id, st, fork, wg, b=None,
+    def _post_attn_bwd(self, layer, bf, gb, d_out, x_res, R2, P, res_rows, w_rows, d_xres, d_ctx, p_h, rngp, base, act_id, st, wg, b=None,
                        dops=None):
         """backward of _post_attn_fwd over R2 cotangent rows ([stream 0 ; stream 1]); the saved forward tensors of bf repeat
         with period P, the residual x_res with period res_rows; rows [0, w_rows) (stream 0) feed the parameter gradients.
@@ -724,9 +641,9 @@ class FusedTrainStep(object):
                      base + 3, base + 5, _p(gb['d_z2']), _p(gb['d_z1']), _p(gb['d_hz']), _p(d_xres), _p(d_ctx),
                      _p(ff.LayerNorm.weight.grad), _p(ff.LayerNorm.bias.grad), _p(aa.LayerNorm.weight.grad),
                      _p(aa.LayerNorm.bias.grad), self.passes, st)
-            self._wgrad(gb['d_z2'], bf['a1'], w_rows, ff.dense_2.weight.grad, ff.dense_2.bias.grad, fork, wg)
-            self._wgrad(gb['d_z1'], bf['h'], w_rows, ff.dense_1.weight.grad, ff.dense_1.bias.grad, fork, wg)
-            self._wgrad(gb['d_hz'], bf['ctx'], w_rows, aa.dense.weight.grad, aa.dense.bias.grad, fork, wg)
+            self._wgrad(gb['d_z2'], bf['a1'], w_rows, ff.dense_2.weight.grad, ff.dense_2.bias.grad, wg)
+            self._wgrad(gb['d_z1'], bf['h'], w_rows, ff.dense_1.weight.grad, ff.dense_1.bias.grad, wg)
+            self._wgrad(gb['d_hz'], bf['ctx'], w_rows, aa.dense.weight.grad, aa.dense.bias.grad, wg)
             return
         d_h = gb['d_h'] if b is None else b['d_h']
         d_a1 = gb['d_a1'] if b is None else b['d_a1']
@@ -736,21 +653,14 @@ class FusedTrainStep(object):
                  _p(ff.LayerNorm.weight), _p(bf['st_f']), R2, d, P, P, w_rows, p_h, _p(bf['m_f']), rngp, base + 5,
                  _p(gb['d_z2']), _p(d_h), _p(ff.dense_2.bias.grad), _p(ff.LayerNorm.weight.grad),
                  _p(ff.LayerNorm.bias.grad), st)
-        self._wgrad(gb['d_z2'], bf['a1'], w_rows, ff.dense_2.weight.grad, None, fork, wg)
-        if self.tc and self.tc_wgrad and self.fuse_act_bwd:
-            # d_z1 = (d_z2.W2) * act'(z1 + b1) in ONE launch (the activation backward in the GEMM's TMEM epilogue); the bias gradient
-            # comes out of the weight-gradient launch (row sums of its left operand)
-            ops.linear_tok_actbwd(gb['d_z2'], R2, d, ff.dense_2.weight, I, bf['z1'], P, ff.dense_1.bias, act_id, gb['d_z1'],
-                                  w_sn=1, w_sk=I, wkb=64 * I)
-            self._wgrad(gb['d_z1'], bf['h'], w_rows, ff.dense_1.weight.grad, ff.dense_1.bias.grad, fork, wg)
+        self._wgrad(gb['d_z2'], bf['a1'], w_rows, ff.dense_2.weight.grad, None, wg)
+        if self.tc:                                          # d_a1 = d_z2.W2 : the weight is read transposed
+            ops.linear_tok(gb['d_z2'], R2, d, ff.dense_2.weight, I, d_a1, I, w_sn=1, w_sk=I, wkb=64 * I)
         else:
-            if self.tc:                                      # d_a1 = d_z2.W2 : the weight is read transposed
-                ops.linear_tok(gb['d_z2'], R2, d, ff.dense_2.weight, I, d_a1, I, w_sn=1, w_sk=I, wkb=64 * I)
-            else:
-                ops.gemm_batch([gp(gb['d_z2'], ff.dense_2.weight, d_a1, R2, I, d, b_strides=(1, I, 0, d))], passes=ps)
-            LIB.call('acsr_bias_act_bwd', _p(d_a1), _p(bf['z1']), _p(ff.dense_1.bias), R2, I, act_id, P, w_rows, _p(gb['d_z1']),
-                     _p(ff.dense_1.bias.grad), st)
-            self._wgrad(gb['d_z1'], bf['h'], w_rows, ff.dense_1.weight.grad, None, fork, wg)
+            ops.gemm_batch([gp(gb['d_z2'], ff.dense_2.weight, d_a1, R2, I, d, b_strides=(1, I, 0, d))], passes=ps)
+        LIB.call('acsr_bias_act_bwd', _p(d_a1), _p(bf['z1']), _p(ff.dense_1.bias), R2, I, act_id, P, w_rows, _p(gb['d_z1']),
+                 _p(ff.dense_1.bias.grad), st)
+        self._wgrad(gb['d_z1'], bf['h'], w_rows, ff.dense_1.weight.grad, None, wg)
         if self.tc:
             ops.linear_tok(gb['d_z1'], R2, I, ff.dense_1.weight, d, d_h, d, w_sn=1, w_sk=d, wkb=64 * d, accumulate=True)
         else:
@@ -759,21 +669,17 @@ class FusedTrainStep(object):
         LIB.call('acsr_bias_dropout_res_ln_bwd', _p(d_h), _p(bf['hz']), _p(aa.dense.bias), _p(x_res),
                  _p(aa.LayerNorm.weight), _p(bf['st_a']), R2, d, P, res_rows, w_rows, p_h, _p(bf['m_a']), rngp, base + 3,
                  _p(gb['d_hz']), _p(d_xres), _p(aa.dense.bias.grad), _p(aa.LayerNorm.weight.grad), _p(aa.LayerNorm.bias.grad), st)
-        self._wgrad(gb['d_hz'], bf['ctx'], w_rows, aa.dense.weight.grad, None, fork, wg)
+        self._wgrad(gb['d_hz'], bf['ctx'], w_rows, aa.dense.weight.grad, None, wg)
         if self.tc:
             ops.linear_tok(gb['d_hz'], R2, d, aa.dense.weight, d, d_ctx, d, w_sn=1, w_sk=d, wkb=64 * d)
         else:
             ops.gemm_batch([gp(gb['d_hz'], aa.dense.weight, d_ctx, R2, d, d, b_strides=(1, d, 0, d))], passes=ps)
 
-    def _wgrad(self, dY, X, rows, dW, db, fork, wg):
+    @staticmethod
+    def _wgrad(dY, X, rows, dW, db, wg):
         """weight-gradient reduction dW [N,K] += dY[:rows]^T . X[:rows] (+ db += column sums): a problem of the layer's single
-        tcgen05 launch (gemm_ks.cu, token axis on K, split over the CTAs), or -- tc_wgrad off -- one launch of the fp32
-        token-split kernel on the side stream."""
-        N, K = dY.shape[-1], X.shape[-1]
-        if self.tc_wgrad:
-            wg.append(ops.wgrad_problem(dY, X, rows, N, K, dW, db))
-        else:
-            LIB.call('acsr_linear_wgrad', _p(dY), _p(X), rows, N, K, _p(dW), _p(db), fork())
+        tcgen05 launch (gemm_ks.cu, token axis on K, split over the CTAs)."""
+        wg.append(ops.wgrad_problem(dY, X, rows, dY.shape[-1], X.shape[-1], dW, db))
 
     def _sharded(self):
         return self.vp is not None and self.vp.sharded
@@ -791,21 +697,11 @@ class FusedTrainStep(object):
         key = ('folded', l)
         if key not in self.buf:
             d = self.m.hidden_size
-            self.buf[key] = dict(W=torch.zeros((6, d, d), dtype=torch.float32, device=dev), b=torch.zeros((6, 1, d), dtype=torch.float32, device=dev))
+            self.buf[key] = dict(W=torch.zeros((5, d, d), dtype=torch.float32, device=dev), b=torch.zeros((5, 1, d), dtype=torch.float32, device=dev))
             # written once per step by acsr_fold_attack_weights, which completes (full event dependency) before the first kernel
             # of the chain that reads them starts: safe to read ahead of programmatic-launch synchronisation
             for t in list(self.buf[key].values()):
                 LIB.query('acsr_register_static', t.data_ptr(), t.numel() * 4)
-        return self.buf[key]
-
-    def _dense_ops_buffer(self, l, dev):
-        key = ('dense_ops', l)
-        if key not in self.buf:
-            n = LIB.query('acsr_dense_prep_floats', int(self.m.inner_size))
-            t = torch.empty(n, dtype=torch.float32, device=dev)
-            # written once per step by acsr_dense_prep, complete (event dependency) before its reader starts: static for the PDL chain
-            LIB.query('acsr_register_static', t.data_ptr(), t.numel() * 4)
-            self.buf[key] = dict(ops=t)
         return self.buf[key]
 
     def _dense_bwd_ops_buffer(self, l, s, dev):

@@ -529,29 +529,11 @@ def linear_tc(X, rows, W, N, w_sn, w_sk, bias, Y, ldy, accumulate=False, batch=1
 
 
 def linear_tok(X, rows, K, W, N, Y, ldy, ldx=None, xkb=64, w_sn=None, w_sk=1, wkb=64, bias=None, accumulate=False,
-               batch=1, sx=0, sw=0, sb=0, sy=0, passes=3, last_n=0, last_ldy=0):
-    """Y[rows,N] (+)= X.W^T + bias on tcgen05 with token rows on the M axis (acsr_linear_tok); strides in floats.
-    last_n > 0: the last problem of a batched launch has last_n features written with row stride last_ldy."""
-    if not last_n:
-        LIB.call('acsr_linear_tok', _p(X), int(K if ldx is None else ldx), int(xkb), int(rows), int(K), _p(W),
-                 int(K if w_sn is None else w_sn), int(w_sk), int(wkb), int(N), _p(bias), int(bool(accumulate)), _p(Y), int(ldy),
-                 int(batch), int(sx), int(sw), int(sb), int(sy), passes, _stream())
-        return
-    LIB.call('acsr_linear_tok_ragged', _p(X), int(K if ldx is None else ldx), int(xkb), int(rows), int(K), _p(W),
+               batch=1, sx=0, sw=0, sb=0, sy=0, passes=3):
+    """Y[rows,N] (+)= X.W^T + bias on tcgen05 with token rows on the M axis (acsr_linear_tok); strides in floats."""
+    LIB.call('acsr_linear_tok', _p(X), int(K if ldx is None else ldx), int(xkb), int(rows), int(K), _p(W),
              int(K if w_sn is None else w_sn), int(w_sk), int(wkb), int(N), _p(bias), int(bool(accumulate)), _p(Y), int(ldy),
-             int(batch), int(sx), int(sw), int(sb), int(sy), int(last_n), int(last_ldy), passes, _stream())
-
-
-def linear_tok_actbwd(X, rows, K, W, N, Z, z_rows, bias, act, Y, w_sn, w_sk, wkb, passes=3):
-    """Y = (X.W^T) * act'(Z + bias): input gradient through dense_2 and the activation in one launch (acsr_linear_tok_actbwd)."""
-    LIB.call('acsr_linear_tok_actbwd', _p(X), int(K), int(rows), int(K), _p(W), int(w_sn), int(w_sk), int(wkb), int(N), _p(Z),
-             int(z_rows), _p(bias), int(act), _p(Y), passes, _stream())
-
-
-def linear_tok_act(X, rows, K, W, N, bias, act, Z, A, passes=3):
-    """Z = X.W^T, A = act(Z + bias)  (acsr_linear_tok_act)."""
-    LIB.call('acsr_linear_tok_act', _p(X), int(K), int(rows), int(K), _p(W), int(N), _p(bias), int(act), _p(Z), _p(A), int(N),
-             passes, _stream())
+             int(batch), int(sx), int(sw), int(sb), int(sy), passes, _stream())
 
 
 def linear_tok_bdrl(X, rows, K, W, bias, res, res_rows, ln_w, ln_b, eps, p, mask, rngp, rng_stream, HZ, out, stats, passes=3):

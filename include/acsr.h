@@ -305,10 +305,6 @@ int acsr_topk_select_rank(const float* scores, int M, int64_t V, int64_t ld, int
  * {bq, bk, bv, Waq.bq + baq, Wak.bk + bak}.  Wqkv [3,d,d], bqkv [3,d], Waqk [2,d,d], baqk [2,d] (row-major [out,in]). */
 int acsr_fold_attack_weights(const float* Wqkv, const float* bqkv, const float* Waqk, const float* baqk, int d, float* out_W,
                              float* out_b, void* stream);
-/* the same with the gate of combine_option 'gate' (layers.py:887, gate(mixed_q)) folded in as a sixth slot: out_W [6,d,d] /
- * out_b [6,d], slot 5 rows [0,Lg) = Wg.Wq and Wg.bq + bg (Wg [Lg,d], Lg <= d); Lg = 0: five slots as above. */
-int acsr_fold_projection_weights(const float* Wqkv, const float* bqkv, const float* Waqk, const float* baqk, int d,
-                                 const float* Wg, const float* bg, int Lg, float* out_W, float* out_b, void* stream);
 
 /* ---- encoder GEMMs on tcgen05 with the token rows on the UMMA M axis (3xTF32, fp32-level accuracy) ----
  * replaces the nn.Linear forward / input-gradient GEMMs of model/layers.py:658-659, 680, 687-689, 791-794, 887.
@@ -322,22 +318,6 @@ int acsr_linear_tok(const float* X, int64_t ldx, int64_t x_kblock_stride, int64_
                     const float* bias, int accumulate, float* Y, int64_t ldy,
                     int batch, int64_t stride_x, int64_t stride_w, int64_t stride_bias, int64_t stride_y,
                     int passes, void* stream);
-/* batched launch whose LAST problem is narrower: last_n <= N features written with row stride last_ldy (the gate logits
- * [T, L] riding along with the five [T, d] projections of a layer); last_n = 0: acsr_linear_tok. */
-int acsr_linear_tok_ragged(const float* X, int64_t ldx, int64_t x_kblock_stride, int64_t rows, int K, const float* W, int64_t w_stride_n,
-                           int64_t w_stride_k, int64_t w_kblock_stride, int N, const float* bias, int accumulate, float* Y, int64_t ldy,
-                           int batch, int64_t stride_x, int64_t stride_w, int64_t stride_bias, int64_t stride_y, int last_n,
-                           int64_t last_ldy, int passes, void* stream);
-/* input gradient through a linear layer AND the activation in front of it in one launch (layers.py:776-792 backward):
- * Y[r, n] = (sum_k X(r,k) * W(n,k)) * act'(Z[(r % z_rows), n] + bias[n]), Z [z_rows, N] = the saved pre-activation GEMM output,
- * Y [rows, N] contiguous.  X / W strides as acsr_linear_tok (the weight is usually read transposed). */
-int acsr_linear_tok_actbwd(const float* X, int64_t ldx, int64_t rows, int K, const float* W, int64_t w_stride_n, int64_t w_stride_k,
-                           int64_t w_kblock_stride, int N, const float* Z, int64_t z_rows, const float* bias, int act, float* Y,
-                           int passes, void* stream);
-/* FFN first half fused (model/layers.py:776-792): Z = X.W^T (saved pre-bias for the backward), A = act(Z + bias).
- * X [rows,K] (row stride ldx), W [N,K] row-major, Z,A [rows,N] (row stride ldy). */
-int acsr_linear_tok_act(const float* X, int64_t ldx, int64_t rows, int K, const float* W, int N, const float* bias, int act,
-                        float* Z, float* A, int64_t ldy, int passes, void* stream);
 /* projection + bias + dropout + residual + LayerNorm fused (model/layers.py:680-683, 793-796), output width 64:
  * HZ = X.W^T (saved for the backward), out = LN(dropout(HZ + bias) + res[r % res_rows]), stats[r] = (mean, rstd).
  * Dropout masks use the same Philox counters as acsr_bias_dropout_res_ln_{fwd,bwd}, which stays the backward. */
@@ -445,23 +425,9 @@ int acsr_tail_bwd(const float* d_out, const int64_t* item_len, int B, int L, int
                   float* d_ctx_first, float* d_ctx_second, float* g_bo, float* g_lnA_w, float* g_lnA_b, float* g_b1, float* g_b2,
                   float* g_lnF_w, float* g_lnF_b, void* stream);
 
-/* ---- an encoder layer's dense part after its attention, forward, as ONE tcgen05 kernel (hidden size 64, inner size a multiple of
- * 64 up to 256): hz = ctx.Wo^T ; h = LN(drop(hz + bo) + res) ; z1 = h.W1^T ; a1 = act(z1 + b1) ; z2 = a1.W2^T ;
- * out = LN(drop(z2 + b2) + h)  (layers.py:676-684, 790-798).  The activations stay in tensor memory between the GEMMs (each
- * epilogue's output is the next MMA's A operand).  `ops` = the layer's weights pre-split by acsr_dense_prep (once per step) into
- * (hi, lo) TF32 operands: acsr_dense_prep_floats(I) floats.  res [res_rows, 64] is the layer input (row r uses res[r % res_rows]).
- * Outputs (all saved for the backward, same meaning as the unfused path): hz, h, z2, out [rows,64]; z1, a1 [rows,I];
- * st_a, st_f [rows,2] = (mean, rstd).  Dropout: masks [rows,64] or Philox streams as acsr_bias_dropout_res_ln_fwd. */
-int64_t acsr_dense_prep_floats(int I);
-int acsr_dense_prep(const float* Wo, const float* W1, const float* W2, int d, int I, float* ops, void* stream);
-int acsr_dense_fwd(const float* ctx, const float* res, int64_t rows, int64_t res_rows, int d, int I, int act, const float* ops,
-                   const float* bo, const float* lnA_w, const float* lnA_b, float epsA, const float* b1, const float* b2,
-                   const float* lnF_w, const float* lnF_b, float epsF, float p_drop, const float* mask_a, const float* mask_f,
-                   const void* rng, uint32_t stream_a, uint32_t stream_f, float* hz, float* st_a, float* h, float* z1, float* a1,
-                   float* z2, float* st_f, float* out, int passes, void* stream);
-
-/* ---- backward of that dense part as ONE tcgen05 kernel (hidden size 64, inner size a multiple of 64 up to 256), the chain of two
- * acsr_bias_dropout_res_ln_bwd calls, acsr_bias_act_bwd and three input-gradient GEMMs:
+/* ---- backward of an encoder layer's dense part after its attention (layers.py:676-684, 790-798) as ONE tcgen05 kernel (hidden
+ * size 64, inner size a multiple of 64 up to 256), the chain of two acsr_bias_dropout_res_ln_bwd calls, acsr_bias_act_bwd and
+ * three input-gradient GEMMs:
  *   d_pre_f = LN_f backward of d_out ; d_z2 = d_pre_f * mask_f ; d_z1 = (d_z2.W2) * act'(z1 + b1) ; d_h = d_pre_f + d_z1.W1 ;
  *   d_xres = LN_a backward of d_h ; d_hz = d_xres * mask_a ; d_ctx = d_hz.Wo
  * with the argument meaning of those calls: `rows` cotangent rows; the saved tensors z2, h, st_f, z1 [., I], hz, st_a (and the

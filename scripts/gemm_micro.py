@@ -37,7 +37,6 @@ for rows in (T, 2 * T):
     W1 = torch.randn(I, d, device=dev) * .1
     W2 = torch.randn(d, I, device=dev) * .1
     b = torch.randn(d, device=dev)
-    b1 = torch.randn(I, device=dev)
     y = torch.empty(rows, d, device=dev)
     z1, a1 = torch.empty(rows, I, device=dev), torch.empty(rows, I, device=dev)
     a1.normal_()
@@ -50,9 +49,6 @@ for rows in (T, 2 * T):
     print('  64->64 acc tok %.1f | addmm_ %.1f' % (bench(lambda: ops.linear_tok(x, rows, d, W, d, y, d, w_sn=1, w_sk=d, wkb=64 * d, accumulate=True)), bench(lambda: y.addmm_(x, W))))
     print('  64->256   tok %.1f  | mm %.1f' % (bench(lambda: ops.linear_tok(x, rows, d, W1, I, z1, I)), bench(lambda: torch.mm(x, W1.t(), out=z1))))
     print('  256->64   tok %.1f  | mm %.1f' % (bench(lambda: ops.linear_tok(a1, rows, I, W2, d, y, d)), bench(lambda: torch.mm(a1, W2.t(), out=y))))
-    print('  64->256 +act fused %.1f | tok + bias_act %.1f' % (
-        bench(lambda: ops.linear_tok_act(x, rows, d, W1, I, b1, 0, z1, a1)),
-        bench(lambda: (ops.linear_tok(x, rows, d, W1, I, z1, I), A.LIB.call('acsr_bias_act_fwd', z1.data_ptr(), b1.data_ptr(), rows, I, 0, a1.data_ptr(), ops._stream())))))
     print('  64->64 +bdrl fused %.1f | tok + bdrl %.1f' % (
         bench(lambda: ops.linear_tok_bdrl(x, rows, d, W, b, res, T, lw, lb, 1e-12, 0.5, None, rng.ptr, 3, y, out, stats)),
         bench(lambda: (ops.linear_tok(x, rows, d, W, d, y, d), A.LIB.call('acsr_bias_dropout_res_ln_fwd', y.data_ptr(), b.data_ptr(), res.data_ptr(), lw.data_ptr(), lb.data_ptr(), 1e-12, rows, d, T, 0.5, None, rng.ptr, 3, out.data_ptr(), stats.data_ptr(), ops._stream())))))

@@ -132,7 +132,7 @@ def run(A, t, o, rows, act_rows, res_rows, param_rows, I, act, passes):
 
 
 def six_launches(A, t, o, rows, act_rows, res_rows, param_rows, I, act):
-    """the chain as the fused step ran it before acsr_dense_bwd (and still does with ACSR_DENSE_BWD=0)"""
+    """the six-launch chain the fused step runs where acsr_dense_bwd does not apply (inner sizes not a multiple of 64)"""
     p, st = A.ops._p, A.ops._stream()
     o = {k: v.clone() for k, v in o.items()}
     rngp = t['rng'].ptr if t['rng'] is not None else None

@@ -192,47 +192,6 @@ def test_tail_fused_last_layer(A, B, L, I, groups, act, p):
     close(G['d_hz'][:B].double().t() @ S['ctx'][:B].double(), P[0].grad, 1e-4, 'dWo')
 
 
-@pytest.mark.parametrize('rows,res_rows,I,act,p', [(300, 300, 256, 'gelu', 0.3), (12800, 12800, 256, 'gelu', 0.5), (128, 64, 64, 'relu', 0.0),
-                                                   (1000, 1000, 128, 'swish', 0.2), (40000, 20000, 256, 'gelu', 0.1)])
-def test_dense_fwd_fused_layer(A, rows, res_rows, I, act, p):
-    """acsr_dense_prep + acsr_dense_fwd (out-projection + LayerNorm + feed-forward + LayerNorm of a 128-token tile in one tcgen05
-    kernel, activations kept in tensor memory between the GEMMs) against fp64 (layers.py:676-684, 790-798), injected masks."""
-    from ac_tsr_b200._lib import LIB
-    _p = A.ops._p
-    g = torch.Generator().manual_seed(rows + I)
-    d = 64
-    r = lambda *s: torch.randn(*s, generator=g)       # noqa: E731
-    ctx, res = r(rows, d), r(res_rows, d)
-    Wo, bo, W1, b1, W2, b2 = r(d, d) * 0.2, r(d) * 0.1, r(I, d) * 0.2, r(I) * 0.1, r(d, I) * 0.1, r(d) * 0.1
-    lnAw, lnAb, lnFw, lnFb = 1 + 0.1 * r(d), 0.1 * r(d), 1 + 0.1 * r(d), 0.1 * r(d)
-    m_a, m_f = drop((rows, d), p, g), drop((rows, d), p, g)
-    D = lambda t: t.double()                          # noqa: E731
-    idx = torch.arange(rows) % res_rows
-    hz = D(ctx) @ D(Wo).t()
-    h = torch.nn.functional.layer_norm((hz + D(bo)) * D(m_a) + D(res)[idx], (d,), D(lnAw), D(lnAb), 1e-12)
-    z1 = h @ D(W1).t()
-    a1 = O.act_fn(act)(z1 + D(b1))
-    z2 = a1 @ D(W2).t()
-    out = torch.nn.functional.layer_norm((z2 + D(b2)) * D(m_f) + h, (d,), D(lnFw), D(lnFb), 1e-12)
-    dev = 'cuda'
-    f = lambda *s: torch.empty(*s, device=dev)        # noqa: E731
-    ops_buf = f(LIB.query('acsr_dense_prep_floats', I))
-    st = torch.cuda.current_stream().cuda_stream
-    Wg = [t.to(dev) for t in (Wo, W1, W2, bo, lnAw, lnAb, b1, b2, lnFw, lnFb)]
-    LIB.call('acsr_dense_prep', _p(Wg[0]), _p(Wg[1]), _p(Wg[2]), d, I, _p(ops_buf), st)
-    S = dict(hz=f(rows, d), st_a=f(rows, 2), h=f(rows, d), z1=f(rows, I), a1=f(rows, I), z2=f(rows, d), st_f=f(rows, 2), out=f(rows, d))
-    ctx_g, res_g, ma_g, mf_g = ctx.to(dev), res.to(dev), m_a.to(dev), m_f.to(dev)       # (kept alive: the ABI takes raw pointers)
-    for passes, tol in ((3, 2e-5), (1, 5e-3)):
-        LIB.call('acsr_dense_fwd', _p(ctx_g), _p(res_g), rows, res_rows, d, I, A.ops.ACT_IDS[act], _p(ops_buf), _p(Wg[3]),
-                 _p(Wg[4]), _p(Wg[5]), 1e-12, _p(Wg[6]), _p(Wg[7]), _p(Wg[8]), _p(Wg[9]), 1e-12, p, _p(ma_g), _p(mf_g),
-                 None, 0, 0, _p(S['hz']), _p(S['st_a']), _p(S['h']), _p(S['z1']), _p(S['a1']), _p(S['z2']), _p(S['st_f']), _p(S['out']),
-                 passes, st)
-        for k, ref in (('hz', hz), ('h', h), ('z1', z1), ('a1', a1), ('z2', z2), ('out', out)):
-            close(S[k], ref, tol, '%s (passes=%d)' % (k, passes))
-        if passes == 3:
-            close(S['st_f'][:, 0], ((z2 + D(b2)) * D(m_f) + h).mean(1), 2e-5, 'LayerNorm mean')
-
-
 def test_gather_last(A):
     g = torch.Generator().manual_seed(1)
     B, L, d = 9, 50, 64
@@ -853,20 +812,6 @@ def test_linear_tok_transposed_kconcat_batched(A):
     dmq = dmq0.clone()
     A.ops.linear_tok(dgl, T2, L, Wg, d, dmq, d, ldx=L, w_sn=1, w_sk=d, wkb=64 * d, accumulate=True)
     close(dmq, dmq0.double() + dgl.double() @ Wg.double(), 3e-6, 'K=50')
-
-
-@pytest.mark.parametrize('act', ['gelu', 'relu', 'swish', 'tanh', 'sigmoid'])
-def test_linear_tok_act(A, act):
-    g = torch.Generator().manual_seed(9)
-    R, d, I = 1500, 64, 256
-    X = torch.randn(R, d, generator=g).cuda()
-    W = torch.randn(I, d, generator=g).cuda() * 0.2
-    b = torch.randn(I, generator=g).cuda()
-    Z, A1 = torch.empty(R, I).cuda(), torch.empty(R, I).cuda()
-    A.ops.linear_tok_act(X, R, d, W, I, b, A.ops.ACT_IDS[act], Z, A1)
-    zr = X.double() @ W.double().t()
-    close(Z, zr, 3e-6, 'Z')
-    close(A1, O.act_fn(act)((zr + b.double()).float().cpu()), 1e-5, 'act')
 
 
 @pytest.mark.parametrize('K,p,explicit', [(64, 0.0, False), (64, 0.5, True), (256, 0.5, True), (64, 0.5, False), (128, 0.3, True)])
