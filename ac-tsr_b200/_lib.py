@@ -194,12 +194,46 @@ def _ab_candidate_rank_counts(a):
     return _ab_candidate_rank(a) + 12 * a[5]
 
 
+def _ab_candidate_scores_shard(a):
+    # (out, shard, lo, hi, V, d, cand, M, n_cand, scores, stream): out rows and candidate ids in, the owned candidates' rows
+    # gathered (counted as all of them: the owned share is data-dependent), scores out
+    d, M, C = a[5], a[7], a[8]
+    return 4 * M * d + M * C * (8 + 4 * d) + 4 * M * C
+
+
+def _ab_candidate_rank_scores(a):
+    # (scores, cand, V, M, n_cand, kmax, rec, counts, stream): scores and ids in, hit flags (and counts) out
+    M, C, kmax = a[3], a[4], a[5]
+    return 12 * M * C + 4 * M * (kmax + 1) + (12 * M if a[7] else 0)
+
+
+def _ab_bpr_dots_shard(a):
+    # (out, shard, lo, hi, V, pos, neg, M, d, dots, stream): out rows, two ids and two table rows per row in, two dots out
+    M, d = a[7], a[8]
+    return 4 * M * 3 * d + 16 * M + 8 * M
+
+
+def _ab_bpr_loss_from_dots(a):
+    # (dots, M, n_groups, gamma, row_x, row_loss, loss, stream): dots in, row_x / row_loss out, row_loss read back for the means
+    M = a[1]
+    return 8 * M + 8 * M + 4 * M
+
+
+def _ab_bpr_loss_bwd_shard(a):
+    # (out, shard, lo, hi, V, pos, neg, row_x, row_scale, M, d, gamma, begin, end, d_out, d_shard, stream): per row two ids, x,
+    # scale and two table rows in, d_out out; the training rows also read out and add into two gradient rows
+    M, d, n_tab = a[9], a[10], max(0, a[13] - a[12])
+    return M * (24 + 4 * 2 * d + (4 * d if a[14] else 0)) + n_tab * 4 * (d + 4 * d)
+
+
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
 ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl,
               'acsr_proj_input_grad': _ab_proj_input_grad, 'acsr_dense_bwd': _ab_dense_bwd,
               'acsr_linear_wgrad': _ab_linear_wgrad, 'acsr_linear_wgrad_batched': _ab_linear_wgrad_batched,
               'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank,
-              'acsr_candidate_rank_counts': _ab_candidate_rank_counts}
+              'acsr_candidate_rank_counts': _ab_candidate_rank_counts, 'acsr_candidate_scores_shard': _ab_candidate_scores_shard,
+              'acsr_candidate_rank_scores': _ab_candidate_rank_scores, 'acsr_bpr_dots_shard': _ab_bpr_dots_shard,
+              'acsr_bpr_loss_from_dots': _ab_bpr_loss_from_dots, 'acsr_bpr_loss_bwd_shard': _ab_bpr_loss_bwd_shard}
 
 
 class KernelTimer:

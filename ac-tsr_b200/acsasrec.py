@@ -227,16 +227,19 @@ class ACSASRec(SequentialRecommender):
         """Sampled-candidate ranking (`eval_args.mode: uniN / popN`; trainer.py _neg_sample_batch_eval + collector.py
         eval_batch_collect): candidates [B, 1+N] int64 with the positive in column 0 (written there from `positive` when
         given).  Encodes each sequence once (the reference predicts on the interaction repeated 1+N times) and ranks the
-        calibrated scores -> (scores [B, 1+N], rec_topk [B, k+1]), and with counts=True the counts [B, 3] of ops.candidate_rank."""
+        calibrated scores -> (scores [B, 1+N], rec_topk [B, k+1]), and with counts=True the counts [B, 3] of ops.candidate_rank.
+        Vocab-parallel: each candidate is scored on its owner's rows (dist.VocabParallel.sampled_rank); every rank calls with
+        the same B."""
         vp = getattr(self, '_vp', None)
-        if vp is not None and vp.sharded:
-            raise ValueError('sampled evaluation is not implemented for a vocab-sharded item table')
         if positive is not None:
             candidates[:, 0].copy_(positive)
         was = ops.LIB.query('acsr_set_pdl', 1)
         try:
             out, _ = self._encode(interaction[self.ITEM_SEQ], interaction[self.ITEM_SEQ_LEN], need_attacked=False)
-            r = ops.candidate_rank(out, self.item_embedding.weight, candidates, k, want_scores=True, want_counts=counts)
+            if vp is not None:
+                r = vp.sampled_rank(out, self.item_embedding.weight, candidates, k, counts=counts)
+            else:
+                r = ops.candidate_rank(out, self.item_embedding.weight, candidates, k, want_scores=True, want_counts=counts)
             return (r[1], r[0]) + tuple(r[2:])
         finally:
             ops.LIB.query('acsr_set_pdl', was)

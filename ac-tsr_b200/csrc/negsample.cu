@@ -10,6 +10,9 @@
 //   acsr_candidate_rank  one CTA per row: fp32 gather-dots of out[m] with the candidates' table rows, and the rank of the
 //                        positive = number of DISTINCT negatives scoring strictly higher (a shared-memory hash set de-duplicates
 //                        only those), written as the [M, kmax+1] hit-flag matrix the evaluator consumes.
+// Over a vocab-sharded table the two halves of acsr_candidate_rank run apart: acsr_candidate_scores_shard scores every rank's
+// rows against the owned candidates (0 elsewhere, with the same group_dot, so a sum over ranks is the unsharded score bit for
+// bit), and acsr_candidate_rank_scores ranks a row's summed scores with candidate_rank_kernel's own ranking code (PRE).
 #include "acsr_common.cuh"
 #include "../../include/acsr.h"
 
@@ -125,7 +128,8 @@ __device__ __forceinline__ float group_dot(const float4* __restrict__ o4, const 
 
 // COUNT: every candidate id enters the hash set (the positive's first), and counts[m] = (distinct negatives scoring above the
 // positive = the rank, distinct negatives tied with it, distinct candidates = the finite entries of the scattered score row)
-template <int G, bool COUNT>
+// PRE: the scores are read from `scores` [M, C] instead of computed (out / table unused, d = 0, G = 1: one candidate a thread)
+template <int G, bool COUNT, bool PRE = false>
 __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const float* __restrict__ out, const float* __restrict__ table,
                                                                       long long V, int d, const long long* __restrict__ cand, int C,
                                                                       int kmax, int hash_size, int* __restrict__ rec,
@@ -141,18 +145,20 @@ __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const floa
   if (tid == 0) { s_rank = 0; s_eq = 0; s_distinct = 1; }
   pdl_wait();
   const int d4 = d >> 2;
-  const float4* orow = reinterpret_cast<const float4*>(out + (long long)m * d);
-  for (int i = tid; i < d4; i += kRankThreads) o4[i] = orow[i];
+  if (!PRE) {
+    const float4* orow = reinterpret_cast<const float4*>(out + (long long)m * d);
+    for (int i = tid; i < d4; i += kRankThreads) o4[i] = orow[i];
+  }
   __syncthreads();
   const long long* crow = cand + (long long)m * C;
   const int lane = tid & 31, sub = lane & (G - 1);
   if (tid < 32) {
     long long id = crow[0];
     id = id < 0 ? 0 : (id >= V ? V - 1 : id);
-    const float s = group_dot<G>(o4, reinterpret_cast<const float4*>(table + id * d), d4, sub);
+    const float s = PRE ? scores[(long long)m * C] : group_dot<G>(o4, reinterpret_cast<const float4*>(table + id * d), d4, sub);
     if (tid == 0) {
       s_pos = s;
-      if (scores != nullptr) scores[(long long)m * C] = s;
+      if (!PRE && scores != nullptr) scores[(long long)m * C] = s;
     }
   }
   const unsigned mask = (unsigned)hash_size - 1;
@@ -166,9 +172,10 @@ __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const floa
     const bool live = c < C;
     long long id = live ? crow[c] : 0;
     id = id < 0 ? 0 : (id >= V ? V - 1 : id);
-    const float s = group_dot<G>(o4, reinterpret_cast<const float4*>(table + id * d), d4, sub);
+    const float s = PRE ? (live ? scores[(long long)m * C + c] : 0.f)
+                        : group_dot<G>(o4, reinterpret_cast<const float4*>(table + id * d), d4, sub);
     if (live && sub == 0) {
-      if (scores != nullptr) scores[(long long)m * C + c] = s;
+      if (!PRE && scores != nullptr) scores[(long long)m * C + c] = s;
       if (COUNT) {
         unsigned h = hash_slot(id, mask);
         while (true) {
@@ -203,6 +210,37 @@ __global__ void __launch_bounds__(kRankThreads) candidate_rank_kernel(const floa
     counts[3 * m] = rank;
     counts[3 * m + 1] = s_eq;
     counts[3 * m + 2] = s_distinct;
+  }
+}
+
+// scores[m, c] = out[m] . shard[id - lo] for an owned candidate id (cand[m, c] clamped to [0, V) as candidate_rank_kernel
+// clamps), 0 otherwise: candidate_rank_kernel's grid, lane groups and group_dot<G>, so an owned score is its score bit for bit
+template <int G>
+__global__ void __launch_bounds__(kRankThreads) candidate_scores_shard_kernel(const float* __restrict__ out,
+                                                                              const float* __restrict__ shard, long long lo,
+                                                                              long long hi, long long V, int d,
+                                                                              const long long* __restrict__ cand, int C,
+                                                                              float* __restrict__ scores) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float4* o4 = reinterpret_cast<float4*>(smem_raw);
+  pdl_launch_dependents();
+  pdl_wait();
+  const int m = blockIdx.x, tid = threadIdx.x;
+  const int d4 = d >> 2;
+  const float4* orow = reinterpret_cast<const float4*>(out + (long long)m * d);
+  for (int i = tid; i < d4; i += kRankThreads) o4[i] = orow[i];
+  __syncthreads();
+  const long long* crow = cand + (long long)m * C;
+  const int lane = tid & 31, sub = lane & (G - 1);
+  const int groups = kRankThreads / G;
+  for (int c = tid / G; c - (tid / G) < C; c += groups) {             // every lane of a warp iterates the same number of times
+    const bool live = c < C;
+    long long id = live ? crow[c] : 0;
+    id = id < 0 ? 0 : (id >= V ? V - 1 : id);
+    const bool own = live && id >= lo && id < hi;
+    // a row this rank does not own runs no loads: the group's sum is exactly 0
+    const float s = group_dot<G>(o4, reinterpret_cast<const float4*>(shard + (own ? id - lo : 0) * d), own ? d4 : 0, sub);
+    if (live && sub == 0) scores[(long long)m * C + c] = s;
   }
 }
 
@@ -283,6 +321,62 @@ int acsr_candidate_rank_counts(const float* out, const float* table, int64_t V, 
                                int32_t* rec, float* scores, int32_t* counts, void* stream) {
   ACSR_REQUIRE(counts, "candidate_rank_counts: NULL counts");
   return candidate_rank_impl(out, table, V, d, cand, M, n_cand, kmax, rec, scores, counts, stream);
+}
+
+int acsr_candidate_scores_shard(const float* out, const float* shard, int64_t lo, int64_t hi, int64_t V, int d, const int64_t* cand,
+                                int M, int n_cand, float* scores, void* stream) {
+  ACSR_REQUIRE(out && shard && cand && scores, "candidate_scores_shard: NULL pointer");
+  ACSR_REQUIRE(M > 0 && V > 0 && n_cand >= 1, "candidate_scores_shard: bad sizes");
+  ACSR_REQUIRE(lo >= 0 && lo < hi && hi <= V, "candidate_scores_shard: rows [%lld, %lld) not a non-empty range of [0, %lld)",
+               (long long)lo, (long long)hi, (long long)V);
+  ACSR_REQUIRE(d > 0 && d % 4 == 0, "candidate_scores_shard: hidden size %d must be a positive multiple of 4", d);
+  if (d > 1024) { set_error("candidate_scores_shard: hidden size %d unsupported (at most 1024)", d); return ACSR_ERR_UNSUPPORTED; }
+  if (n_cand > kRankMaxCand) {
+    set_error("candidate_scores_shard: %d candidates per row unsupported (1 + N <= %d)", n_cand, kRankMaxCand);
+    return ACSR_ERR_UNSUPPORTED;
+  }
+  ACSR_REQUIRE(((uintptr_t)out & 15) == 0 && ((uintptr_t)shard & 15) == 0, "candidate_scores_shard: out / shard must be 16-byte aligned");
+  const size_t smem = (size_t)d * 4;
+  const int d4 = d / 4;
+  cudaStream_t st = (cudaStream_t)stream;
+#define ACSR_SCORES_LAUNCH(G)                                                                                                   \
+  launch_pdl(candidate_scores_shard_kernel<G>, dim3(M), dim3(kRankThreads), smem, st, out, shard, (long long)lo, (long long)hi, \
+             (long long)V, d, (const long long*)cand, n_cand, scores)
+  if (d4 > 16) ACSR_SCORES_LAUNCH(32);          // the G of candidate_rank_impl: the same group_dot, the same bits
+  else if (d4 > 8) ACSR_SCORES_LAUNCH(16);
+  else if (d4 > 4) ACSR_SCORES_LAUNCH(8);
+  else ACSR_SCORES_LAUNCH(4);
+#undef ACSR_SCORES_LAUNCH
+  return check_launch("candidate_scores_shard");
+}
+
+int acsr_candidate_rank_scores(const float* scores, const int64_t* cand, int64_t V, int M, int n_cand, int kmax, int32_t* rec,
+                               int32_t* counts, void* stream) {
+  ACSR_REQUIRE(scores && cand && rec, "candidate_rank_scores: NULL pointer");
+  ACSR_REQUIRE(M > 0 && V > 0 && n_cand >= 1 && kmax >= 1, "candidate_rank_scores: bad sizes");
+  if (n_cand > kRankMaxCand) {
+    set_error("candidate_rank_scores: %d candidates per row unsupported (1 + N <= %d)", n_cand, kRankMaxCand);
+    return ACSR_ERR_UNSUPPORTED;
+  }
+  if (kmax > kRankMaxK) { set_error("candidate_rank_scores: kmax=%d unsupported (1..%d)", kmax, kRankMaxK); return ACSR_ERR_UNSUPPORTED; }
+  int hash_size = 64;
+  while (hash_size < 2 * n_cand) hash_size <<= 1;
+  const size_t smem = (size_t)hash_size * 8;
+  cudaStream_t st = (cudaStream_t)stream;
+  // the kernel only reads `scores` under PRE
+  float* sc = const_cast<float*>(scores);
+  if (counts != nullptr) {
+    cudaError_t e = cudaFuncSetAttribute(candidate_rank_kernel<1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) { set_error("candidate_rank_scores: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
+    launch_pdl(candidate_rank_kernel<1, true, true>, dim3(M), dim3(kRankThreads), smem, st, (const float*)nullptr,
+               (const float*)nullptr, (long long)V, 0, (const long long*)cand, n_cand, kmax, hash_size, (int*)rec, sc, (int*)counts);
+  } else {
+    cudaError_t e = cudaFuncSetAttribute(candidate_rank_kernel<1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) { set_error("candidate_rank_scores: smem attr: %s", cudaGetErrorString(e)); return ACSR_ERR_CUDA; }
+    launch_pdl(candidate_rank_kernel<1, false, true>, dim3(M), dim3(kRankThreads), smem, st, (const float*)nullptr,
+               (const float*)nullptr, (long long)V, 0, (const long long*)cand, n_cand, kmax, hash_size, (int*)rec, sc, (int*)nullptr);
+  }
+  return check_launch("candidate_rank_scores");
 }
 
 }  // extern "C"

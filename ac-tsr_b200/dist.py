@@ -17,8 +17,15 @@ Two storage modes:
               backward: d_out partial = G.E_shard and dE_shard = G^T.out_calibrated with the shard-local G recomputed tile by
               tile inside the two kernels (acsr_ce_bwd_dout / _dtable: no gradient matrix in HBM); reduce-scatter(sum) of
               d_out; dE_shard needs no traffic.
+  training, loss_type BPR: all-gather `out` and the (pos, neg) ids -> every rank computes the (s_pos, s_neg) dot partials of
+              the ids it owns for ALL rows (0 for the others, acsr_bpr_dots_shard) -> reduce-scatter(sum) of the [W*R, 2] dots, exact
+              because each dot has one non-zero term -> local x, row losses and means; backward: all-gather of (row_x, row_scale) ->
+              owned part of d_out and dE of the owned rows (acsr_bpr_loss_bwd_shard) -> reduce-scatter(sum) of d_out.
   evaluation: all-gather `out` -> fused top-k on the shard (indices offset by the shard start, column 0 skipped on shard 0)
               -> merge of the shard's chunk lists into one list per row -> all-gather of those lists -> merge of the rank's own rows.
+  sampled evaluation: all-gather `out` and the candidate ids (every rank draws its own rows' negatives) -> scores of the owned
+              candidates for ALL rows (0 for the others, acsr_candidate_scores_shard) -> reduce-scatter(sum) of the [W*R, 1+N] scores
+              -> the rank's own rows ranked (acsr_candidate_rank_scores), bit-identical to acsr_candidate_rank on the full table.
 
 The collective plumbing is backend-agnostic: `compute` supplies the local kernels (CUDA ops by default; the gloo CPU tests
 inject torch restatements), so world_size-2 tests run without a GPU.  Nothing here allocates by value from the host inside the
@@ -89,6 +96,21 @@ class CudaCompute(object):
     def scatter_add_rows(self, ids, rows, lo, hi, shard_grad):
         self.LIB.call('acsr_shard_scatter_add_rows', self.ops._p(ids, torch.int64), ids.numel(), self.ops._p(rows), lo, hi, rows.shape[1],
                       self.ops._p(shard_grad), self.ops._stream())
+
+    def candidate_scores_shard(self, out, shard, lo, hi, V, cand):
+        return self.ops.candidate_scores_shard(out, shard, lo, hi, V, cand)
+
+    def candidate_rank_scores(self, scores, cand, V, k, counts):
+        return self.ops.candidate_rank_scores(scores, cand, V, k, want_counts=counts)
+
+    def bpr_dots_shard(self, out, shard, lo, hi, V, pos, neg):
+        return self.ops.bpr_dots_shard(out, shard, lo, hi, V, pos, neg)
+
+    def bpr_loss_from_dots(self, dots, n_groups, gamma):
+        return self.ops.bpr_loss_from_dots(dots, n_groups, gamma)
+
+    def bpr_loss_bwd_shard(self, out, shard, lo, hi, V, pos, neg, row_x, row_scale, gamma, row_begin, row_end, shard_grad):
+        return self.ops.bpr_loss_bwd_shard(out, shard, lo, hi, V, pos, neg, row_x, row_scale, gamma, row_begin, row_end, shard_grad)
 
 
 class VocabParallel(object):
@@ -208,6 +230,61 @@ class VocabParallel(object):
         # back to [rank][group][row] blocks, then every rank receives the sum of its own rows
         d_out_all = d_out_all.view(n_groups, W, per, d).permute(1, 0, 2, 3).reshape(W * R, d)
         return self._reduce_scatter(d_out_all, R)
+
+    def _group_major(self, t_local, n_groups):
+        """[R, ...] of every rank -> [W*R, ...] laid out [group][rank][row] (ce_forward's layout)"""
+        R = t_local.shape[0]
+        rest = tuple(t_local.shape[1:])
+        g = self._all_gather(t_local.reshape((n_groups, R // n_groups) + rest))           # [W, n_groups, per, ...]
+        return g.transpose(0, 1).reshape((self.world * R,) + rest).contiguous()
+
+    def _rank_major(self, t_all, n_groups):
+        """[W*R, ...] in [group][rank][row] -> [rank][group][row], the blocks _reduce_scatter hands to each rank"""
+        W = self.world
+        rest = tuple(t_all.shape[1:])
+        per = t_all.shape[0] // (W * n_groups)
+        return t_all.reshape((n_groups, W, per) + rest).transpose(0, 1).reshape(t_all.shape)
+
+    def bpr_forward(self, out_local, table, pos_local, neg_local, n_groups, gamma):
+        """loss_type BPR over the table rows: -> (loss [n_groups] over this rank's rows, saved state for bpr_backward).  Every
+        rank computes the (s_pos, s_neg) partials of the ids it owns for the rows of all ranks (ce_forward's group-major layout);
+        a reduce-scatter(sum) hands each rank the exact dots of its own rows, from which it forms x, the row losses and the means."""
+        R, d = out_local.shape
+        out_all = self._group_major(out_local, n_groups)
+        pos_all = self._group_major(pos_local, n_groups)
+        neg_all = self._group_major(neg_local, n_groups)
+        dots_all = self.compute.bpr_dots_shard(out_all, self.shard(table), self.lo, self.hi, self.V, pos_all, neg_all)   # [W*R, 2]
+        dots = self._reduce_scatter(self._rank_major(dots_all, n_groups), R)
+        loss, row_x = self.compute.bpr_loss_from_dots(dots, n_groups, gamma)
+        return loss, dict(out_all=out_all, pos_all=pos_all, neg_all=neg_all, row_x=row_x, R=R, n_groups=n_groups, gamma=gamma)
+
+    def bpr_backward(self, st, table, row_scale_local, table_grad=None, table_half=None):
+        """row_scale_local [R]: d loss / d row_loss of this rank's rows.  -> d_out_local [R, d]; when table_grad is given, dE of
+        the owned ids from row group `table_half` of every rank is added into it (the stored gradient shard, or rows [lo, hi) of a
+        full-size gradient), as ce_backward does."""
+        R, W, n_groups = st['R'], self.world, st['n_groups']
+        per = R // n_groups
+        xs = self._group_major(torch.stack((st['row_x'], row_scale_local.to(st['row_x'].dtype)), 1), n_groups)       # [W*R, 2]
+        tg = self.shard(table_grad) if table_grad is not None else None
+        begin = (table_half or 0) * W * per
+        d_out_all = self.compute.bpr_loss_bwd_shard(st['out_all'], self.shard(table), self.lo, self.hi, self.V, st['pos_all'],
+                                                    st['neg_all'], xs[:, 0].contiguous(), xs[:, 1].contiguous(), st['gamma'],
+                                                    begin, begin + W * per, tg)
+        return self._reduce_scatter(self._rank_major(d_out_all, n_groups), R)
+
+    # ------------------------------------------------------------------------------------------
+    def sampled_rank(self, out_local, table, cand_local, k, counts=False):
+        """sampled-candidate ranking (ops.candidate_rank) over the table rows: every rank scores the candidates it owns for the
+        rows of all ranks (0 for the others), a reduce-scatter(sum) hands each rank the exact scores of its own rows, which it
+        ranks.  cand_local [R, 1+N] holds this rank's candidates, the positive in column 0.  -> (rec [R, k+1], scores [R, 1+N])
+        and with counts=True the counts [R, 3] as a third entry."""
+        R, d = out_local.shape
+        out_all = self._all_gather(out_local).view(self.world * R, d)
+        cand_all = self._all_gather(cand_local).view(self.world * R, -1)
+        part = self.compute.candidate_scores_shard(out_all, self.shard(table), self.lo, self.hi, self.V, cand_all)
+        scores = self._reduce_scatter(part, R)
+        rec, cnt = self.compute.candidate_rank_scores(scores, cand_local, self.V, k, counts)
+        return (rec, scores, cnt) if counts else (rec, scores)
 
     # ------------------------------------------------------------------------------------------
     def full_sort_topk(self, out_local, table, k, positive_local=None, counts=False):

@@ -207,20 +207,22 @@ class FusedTrainStep(object):
         st = _stream()
         passes = m.logits_passes
         vst = None
-        if self.vp is not None:       # all-gather out -> shard-local partial CE -> all-gather (max, sum-exp) -> combine
+        bpr = m.loss_type == 'BPR'
+        if self.vp is not None and not bpr:       # all-gather out -> shard-local partial CE -> all-gather (max, sum-exp) -> combine
             loss2, vst = self.vp.ce_forward(jb['out2'], E, jb['target2'], 2)
             jb['loss'].copy_(loss2)
         wp = m.mask_loss_weight.detach() if m.trainable_mask_loss_weight else None
         wv = 0.0 if wp is not None else float(m.mask_loss_weight)
-        bpr = m.loss_type == 'BPR'
         if bpr:
             # acsasrec.py:109-116: one sampled negative per row; rows [0,B) calibrated, [B,2B) attacked share the two kernels
-            if self.vp is not None:
-                raise NotImplementedError('vocab-parallel logits are a CE construct; loss_type BPR touches two table rows per sequence')
             neg_items = interaction[m.NEG_ITEM_ID]
             torch.cat((neg_items, neg_items), out=jb['neg2'])
-            LIB.call('acsr_bpr_loss_fwd', _p(jb['out2']), _p(E), _p(jb['target2'], torch.int64), _p(jb['neg2'], torch.int64), 2 * B, d, 2,
-                     float(m.loss_fct.gamma), _p(jb['row_x']), _p(jb['row_loss']), _p(jb['loss']), st)
+            if self.vp is not None:   # all-gather out and ids -> owned (s_pos, s_neg) partials -> reduce-scatter -> loss
+                loss2, vst = self.vp.bpr_forward(jb['out2'], E, jb['target2'], jb['neg2'], 2, float(m.loss_fct.gamma))
+                jb['loss'].copy_(loss2)
+            else:
+                LIB.call('acsr_bpr_loss_fwd', _p(jb['out2']), _p(E), _p(jb['target2'], torch.int64), _p(jb['neg2'], torch.int64), 2 * B,
+                         d, 2, float(m.loss_fct.gamma), _p(jb['row_x']), _p(jb['row_loss']), _p(jb['loss']), st)
             LIB.call('acsr_loss_combine', jb['pen'].data_ptr(), N, _p(jb['loss'][1:]), _p(wp), wv, _p(jb['loss_att']), _p(jb['dpen']), st)
         elif self.vp is None:
             # per-chunk (max, sum-exp) -> lse / target logit / row losses -> the two CE means -> pen_l = sqrt(sum (1-M_l)^2),
@@ -242,7 +244,9 @@ class FusedTrainStep(object):
         # ---------------- backward ----------------
         dpen = jb['dpen']
         main.wait_event(zero_done)
-        if bpr:                       # d_out2 = +-g (E[pos] - E[neg]) / B ; the calibrated rows scatter +-g.out into dE[pos], dE[neg]
+        if bpr and self.vp is not None:     # owned parts of d_out2 reduce-scattered; dE of the calibrated rows into the owner's rows
+            jb['d_out2'].copy_(self.vp.bpr_backward(vst, E, jb['row_scale'], E.grad, table_half=0))
+        elif bpr:                     # d_out2 = +-g (E[pos] - E[neg]) / B ; the calibrated rows scatter +-g.out into dE[pos], dE[neg]
             LIB.call('acsr_bpr_loss_bwd', _p(jb['out2']), _p(E), _p(jb['target2'], torch.int64), _p(jb['neg2'], torch.int64),
                      _p(jb['row_x']), _p(jb['row_scale']), 2 * B, d, float(m.loss_fct.gamma), 0, B, _p(jb['d_out2']), _p(E.grad), st)
         elif self.vp is not None:       # shard-local G^T, reduce-scatter of d_out, dE into the owner's rows

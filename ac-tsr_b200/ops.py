@@ -776,6 +776,41 @@ class BprLossFn(torch.autograd.Function):
         return d_out, d_table, None, None, None, None
 
 
+def bpr_dots_shard(out, shard, lo, hi, V, pos_items, neg_items):
+    """dots [M, 2] = (out . E[pos], out . E[neg]) over the ids this rank owns (E[i] = shard[i - lo] for i in [lo, hi)), 0 for
+    the others: summed over the ranks, BprLossFn's two scores bit for bit (acsr_bpr_dots_shard)"""
+    out, pos_items, neg_items = out.contiguous(), pos_items.contiguous(), neg_items.contiguous()
+    M, d = out.shape
+    dots = torch.empty((M, 2), dtype=torch.float32, device=out.device)
+    LIB.call('acsr_bpr_dots_shard', _p(out), _p(shard.contiguous()), int(lo), int(hi), int(V), _p(pos_items, torch.int64),
+             _p(neg_items, torch.int64), M, d, _p(dots), _stream())
+    return dots
+
+
+def bpr_loss_from_dots(dots, n_groups, gamma):
+    """summed dots [M, 2] -> (loss [n_groups], row_x [M]) as BprLossFn's forward computes them (acsr_bpr_loss_from_dots)"""
+    dots = dots.contiguous()
+    M = dots.shape[0]
+    row_x = torch.empty(M, dtype=torch.float32, device=dots.device)
+    row_loss = torch.empty(M, dtype=torch.float32, device=dots.device)
+    loss = torch.empty(n_groups, dtype=torch.float32, device=dots.device)
+    LIB.call('acsr_bpr_loss_from_dots', _p(dots), M, int(n_groups), float(gamma), _p(row_x), _p(row_loss), _p(loss), _stream())
+    return loss, row_x
+
+
+def bpr_loss_bwd_shard(out, shard, lo, hi, V, pos_items, neg_items, row_x, row_scale, gamma, table_row_begin=0, table_row_end=0,
+                       shard_grad=None):
+    """BprLossFn's backward over the ids this rank owns (acsr_bpr_loss_bwd_shard) -> d_out [M, d], this rank's part of
+    g * (E[pos] - E[neg]); rows [table_row_begin, table_row_end) add +-g * out into shard_grad rows of owned ids"""
+    out = out.contiguous()
+    M, d = out.shape
+    d_out = torch.empty_like(out)
+    LIB.call('acsr_bpr_loss_bwd_shard', _p(out), _p(shard.contiguous()), int(lo), int(hi), int(V), _p(pos_items.contiguous(), torch.int64),
+             _p(neg_items.contiguous(), torch.int64), _p(row_x.contiguous()), _p(row_scale.contiguous()), M, d, float(gamma),
+             int(table_row_begin), int(table_row_end), _p(d_out), _p(shard_grad), _stream())
+    return d_out
+
+
 def logits_scores(out, table, passes=3):
     """scores [M,V] = out.E^T (contiguous)  -- acsasrec.py:162-163."""
     out, table = out.contiguous(), table.contiguous()
@@ -977,6 +1012,37 @@ def candidate_rank(out, table, cand, k, want_scores=False, want_counts=False):
     LIB.call('acsr_candidate_rank', _p(out), _p(table), table.shape[0], d, _p(cand, torch.int64), M, cand.shape[1], int(k),
              _p(rec, torch.int32), _p(scores), _stream())
     return rec, scores
+
+
+def candidate_scores_shard(out, shard, lo, hi, V, cand):
+    """scores [M, 1+N] = out[m] . shard[id - lo] for the candidate ids (clamped to [0, V)) this rank owns, 0 for the others:
+    the sum over the ranks is candidate_rank's scores bit for bit (acsr_candidate_scores_shard)"""
+    out, cand = out.contiguous(), cand.contiguous()
+    if out.dim() != 2 or shard.dim() != 2 or cand.dim() != 2 or shard.shape[1] != out.shape[1] or cand.shape[0] != out.shape[0]:
+        raise AcsrError('candidate_scores_shard: out [M, d], shard [rows, d] and cand [M, 1+N] disagree (%s, %s, %s)'
+                        % (tuple(out.shape), tuple(shard.shape), tuple(cand.shape)))
+    if int(hi) - int(lo) > shard.shape[0]:
+        raise AcsrError('candidate_scores_shard: rows [%d, %d) exceed the %d rows of the shard' % (int(lo), int(hi), shard.shape[0]))
+    M, d = out.shape
+    scores = torch.empty(cand.shape, dtype=torch.float32, device=out.device)
+    LIB.call('acsr_candidate_scores_shard', _p(out), _p(shard.contiguous()), int(lo), int(hi), int(V), d, _p(cand, torch.int64), M,
+             cand.shape[1], _p(scores), _stream())
+    return scores
+
+
+def candidate_rank_scores(scores, cand, V, k, want_counts=False):
+    """candidate_rank's ranking of precomputed scores [M, 1+N] (acsr_candidate_rank_scores) -> (rec [M, k+1] int32, counts
+    [M, 3] int32 | None)"""
+    scores, cand = scores.contiguous(), cand.contiguous()
+    if scores.dtype != torch.float32 or scores.dim() != 2 or tuple(cand.shape) != tuple(scores.shape) or int(k) < 1:
+        raise AcsrError('candidate_rank_scores: float32 scores %s and cand %s must have one shape (and k=%d >= 1)'
+                        % (tuple(scores.shape), tuple(cand.shape), int(k)))
+    M = scores.shape[0]
+    rec = torch.empty((M, k + 1), dtype=torch.int32, device=scores.device)
+    counts = torch.empty((M, 3), dtype=torch.int32, device=scores.device) if want_counts else None
+    LIB.call('acsr_candidate_rank_scores', _p(scores), _p(cand, torch.int64), int(V), M, scores.shape[1], int(k), _p(rec, torch.int32),
+             _p(counts, torch.int32), _stream())
+    return rec, counts
 
 
 def used_item_csr(uid, iid, n_users, n_items):

@@ -271,7 +271,9 @@ class ACSASRecTrainer(object):
     def enable_data_parallel(self, vocab_parallel=False, shard_table=None):
         """One process per GPU: broadcast rank 0's weights, then all-reduce gradients every step (batch data-parallel).
         vocab_parallel=True additionally splits the full-catalogue logits / CE / top-k by item rows across ranks
-        (dist.VocabParallel: all-gather of `out`, all-gather of per-row (max, sum-exp, target logit), reduce-scatter of d_out).
+        (dist.VocabParallel: all-gather of `out`, all-gather of per-row (max, sum-exp, target logit), reduce-scatter of d_out);
+        under loss_type BPR the two table rows of each row are scored by their owners (reduce-scatter of the dots and of d_out),
+        and sampled evaluation scores each candidate on its owner's rows.
         shard_table=True (default for catalogues above the break-even 2*W*B*L rows, see dist.py) also shards the STORAGE: this
         rank keeps rows [lo, hi) of the item table, their gradient and their Adam moments; the embedding rows of its own tokens
         are exchanged every step and the data-parallel all-reduce shrinks to the encoder parameters."""
@@ -283,8 +285,8 @@ class ACSASRecTrainer(object):
         self.vp = None
         if not vocab_parallel:
             return
-        if self.fused is None or self.model.loss_type != 'CE':
-            raise ValueError('vocab-parallel logits need the fused step with loss_type CE')
+        if self.fused is None:
+            raise ValueError('vocab-parallel logits need the fused step (loss_type CE or BPR)')
         from .dist import VocabParallel, CudaCompute
         m = self.model
         if shard_table is None:
@@ -785,15 +787,13 @@ class ACSASRecTrainer(object):
     @torch.no_grad()
     def _sampled_eval(self, interaction, positive_i, sampler, N, kmax, rec_out=None, need=None):
         """one batch of sampled-candidate evaluation: sampler -> encoder -> acsr_candidate_rank, eagerly or as a CUDA-graph
-        replay (one graph per batch shape and `need`; every replay draws fresh negatives)"""
+        replay (one graph per batch shape and `need`; every replay draws fresh negatives).  Vocab-parallel: every rank draws its
+        own rows' negatives and the graph captures the collectives of VocabParallel.sampled_rank."""
         m = self.model
         if need is not None and need[1]:
             raise NotImplementedError('the item-distribution metrics (ItemCoverage, AveragePopularity, GiniIndex, ShannonEntropy, '
                                       'TailPercentage) are not available in sampled evaluation (eval_args.mode uniN / popN): '
                                       'use full-sort evaluation for them')
-        if self._sharded():
-            raise ValueError('sampled evaluation (eval_args.mode uniN / popN) needs the replicated item table; '
-                             'it is not implemented for a vocab-sharded table')
         if not hasattr(m, 'sampled_topk'):
             raise NotImplementedError('%s has no sampled_topk: sampled evaluation is not available for it' % type(m).__name__)
         dev = self.device

@@ -455,6 +455,19 @@ int acsr_bpr_loss_fwd(const float* out, const float* table, const int64_t* pos_i
 int acsr_bpr_loss_bwd(const float* out, const float* table, const int64_t* pos_items, const int64_t* neg_items, const float* row_x,
                       const float* row_scale, int M, int d, float gamma, int table_row_begin, int table_row_end, float* d_out,
                       float* d_table, void* stream);
+/* the same over a vocab-sharded table (dist.VocabParallel): this rank holds rows [lo, hi) of the V-row table as shard[0, hi-lo).
+ * acsr_bpr_dots_shard: dots [M, 2] = (out_m . E[pos_m], out_m . E[neg_m]) for owned ids, 0 for the others, in acsr_bpr_loss_fwd's
+ * arithmetic: summed over ranks, the dots are acsr_bpr_loss_fwd's two scores bit for bit.  acsr_bpr_loss_from_dots: row_x,
+ * row_loss and loss of acsr_bpr_loss_fwd from the summed dots.  acsr_bpr_loss_bwd_shard: acsr_bpr_loss_bwd with the rows of
+ * unowned ids read as 0 in d_out (the ranks' d_out sum to g * (E[pos] - E[neg])) and only owned ids scattered into d_shard_grad
+ * (rows [0, hi-lo)). */
+int acsr_bpr_dots_shard(const float* out, const float* shard, int64_t lo, int64_t hi, int64_t V, const int64_t* pos_items,
+                        const int64_t* neg_items, int M, int d, float* dots, void* stream);
+int acsr_bpr_loss_from_dots(const float* dots, int M, int n_groups, float gamma, float* row_x, float* row_loss, float* loss,
+                            void* stream);
+int acsr_bpr_loss_bwd_shard(const float* out, const float* shard, int64_t lo, int64_t hi, int64_t V, const int64_t* pos_items,
+                            const int64_t* neg_items, const float* row_x, const float* row_scale, int M, int d, float gamma,
+                            int table_row_begin, int table_row_end, float* d_out, float* d_shard_grad, void* stream);
 
 /* ---- vocab-sharded item table (north_star; the reference has only the dense nn.Embedding of acsasrec.py:37) ----
  * this rank stores table rows [row_lo, row_hi).  gather: out[i] = shard[ids[i] - row_lo] when the row is owned, else 0 (the owners'
@@ -505,6 +518,14 @@ int acsr_candidate_rank(const float* out, const float* table, int64_t V, int d, 
  * candidates including the positive): GAUC's rank inputs and user_len, the number of finite entries of the scattered row. */
 int acsr_candidate_rank_counts(const float* out, const float* table, int64_t V, int d, const int64_t* cand, int M, int n_cand, int kmax,
                                int32_t* rec, float* scores, int32_t* counts, void* stream);
+/* acsr_candidate_rank split in two for a vocab-sharded table (dist.VocabParallel).  acsr_candidate_scores_shard: scores[m, c] =
+ * out[m] . shard[id - lo] where id = cand[m, c] clamped to [0, V) lies in this rank's rows [lo, hi), else 0; each owned score is
+ * bit for bit the one acsr_candidate_rank computes on the full table, so the sum over ranks is exact.  acsr_candidate_rank_scores:
+ * the ranking of acsr_candidate_rank (counts == NULL) or acsr_candidate_rank_counts on precomputed scores [M, n_cand]. */
+int acsr_candidate_scores_shard(const float* out, const float* shard, int64_t lo, int64_t hi, int64_t V, int d, const int64_t* cand,
+                                int M, int n_cand, float* scores, void* stream);
+int acsr_candidate_rank_scores(const float* scores, const int64_t* cand, int64_t V, int M, int n_cand, int kmax, int32_t* rec,
+                               int32_t* counts, void* stream);
 
 /* ---- K13: fused Adam over one flat fp32 buffer (trainer/trainer.py:614-615,687) ---------
  * torch.optim.Adam semantics (no amsgrad); step_count device int64[1], incremented by the call. */
