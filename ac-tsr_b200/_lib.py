@@ -226,6 +226,18 @@ def _ab_bpr_loss_bwd_shard(a):
     return M * (24 + 4 * 2 * d + (4 * d if a[14] else 0)) + n_tab * 4 * (d + 4 * d)
 
 
+def _ab_grad_norm_partial(a):
+    # (grad, n, ranges, n_ranges, norm_type, block_partials, counter, out, stream): the ranges' gradients read once, the norm out
+    rg, nr = a[2], a[3]
+    return 4 * sum(rg[2 * r + 1] - rg[2 * r] for r in range(nr)) + 8
+
+
+def _ab_adam_step_clipped(a):
+    # (param, grad, exp_avg, exp_avg_sq, n, lr, b1, b2, eps, wd, step_count, partials, n_partials, ...): Adam's 28 B per parameter,
+    # the clipped gradient written back, the norm partials read
+    return 32 * a[4] + 8 * a[12]
+
+
 # ALGORITHMIC bytes of one launch, from the call's own arguments (DESIGN.md section 4)
 ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_linear_tok_bdrl,
               'acsr_proj_input_grad': _ab_proj_input_grad, 'acsr_dense_bwd': _ab_dense_bwd,
@@ -233,7 +245,8 @@ ALGO_BYTES = {'acsr_linear_tok': _ab_linear_tok, 'acsr_linear_tok_bdrl': _ab_lin
               'acsr_gemm_batch': _ab_gemm_batch, 'acsr_neg_sample': _ab_neg_sample, 'acsr_candidate_rank': _ab_candidate_rank,
               'acsr_candidate_rank_counts': _ab_candidate_rank_counts, 'acsr_candidate_scores_shard': _ab_candidate_scores_shard,
               'acsr_candidate_rank_scores': _ab_candidate_rank_scores, 'acsr_bpr_dots_shard': _ab_bpr_dots_shard,
-              'acsr_bpr_loss_from_dots': _ab_bpr_loss_from_dots, 'acsr_bpr_loss_bwd_shard': _ab_bpr_loss_bwd_shard}
+              'acsr_bpr_loss_from_dots': _ab_bpr_loss_from_dots, 'acsr_bpr_loss_bwd_shard': _ab_bpr_loss_bwd_shard,
+              'acsr_grad_norm_partial': _ab_grad_norm_partial, 'acsr_adam_step_clipped': _ab_adam_step_clipped}
 
 
 class KernelTimer:

@@ -1,8 +1,10 @@
 // Memory-bound row-wise kernels: K1 (gather + pos + LayerNorm + dropout), the
-// bias+dropout+residual+LayerNorm epilogue, bias+activation, last-position gather, fused Adam.
+// bias+dropout+residual+LayerNorm epilogue, bias+activation, last-position gather, fused Adam (optionally with the
+// gradient clipped by global norm).
 // One warp owns one token row; every lane reads/writes 16-byte (or 8-byte at d=64) vectors so a
 // warp touches whole 128-byte lines; grids are persistent (a multiple of the 148 SMs) and
 // grid-stride over rows so LayerNorm weight/bias gradients are reduced in registers first.
+#include <type_traits>
 #include "acsr_common.cuh"
 #include "../../include/acsr.h"
 
@@ -386,18 +388,47 @@ __global__ void gather_last_bwd_kernel(const float* __restrict__ d_out, const in
 
 // ------------------------------------------------------------------------------------------
 // fused Adam (torch.optim.Adam, amsgrad=False, maximize=False)
+// kClip: torch.nn.utils.clip_grad_norm_ folded in.  Every CTA combines the norm partials of acsr_grad_norm_partial in index
+// order (so every CTA, and every rank, derives the same coefficient), scales the gradient, writes the clipped gradient back
+// (p.grad after clip_grad_norm_) and runs the same update on it.
 // ------------------------------------------------------------------------------------------
-__global__ void adam_kernel(float* __restrict__ param, const float* __restrict__ grad, float* __restrict__ m, float* __restrict__ v,
-                            long long n, float lr, float b1, float b2, float eps, float wd, const long long* __restrict__ step_count) {
+template <bool kClip>
+__global__ void adam_kernel(float* __restrict__ param, std::conditional_t<kClip, float, const float>* __restrict__ grad,
+                            float* __restrict__ m, float* __restrict__ v, long long n, float lr, float b1, float b2, float eps,
+                            float wd, const long long* __restrict__ step_count, const double* __restrict__ partials,
+                            int n_partials, double norm_type, float max_norm, float* __restrict__ total_out) {
   // (no early programmatic-launch trigger: this kernel WRITES the parameters, which later kernels may read ahead of their
   // griddepcontrol.wait -- acsr_register_static -- so nothing that follows may start before it has completed)
   pdl_wait();
+  float coef = 1.f;
+  if constexpr (kClip) {
+    __shared__ float s_coef;
+    if (threadIdx.x == 0) {
+      const bool inf_norm = isinf(norm_type);
+      double s = partials[0];
+      for (int i = 1; i < n_partials; ++i) {
+        const double p = partials[i];
+        s = inf_norm ? ((p > s || p != p) ? p : s) : s + p;         // the max keeps a NaN, as torch's inf-norm does
+      }
+      const float total = (float)(inf_norm || norm_type == 1.0 ? s : norm_type == 2.0 ? sqrt(s) : pow(s, 1.0 / norm_type));
+      // torch: clamp(max_norm / (total + 1e-6), max=1), the division as reciprocal * max_norm; a NaN coefficient propagates
+      const float c = (1.f / (total + 1e-6f)) * max_norm;
+      s_coef = c > 1.f ? 1.f : c;
+      if (blockIdx.x == 0) total_out[0] = total;
+    }
+    __syncthreads();
+    coef = s_coef;
+  }
   const double step = (double)(step_count[0] + 1);
   const float bc1 = (float)(1.0 - pow((double)b1, step));
   const float bc2_sqrt = (float)sqrt(1.0 - pow((double)b2, step));
   const float step_size = lr / bc1;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     float g = grad[i], pm = param[i];
+    if constexpr (kClip) {
+      g *= coef;
+      grad[i] = g;
+    }
     if (wd != 0.f) g += wd * pm;
     float mi = b1 * m[i] + (1.f - b1) * g;
     float vi = b2 * v[i] + (1.f - b2) * g * g;
@@ -529,11 +560,29 @@ int acsr_adam_step(float* param, const float* grad, float* exp_avg, float* exp_a
   ACSR_REQUIRE(param && grad && exp_avg && exp_avg_sq && step_count, "adam_step: NULL pointer");
   if (n > 0) {
     long long need = (n + 255) / 256, cap = kNumSMs * 8;
-    launch_pdl(adam_kernel, dim3((int)(need < cap ? need : cap)), dim3(256), 0, (cudaStream_t)stream, 
-        param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, (const long long*)step_count);
+    launch_pdl(adam_kernel<false>, dim3((int)(need < cap ? need : cap)), dim3(256), 0, (cudaStream_t)stream,
+        param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, (const long long*)step_count,
+        (const double*)nullptr, 0, 0.0, 0.f, (float*)nullptr);
   }
   launch_pdl(step_inc_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, (long long*)step_count);
   return check_launch("adam_step");
+}
+
+int acsr_adam_step_clipped(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
+                           float beta2, float eps, float weight_decay, int64_t* step_count, const double* partials, int n_partials,
+                           double norm_type, float max_norm, float* total_out, void* stream) {
+  ACSR_REQUIRE(param && grad && exp_avg && exp_avg_sq && step_count && partials && total_out, "adam_step_clipped: NULL pointer");
+  ACSR_REQUIRE(n >= 0, "adam_step_clipped: n=%lld", (long long)n);
+  ACSR_REQUIRE(n_partials >= 1 && n_partials <= 1024, "adam_step_clipped: n_partials=%d (need 1..1024)", n_partials);
+  ACSR_REQUIRE(norm_type > 0.0, "adam_step_clipped: norm_type=%f (need a positive number or inf)", norm_type);
+  ACSR_REQUIRE(max_norm > 0.f, "adam_step_clipped: max_norm=%f (need > 0)", max_norm);
+  // one CTA even for n == 0: the norm is still reported
+  long long need = (n + 255) / 256, cap = kNumSMs * 8;
+  launch_pdl(adam_kernel<true>, dim3((int)(need < cap ? (need > 0 ? need : 1) : cap)), dim3(256), 0, (cudaStream_t)stream,
+      param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, (const long long*)step_count,
+      partials, n_partials, norm_type, max_norm, total_out);
+  launch_pdl(step_inc_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, (long long*)step_count);
+  return check_launch("adam_step_clipped");
 }
 
 }  // extern "C"

@@ -4,6 +4,8 @@ PyTorch is plumbing here: it owns device memory, the stream and the autograd tap
 below launches hand-written sm_100a kernels from libacsr.so.  Tensors must be CUDA, contiguous,
 float32 (ids int64) -- anything else raises; there is no CPU or eager fallback.
 """
+import ctypes
+
 import numpy as np
 import torch
 
@@ -1139,6 +1141,37 @@ class NegSampler(object):
 def adam_step(param, grad, exp_avg, exp_avg_sq, step_count, lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0):
     LIB.call('acsr_adam_step', _p(param), _p(grad), _p(exp_avg), _p(exp_avg_sq), param.numel(), lr, beta1, beta2, eps,
              weight_decay, _p(step_count, torch.int64), _stream())
+
+
+def grad_norm_work(device):
+    """scratch of grad_norm_partial: (per-CTA partials, arrival counter).  The counter starts at zero and the kernel leaves it
+    at zero; launches that share one work pair must run in stream order."""
+    return (torch.empty(LIB.query('acsr_grad_norm_max_blocks'), dtype=torch.float64, device=device),
+            torch.zeros(1, dtype=torch.int32, device=device))
+
+
+def grad_norm_partial(grad, norm_type, ranges=None, out=None, work=None):
+    """acsr_grad_norm_partial -> out [1] float64: the sum of |g|^q over grad[begin:end] for every (begin, end) in ranges (default:
+    all of grad), or max |g| for q = norm_type = inf.  acsr_adam_step_clipped combines such partials into the total norm."""
+    ranges = [(0, grad.numel())] if ranges is None else [(int(b), int(e)) for b, e in ranges]
+    rg = (ctypes.c_int64 * (2 * len(ranges)))(*[x for r in ranges for x in r])
+    out = torch.empty(1, dtype=torch.float64, device=grad.device) if out is None else out
+    work = grad_norm_work(grad.device) if work is None else work
+    LIB.call('acsr_grad_norm_partial', _p(grad), grad.numel(), rg, len(ranges), float(norm_type), _p(work[0], torch.float64),
+             _p(work[1], torch.int32), _p(out, torch.float64), _stream())
+    return out
+
+
+def adam_step_clipped(param, grad, exp_avg, exp_avg_sq, step_count, lr, partials, norm_type, max_norm, beta1=0.9, beta2=0.999,
+                      eps=1e-8, weight_decay=0.0, total=None):
+    """acsr_adam_step_clipped: clip_grad_norm_(max_norm, norm_type) with the total norm combined from `partials` (float64 [n],
+    grad_norm_partial results of disjoint ranges, summed in index order), then adam_step on the clipped gradient, which is
+    also written back to grad.  -> total [1] float32, the norm clip_grad_norm_ returns."""
+    total = torch.empty(1, dtype=torch.float32, device=param.device) if total is None else total
+    LIB.call('acsr_adam_step_clipped', _p(param), _p(grad), _p(exp_avg), _p(exp_avg_sq), param.numel(), lr, beta1, beta2, eps,
+             weight_decay, _p(step_count, torch.int64), _p(partials, torch.float64), partials.numel(), float(norm_type),
+             float(max_norm), _p(total), _stream())
+    return total
 
 
 # ------------------------------------------------------------------------------------------

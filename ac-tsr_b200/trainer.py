@@ -42,9 +42,24 @@ def early_stopping(value, best, cur_step, max_step, bigger=True):
 
 
 class FlatAdam(object):
-    """torch.optim.Adam semantics (trainer.py:614-615) over flat buffers; step() is one fused kernel."""
+    """torch.optim.Adam semantics (trainer.py:614-615) over flat buffers; step() is one fused kernel.  With `clip` (device_clip of
+    the `clip_grad_norm` setting) step() first clips the gradient as torch.nn.utils.clip_grad_norm_ does: one norm launch over the
+    flat gradient, and the scale folded into the Adam kernel."""
 
-    def __init__(self, model, lr, weight_decay=0.0, betas=(0.9, 0.999), eps=1e-8):
+    @staticmethod
+    def device_clip(clip_grad_norm):
+        """`clip_grad_norm` (clip_grad_norm_'s keyword arguments) -> (max_norm, norm_type) when step() can clip on the device, else
+        None (unset, or settings only torch's clip_grad_norm_ handles: other keys such as error_if_nonfinite, which needs a host
+        sync, norm_type <= 0, max_norm <= 0)"""
+        if not isinstance(clip_grad_norm, dict) or 'max_norm' not in clip_grad_norm or set(clip_grad_norm) - {'max_norm', 'norm_type'}:
+            return None
+        try:
+            max_norm, norm_type = float(clip_grad_norm['max_norm']), float(clip_grad_norm.get('norm_type', 2.0))
+        except (TypeError, ValueError):
+            return None
+        return (max_norm, norm_type) if max_norm > 0 and norm_type > 0 else None
+
+    def __init__(self, model, lr, weight_decay=0.0, betas=(0.9, 0.999), eps=1e-8, clip=None):
         params = [p for p in model.parameters()]
         dev = params[0].device
         align = 64                      # floats: every group starts on a 256-byte boundary (float4 / bulk-copy loads)
@@ -90,6 +105,13 @@ class FlatAdam(object):
             from ._lib import LIB
             LIB.query('acsr_register_static', self.flat_param.data_ptr(), self.flat_param.numel() * 4)
         self.no_grad_params = [p for n, p in model.named_parameters() if n == 'mask_loss_weight']
+        self.clip = clip
+        self._table_shard = None
+        self._norm_partial = ops.grad_norm_partial       # the local norm kernel (the CPU gloo tests put a torch restatement here)
+        if clip is not None:
+            self._norm_work = ops.grad_norm_work(dev) if self.flat_param.is_cuda else None
+            self._norm_parts = torch.zeros(2, dtype=torch.float64, device=dev)
+            self.grad_norm = torch.zeros(1, dtype=torch.float32, device=dev)      # the total norm of the last step
 
     def stacked(self, plist, grad=False):
         """view of adjacent, equally shaped parameters (or their grads) as one [len, *shape] tensor; None if not adjacent."""
@@ -101,6 +123,28 @@ class FlatAdam(object):
         src = self.flat_grad if grad else self.flat_param
         return src[off0:off0 + len(plist) * k].view(len(plist), *plist[0].shape)
 
+    def slot(self, p):
+        """[begin, end) of the flat buffers reserved for a parameter that forms a group of its own (its padding included)"""
+        a = self.offsets[id(p)]
+        return a, a + (p.numel() + 63) // 64 * 64
+
+    def set_table_shard(self, table, own_elems, all_gather):
+        """the item table `table` is this rank's shard of a vocab-sharded table: its first own_elems gradient entries are this rank's
+        rows, the rest of its slot is padding, and every other parameter is replicated.  The clip norm then combines the partial of
+        the replicated ranges with every rank's shard partial, all_gather(t [1]) -> [world, 1] collecting those in rank order."""
+        a, b = self.slot(table)
+        self._table_shard = ([(0, a), (b, self.flat_grad.numel())], (a, a + int(own_elems)), all_gather)
+
+    def _clip_partials(self):
+        """-> float64 [n] norm partials of the whole (logical) gradient, combined in index order by the clipped Adam"""
+        q, norm = self.clip[1], self._norm_partial
+        if self._table_shard is None:
+            return norm(self.flat_grad, q, out=self._norm_parts[:1], work=self._norm_work)
+        replicated, own, all_gather = self._table_shard
+        norm(self.flat_grad, q, [r for r in replicated if r[1] > r[0]] or [(0, 0)], out=self._norm_parts[:1], work=self._norm_work)
+        norm(self.flat_grad, q, [own], out=self._norm_parts[1:], work=self._norm_work)
+        return torch.cat((self._norm_parts[:1], all_gather(self._norm_parts[1:]).view(-1)))
+
     def zero_grad(self, set_to_none=False):
         self.flat_grad.zero_()
 
@@ -109,8 +153,13 @@ class FlatAdam(object):
         # only enters the attacked loss and is routed away (trainer.py:672-686): with weight decay the flat kernel would
         # still shrink it, so its value is put back after the step
         keep = [(p, p.detach().clone()) for p in self.no_grad_params] if (self.weight_decay and self.no_grad_params) else []
-        ops.adam_step(self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr,
-                      self.betas[0], self.betas[1], self.eps, self.weight_decay)
+        if self.clip is None:
+            ops.adam_step(self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr,
+                          self.betas[0], self.betas[1], self.eps, self.weight_decay)
+        else:
+            ops.adam_step_clipped(self.flat_param, self.flat_grad, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr,
+                                  self._clip_partials(), self.clip[1], self.clip[0], self.betas[0], self.betas[1], self.eps,
+                                  self.weight_decay, total=self.grad_norm)
         for p, v in keep:
             p.data.copy_(v)
 
@@ -207,10 +256,13 @@ class ACSASRecTrainer(object):
         self.dp_world = 1
         self.fused = None
         if (bool(cfg_get(config, 'fused_step', True)) and isinstance(self.optimizer, FlatAdam) and type(model).__name__ == 'ACSASRec'
-                and getattr(model, 'loss_type', None) in ('CE', 'BPR') and not self.clip_grad_norm):
+                and getattr(model, 'loss_type', None) in ('CE', 'BPR') and not self.torch_clip):
             from .fused_step import FusedTrainStep
             self.fused = FusedTrainStep(model, self.optimizer)
             model._fused_step = self.fused          # eval batches reuse the fused forward (ACSASRec._encode)
+        if self.clip_grad_norm:
+            self.logger.info('clip_grad_norm by torch.nn.utils.clip_grad_norm_' if self.torch_clip else
+                             'clip_grad_norm on the device (%s step)' % ('fused' if self.fused is not None else 'autograd'))
         self.nan_check_interval = int(cfg_get(config, 'nan_check_interval', 50))
         # BPR with `neg_sampling` on host-side batches: the ops.NegSampler that draws each step's negatives on the device
         # (set from the training loader by _train_epoch; a DeviceTrainDataLoader draws inside its own gather instead)
@@ -226,7 +278,7 @@ class ACSASRecTrainer(object):
         lr = kwargs.pop('learning_rate', self.learning_rate)
         wd = kwargs.pop('weight_decay', self.weight_decay)
         if learner == 'adam':
-            return FlatAdam(self.model, lr, wd)
+            return FlatAdam(self.model, lr, wd, clip=FlatAdam.device_clip(self.clip_grad_norm))
         import torch.optim as optim         # other learners are outside the hot path: library optimizers
         params = self.model.parameters()
         if learner == 'sgd':
@@ -236,7 +288,13 @@ class ACSASRecTrainer(object):
         if learner == 'rmsprop':
             return optim.RMSprop(params, lr=lr, weight_decay=wd or 0.0)
         self.logger.warning('Received unrecognized optimizer, set default Adam optimizer')
-        return FlatAdam(self.model, lr, 0.0)
+        return FlatAdam(self.model, lr, 0.0, clip=FlatAdam.device_clip(self.clip_grad_norm))
+
+    @property
+    def torch_clip(self):
+        """`clip_grad_norm` is set and the optimizer does not clip on the device (FlatAdam.device_clip): the step calls
+        torch.nn.utils.clip_grad_norm_, which rules out the fused step and the captured graph"""
+        return bool(self.clip_grad_norm) and getattr(self.optimizer, 'clip', None) is None
 
     def _route(self, attack):
         for name, p in self.model.named_parameters():
@@ -263,7 +321,7 @@ class ACSASRecTrainer(object):
             p.requires_grad = True
         if self.dp_world > 1:               # batch data-parallel: average the flat gradient over ranks (NCCL / NVLink)
             self._allreduce_grads()
-        if self.clip_grad_norm:
+        if self.torch_clip:
             torch.nn.utils.clip_grad_norm_(self.model.parameters(), **self.clip_grad_norm)
         self.optimizer.step()
         return attacked_loss.detach(), calibrated_loss.detach()
@@ -303,6 +361,8 @@ class ACSASRecTrainer(object):
             m.item_embedding.weight = torch.nn.Parameter(shard)
             del full
             self.optimizer = self._build_optimizer()
+            E = m.item_embedding.weight
+            self.optimizer.set_table_shard(E, (self.vp.hi - self.vp.lo) * E.shape[1], self.vp._all_gather)
             from .fused_step import FusedTrainStep
             self.fused = FusedTrainStep(m, self.optimizer)
             m._fused_step = self.fused
@@ -317,9 +377,7 @@ class ACSASRecTrainer(object):
         import torch.distributed as dist
         g = self.optimizer.flat_grad
         if self.vp is not None and self.vp.sharded:
-            E = self.model.item_embedding.weight
-            a = self.optimizer.offsets[id(E)]
-            b = a + (E.numel() + 63) // 64 * 64
+            a, b = self.optimizer.slot(self.model.item_embedding.weight)
             if a > 0:
                 dist.all_reduce(g[:a])
             if b < g.numel():
@@ -488,7 +546,7 @@ class ACSASRecTrainer(object):
         # the captured step: AC-SASRec's fused one-pass step, or -- for sibling models whose step has no host-side work
         # (GRAPH_SAFE_STEP) -- the autograd Functions' forward + routed double backward + Adam as they launch
         graph_ok = (self.use_graph and (self.fused is not None or getattr(self.model, 'GRAPH_SAFE_STEP', False))
-                    and isinstance(self.optimizer, FlatAdam) and not self.clip_grad_norm)
+                    and isinstance(self.optimizer, FlatAdam) and not self.torch_clip)
         if not getattr(train_data, 'device_resident', False):
             self.train_neg_sampler = getattr(train_data, 'neg_sampler', None)
         if (getattr(train_data, 'device_resident', False) and graph_ok and self.fused is not None and not self._host_schedule()

@@ -533,6 +533,24 @@ int acsr_adam_step(float* param, const float* grad, float* exp_avg, float* exp_a
                    float lr, float beta1, float beta2, float eps, float weight_decay,
                    int64_t* step_count, void* stream);
 
+/* ---- gradient clipping by global norm (trainer.py `clip_grad_norm`: torch.nn.utils.clip_grad_norm_) -----------------------
+ * acsr_grad_norm_partial: out[0] = the fp64 sum of |g|^q over grad[ranges[2r] .. ranges[2r+1]) for r < n_ranges (q = norm_type,
+ * a positive number; q = 1 and 2 need no pow), or max |g| for q = inf.  NaN and Inf propagate.  grad holds n floats; ranges is
+ * a HOST array of 2 * n_ranges int64 (1 <= n_ranges <= 8, 0 <= begin <= end <= n; no alignment needed).  block_partials: scratch of
+ * acsr_grad_norm_max_blocks() doubles; counter: one uint32 in device memory, zero before the first call and reset by the last
+ * CTA, which combines the per-CTA partials in a fixed order: bit-identical from run to run and under graph replay.
+ * acsr_adam_step_clipped: acsr_adam_step on grad * coef with coef = min(1, max_norm / (total + 1e-6)) (NaN propagates), where
+ * total = (sum of partials[0 .. n_partials) in index order)^(1/q), or their max for q = inf -- partials of disjoint ranges
+ * of acsr_grad_norm_partial, e.g. the replicated part of the buffer and every rank's item-table shard.  The clipped gradient
+ * is written back to grad and total_out[0] receives the norm (fp32, the value clip_grad_norm_ returns).  max_norm > 0,
+ * 1 <= n_partials <= 1024. */
+int acsr_grad_norm_max_blocks(void);
+int acsr_grad_norm_partial(const float* grad, int64_t n, const int64_t* ranges, int n_ranges, double norm_type,
+                           double* block_partials, uint32_t* counter, double* out, void* stream);
+int acsr_adam_step_clipped(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
+                           float beta2, float eps, float weight_decay, int64_t* step_count, const double* partials, int n_partials,
+                           double norm_type, float max_norm, float* total_out, void* stream);
+
 /* ---- ACTiSASRec (SURVEY section 8 f-4): time-interval aware keys / values ----------------------------------------------
  * replaces model/sequential_recommender/actisasrec.py:104-124, 146-155 and the time-aware terms of
  * model/transformer_layers.py:1085-1091 (context) and 1116-1134 (scores).  The reference gathers two [B,L,L,d] tensors
